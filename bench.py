@@ -145,6 +145,31 @@ def roofline_block(stage_ms, units, cycles):
     return roofline, stages
 
 
+DUMP_BUDGET = 64 << 20           # bytes --dump-outputs may write in all
+
+
+def dump_outputs(out_dir, rec, counts, max_cands):
+    """Write what one device-resident step returned: counts.npy (records per cycle) and rec_<field>.npy for every field of
+    the records, float64 for the integer fields (exact) and float32 for the float ones.  Every value written is finite: fine_sd,
+    NaN ("not computed") in records decoded before the fine stage (ipass < 2), is written as 0 there; rec_ipass tells those
+    records apart.  When the records of the whole batch could exceed DUMP_BUDGET (max_cands records per cycle), only the
+    records of a fixed seeded sample of cycles are written; cycles.npy lists the cycles written.  The sample depends on the
+    batch size and max_cands alone, so two builds run with the same arguments write the same cycles."""
+    fields = [f for f in rec.dtype.names if f != "reserved"]
+    out_dtype = {f: np.float32 if rec.dtype[f].base.kind == "f" else np.float64 for f in fields}
+    rec_bytes = sum(np.dtype(out_dtype[f]).itemsize * int(np.prod(rec.dtype[f].shape)) for f in fields)
+    B = len(counts)
+    k = min(B, (DUMP_BUDGET - 16 * B) // (max_cands * rec_bytes))
+    cycles = np.arange(B) if k == B else np.sort(np.random.default_rng(0).choice(B, k, replace=False))
+    sel = rec[np.isin(rec["cycle"], cycles)]
+    sel["fine_sd"][sel["ipass"] < 2] = 0
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "counts.npy"), counts.astype(np.float64))
+    np.save(os.path.join(out_dir, "cycles.npy"), cycles.astype(np.float64))
+    for f in fields:
+        np.save(os.path.join(out_dir, f"rec_{f}.npy"), sel[f].astype(out_dtype[f]))
+
+
 class ClockSampler:
     """nvidia-smi clocks / throttle reasons sampled every 200 ms during the timed region."""
     Q = "clocks.sm,clocks.max.sm,power.draw,clocks_event_reasons.hw_slowdown,clocks_event_reasons.hw_thermal_slowdown," \
@@ -559,6 +584,8 @@ def run_gpu(args, dist, rank, local, world):
             shm.close()
     if rank != 0:
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dev_records, dev_counts, eng.max_cands)
     units = {"cycles": B, "candidates": stats["candidates"], "fine_evals": stats["fine_evals"],
              "ldpc_calls": max(stats["ldpc_calls"], 1), "osd_calls": max(stats["osd_calls"], 1)}
     roofline, stages = roofline_block(stage_ms, units, B)
@@ -594,7 +621,7 @@ def run_gpu(args, dist, rank, local, world):
         host_pin.close()
         torch.cuda.empty_cache()
         configs = {"cfg3_fec": config_cfg3_fec(local, args.fec_codewords, args.fec_check),
-                   "cfg4_120sig": config_cycles(local, "cfg4_120sig", args.cfg4_cycles, 2, args.seed + 4)}
+                   "cfg4_120sig": config_cycles(local, "cfg4_120sig", args.cfg4_cycles, args.steps, args.seed + 4)}
     out = {
         "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
         "ms_per_step": ms_dev / args.steps, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
@@ -631,7 +658,13 @@ def main():
     ap.add_argument("--fec-codewords", type=int, default=1000000)
     ap.add_argument("--fec-check", type=int, default=64, help="LDPC vectors per Eb/N0 point re-decoded by the oracle (configs.cfg3_fec)")
     ap.add_argument("--cfg4-cycles", type=int, default=8192)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the records and per-cycle counts of the "
+                    "last device-resident step (rank 0's batch) to DIR/<name>.npy, at most 64 MB in all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the CUDA path's outputs (--impl b200)")
     WORKLOAD = args.workload
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     dist, rank, local, world = _dist_init()
