@@ -188,7 +188,9 @@ int ft8_decode_cycles(ft8_handle* h, const void* audio, int audio_dtype, int B, 
  * still hold the previous cycle; a fresh ring is all 1.0 like np.ones), the first hops' windows reach back into the
  * previous cycle's audio, the search runs with cycle_h0 = 375 * odd_even, and payload rows wrap mod 750 into the other
  * half -- so a signal that starts before the cycle boundary (h0 < -32) is read from real rows, as in the reference.
- * Callers alternate odd_even 0, 1, 0, ... per stream position; ft8_live_reset forgets all streams' history. */
+ * Callers alternate odd_even 0, 1, 0, ... per stream position; ft8_live_reset forgets all streams' history.  A stream
+ * without a previous cycle (first call, after a reset, or beyond the B of every earlier call) reads zeros before its first
+ * sample, like a fresh Receiver; the audio dtype may change from one call to the next. */
 int ft8_decode_cycles_live(ft8_handle* h, const void* audio, int audio_dtype, int B, int odd_even,
                            ft8_record* rec, int rec_capacity, int32_t* n_rec, int mem);
 int ft8_live_reset(ft8_handle* h);

@@ -57,7 +57,8 @@ struct ft8_handle {
     cudaEvent_t pf_ev = nullptr;
     float* d_grid = nullptr;
     // live mode (ft8_decode_cycles_live): the reference's two-cycle waterfall ring per stream + the previous cycle's last window
-    float* d_ring = nullptr; void* d_tail = nullptr; int tail_dtype = -1; bool tail_valid = false;
+    // (float32 whatever the input dtype; zero for a stream that has no previous cycle)
+    float* d_ring = nullptr; float* d_tail = nullptr;
     float2* d_Y = nullptr; size_t y_cycles = 0;
     float2* d_spec = nullptr;
     float* d_best_score = nullptr; int16_t* d_best_h0 = nullptr;
@@ -462,13 +463,13 @@ static CandState cand_state(ft8_handle* h) {
 
 static int launch_spectrogram(ft8_handle* h, const void* d_audio, int dtype, int B, float* d_grid, int row_lo = 1,
                               int row_hi = 375, int out_rows = GRID_ROWS, int out_row0 = 0, int fill_row0 = 1,
-                              const void* d_prev_tail = nullptr, int out_wrap = 0) {
+                              const float* d_prev_tail = nullptr, int out_wrap = 0) {
     const bool ring = d_prev_tail != nullptr || out_wrap != 0;
     dim3 grid((row_hi - row_lo + SP_ROWS) / SP_ROWS, B);
     const int smem = SP_ROWS * SP_BUFS * SP_BUF_LEN * (int)sizeof(float2);
 #define SP_LAUNCH(T, RING)                                                                                                          \
     k_spectrogram<T, RING><<<grid, SP_ROWS * SP_NT, smem, h->stream>>>((const T*)d_audio, d_grid, h->d_hann, h->d_TS, h->d_W3840, row_lo, \
-                                                                       row_hi, out_rows, out_row0, fill_row0, (const T*)d_prev_tail, out_wrap)
+                                                                       row_hi, out_rows, out_row0, fill_row0, d_prev_tail, out_wrap)
     if (dtype == FT8_AUDIO_I16) { if (ring) SP_LAUNCH(int16_t, true); else SP_LAUNCH(int16_t, false); }
     else { if (ring) SP_LAUNCH(float, true); else SP_LAUNCH(float, false); }
 #undef SP_LAUNCH
@@ -988,12 +989,19 @@ extern "C" int ft8_prefetch_audio(ft8_handle* h, const void* audio_host, int aud
     return FT8_OK;
 }
 
-// the previous cycle's last 3840 samples per stream, kept for the next live call (D2D strided copy on the handle's stream)
+// the previous cycle's last 3840 samples per stream, kept for the next live call as float32: int16 -> float is exact, so
+// the next call reads the same values whichever dtype either call was given
+template <typename T>
+__global__ void k_save_tails(const T* __restrict__ audio, float* __restrict__ tail) {
+    const T* x = audio + (size_t)blockIdx.x * CYCLE_SAMPLES + (CYCLE_SAMPLES - NFFT_S);
+    float* t = tail + (size_t)blockIdx.x * NFFT_S;
+    for (int i = threadIdx.x; i < NFFT_S; i += blockDim.x) t[i] = (float)x[i];
+}
+
 static int save_tails(ft8_handle* h, const void* d_audio, int dtype, int B) {
-    const size_t esz = dtype == FT8_AUDIO_I16 ? 2 : 4;
-    CK(cudaMemcpy2DAsync(h->d_tail, (size_t)NFFT_S * esz, (const char*)d_audio + (size_t)(CYCLE_SAMPLES - NFFT_S) * esz,
-                         (size_t)CYCLE_SAMPLES * esz, (size_t)NFFT_S * esz, (size_t)B, cudaMemcpyDeviceToDevice, h->stream));
-    h->tail_dtype = dtype; h->tail_valid = true;
+    if (dtype == FT8_AUDIO_I16) k_save_tails<<<B, 256, 0, h->stream>>>((const int16_t*)d_audio, h->d_tail);
+    else k_save_tails<<<B, 256, 0, h->stream>>>((const float*)d_audio, h->d_tail);
+    CK(cudaGetLastError());
     return FT8_OK;
 }
 
@@ -1018,17 +1026,20 @@ static int decode_cycles_core(ft8_handle* h, const void* audio, int audio_dtype,
     const int cycle_h0 = live ? (odd_even ? 375 : 0) : 0;
     const int grows = live ? LIVE_ROWS : GRID_ROWS;
     float* gbase = h->d_grid;
-    const void* tail = nullptr;
+    const float* tail = nullptr;
     if (live) {
         if (!h->d_ring) {
             const size_t n = h->cap_cycles * (size_t)LIVE_ROWS * GRID_COLS;
             CK(dmalloc(&h->d_ring, n));
             k_fill<<<h->n_sm * 8, 256, 0, h->stream>>>(h->d_ring, n, 1.0f);           // np.ones (receiver.py:238)
             CK(cudaGetLastError());
-            CK(cudaMalloc(&h->d_tail, h->cap_cycles * (size_t)NFFT_S * 4));
+            // a stream without a previous cycle reads zeros before its first sample, as a fresh Receiver does; so does a
+            // stream that joins a later call with a larger B
+            CK(dmalloc(&h->d_tail, h->cap_cycles * (size_t)NFFT_S));
+            CK(cudaMemsetAsync(h->d_tail, 0, h->cap_cycles * (size_t)NFFT_S * sizeof(float), h->stream));
         }
         gbase = h->d_ring;
-        if (h->tail_valid && h->tail_dtype == audio_dtype) tail = h->d_tail;
+        tail = h->d_tail;
     }
     const void* da = audio;
     // A pending prefetch is consumed only by the streaming entry (consume_pf), whose caller named this very buffer as the
@@ -1079,7 +1090,7 @@ static int decode_cycles_core(ft8_handle* h, const void* audio, int audio_dtype,
             const char* a = (const char*)h->d_audio + (size_t)b0 * CYCLE_SAMPLES * esz;
             CK(cudaStreamWaitEvent(h->stream, h->chunk_ev[c], 0));
             float* gc = gbase + (size_t)b0 * grows * GRID_COLS;
-            const void* tc = tail ? (const char*)tail + (size_t)b0 * NFFT_S * esz : nullptr;
+            const float* tc = tail ? tail + (size_t)b0 * NFFT_S : nullptr;
             if (live) TRY(launch_spectrogram(h, a, audio_dtype, nb, gc, 1, 375, LIVE_ROWS, -cycle_h0, 0, tc, 1));
             else TRY(launch_spectrogram(h, a, audio_dtype, nb, gc));
             ++launches;
@@ -1106,7 +1117,7 @@ static int decode_cycles_core(ft8_handle* h, const void* audio, int audio_dtype,
         CK(cudaEventRecord(h->ev[3], h->stream));
     }
     if (next_audio_host && !prefetched) TRY(ft8_prefetch_audio(h, next_audio_host, audio_dtype, B));
-    if (live) TRY(save_tails(h, mem == FT8_MEM_HOST ? h->d_audio : da, audio_dtype, B));      // after S1 / F1 have read this audio
+    if (live) { TRY(save_tails(h, mem == FT8_MEM_HOST ? h->d_audio : da, audio_dtype, B)); ++launches; }   // after S1 has read the old tails
     CandState cs = cand_state(h);
     // ipass 0
     k_pass0<<<persistent_blocks(h, 8), WARPS_PER_CTA * 32, sizeof(PassSmem), h->stream>>>(
@@ -1188,8 +1199,8 @@ extern "C" int ft8_live_reset(ft8_handle* h) {
     if (h->d_ring) {
         k_fill<<<h->n_sm * 8, 256, 0, h->stream>>>(h->d_ring, h->cap_cycles * (size_t)LIVE_ROWS * GRID_COLS, 1.0f);
         CK(cudaGetLastError());
+        CK(cudaMemsetAsync(h->d_tail, 0, h->cap_cycles * (size_t)NFFT_S * sizeof(float), h->stream));
     }
-    h->tail_valid = false;
     CK(cudaStreamSynchronize(h->stream));
     return FT8_OK;
 }

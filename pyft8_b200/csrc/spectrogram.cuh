@@ -49,7 +49,7 @@ template <typename T, bool RING = false>
 __global__ void __launch_bounds__(SP_ROWS* SP_NT, SP_MIN_BLOCKS)
 k_spectrogram(const T* __restrict__ audio, float* __restrict__ grid, const float* __restrict__ hann,
               const float2* __restrict__ TS, const float2* __restrict__ W3840, int row_lo, int row_hi, int out_rows,
-              int out_row0, int fill_row0, const T* __restrict__ prev_tail = nullptr, int out_wrap = 0) {
+              int out_row0, int fill_row0, const float* __restrict__ prev_tail = nullptr, int out_wrap = 0) {
     extern __shared__ float2 sp_smem[];
     const int cyc = blockIdx.y;
     const int g = threadIdx.x / SP_NT, lt = threadIdx.x % SP_NT;
@@ -58,8 +58,9 @@ k_spectrogram(const T* __restrict__ audio, float* __restrict__ grid, const float
     float2* buf = sp_smem + g * SP_BUF_LEN * SP_BUFS;
     const T* x = audio + (size_t)cyc * CYCLE_SAMPLES;
     // live ring (receiver.py:295-306): the windows of the first hops of a cycle reach back into the previous cycle's audio;
-    // prev_tail holds its last 3840 samples per stream (nullptr: isolated cycle, samples before the start read as 0)
-    const T* xp = (RING && prev_tail) ? prev_tail + (size_t)cyc * NFFT_S : nullptr;
+    // prev_tail holds its last 3840 samples per stream as float32, whatever T is (zeros for a stream without a previous
+    // cycle; nullptr: isolated cycle, samples before the start read as 0)
+    const float* xp = (RING && prev_tail) ? prev_tail + (size_t)cyc * NFFT_S : nullptr;
     float* out = grid + (size_t)cyc * out_rows * GRID_COLS;
     if (blockIdx.x == 0 && fill_row0) {
         for (int k = threadIdx.x; k < GRID_COLS; k += blockDim.x) out[k] = 1.0f;
