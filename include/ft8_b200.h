@@ -73,7 +73,7 @@ typedef struct ft8_cfg {
     float   llr_sd_min;        /* Candidate(llr_sd_min=5)                                              */
     int32_t osd_singleflips;   /* osd_012(singleflips=30)                                              */
     int32_t osd_doubleflips;   /* osd_012(doubleflips=2)                                               */
-    int32_t max_codewords;     /* scratch capacity of the stand-alone ft8_llr/ft8_ldpc/ft8_osd/ft8_crc14 ops (0: default 1<<16) */
+    int32_t max_codewords;     /* unused; kept for the layout of this struct                                               */
     int32_t fine_mode;         /* fine sync (receiver.py:140-206): 0 = time scan + tensor-core frequency scan + final transform
                                   (default); 1 = the literal nine-inverse-FFT kernel (A/B reference for the former)            */
     /* Receiver(search_freq_range, search_time_range) as index ranges (receiver.py:311-319): coarse frequency bins
@@ -129,8 +129,9 @@ void* ft8_stream(ft8_handle* h);
 /* Milliseconds spent on the device (CUDA events on the handle's stream).  After ft8_decode_cycles: which = 0 whole
  * device section, 1 spectrogram, 2 sync (scores + top-K), 3 cycle spectrum, 4 pass 0 (grid LLR + GOOD91 + LDPC5),
  * 5 fine sync, 6 passes 2-4 (LDPC), 7 passes 5-6 (OSD), 8 record collection, 9 / 10 / 11 the three kernels of the fine stage
- * (time scan, tensor-core frequency scan, final transform; 0 with fine_mode 1).  After a stand-alone ft8_spectrogram /
- * ft8_sync call: 1 / 2 = that kernel.  After ft8_ldpc / ft8_osd: 0 = that kernel. */
+ * (time scan, tensor-core frequency scan, final transform; 0 with fine_mode 1).  Host audio of more than 256 cycles that was
+ * not prefetched is copied and processed in chunks: then 1 covers the whole front end (1-3) and 2 and 3 are 0.
+ * After a stand-alone ft8_spectrogram / ft8_sync call: 1 / 2 = that kernel.  After ft8_ldpc / ft8_osd: 0 = that kernel. */
 int  ft8_last_kernel_ms(ft8_handle* h, int which, float* ms);
 
 /* S1  AudioIn.get_hop_spectrum x375 (receiver.py:288-293): audio[B][180000] -> grid_db[B][376][976] float32 dB. */

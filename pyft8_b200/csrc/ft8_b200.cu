@@ -1,4 +1,5 @@
-// ft8_b200.cu -- handle, table upload and the C ABI (include/ft8_b200.h) of the B200-native FT8 receive path.
+// ft8_b200.cu -- handle, table upload and the C ABI (include/ft8_b200.h) of the B200-native FT8 receive path, with the
+// ABI's small helper kernels; the stage kernels live in the *.cuh headers.
 //
 // Build: nvcc -gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -shared -Xcompiler -fPIC (see __graft_entry__.build).
 // One handle = one device + one stream + constant tables + scratch sized from ft8_cfg.max_cycles.
@@ -25,10 +26,53 @@
 #include "fine_tc.cuh"
 #include "passes.cuh"
 #include "synth.cuh"
+#include "records.cuh"
 
 using namespace ft8;
 
 static thread_local std::string g_create_error;
+
+// Device memory owned by the handle: move-only and freed with its owner.  ensure() only grows: before it frees the old
+// block it synchronises the streams that may still read it, and when the new allocation fails it leaves the buffer empty.
+template <typename T> class DevBuf {
+  public:
+    DevBuf() = default;
+    DevBuf(DevBuf&& o) noexcept : p_(o.p_), n_(o.n_) { o.p_ = nullptr; o.n_ = 0; }
+    DevBuf& operator=(DevBuf&& o) noexcept { std::swap(p_, o.p_); std::swap(n_, o.n_); return *this; }
+    ~DevBuf() { if (p_) cudaFree(p_); }
+    operator T*() const { return p_; }
+    cudaError_t ensure(size_t count, cudaStream_t reader = nullptr, cudaStream_t reader2 = nullptr) {
+        if (count <= n_) return cudaSuccess;
+        if (p_) {
+            cudaError_t e = reader ? cudaStreamSynchronize(reader) : cudaSuccess;
+            if (e == cudaSuccess && reader2) e = cudaStreamSynchronize(reader2);
+            if (e == cudaSuccess) e = cudaFree(p_);
+            if (e != cudaSuccess) return e;
+            p_ = nullptr; n_ = 0;
+        }
+        const cudaError_t e = cudaMalloc((void**)&p_, count * sizeof(T));
+        if (e != cudaSuccess) { p_ = nullptr; return e; }
+        n_ = count;
+        return cudaSuccess;
+    }
+  private:
+    T* p_ = nullptr;
+    size_t n_ = 0;
+};
+
+// slots of d_counts / h_counts: the work-list lengths of the fine and OSD stages, the records written, the near-tie
+// candidates of the frequency scan, the work cursors of k_pass234 / k_osd_items / k_pass0, ft8_fine's out-of-range count
+enum CountSlot { CNT_FINE, CNT_OSD, CNT_RECORDS, CNT_NEAR_TIE, CNT_CURSOR_PASS234, CNT_CURSOR_OSD, CNT_CURSOR_PASS0,
+                 CNT_FINE_BAD, CNT_SLOTS };
+
+// timing events: event i (1..8) ends stage i of a decode as listed at ft8_last_kernel_ms; then the pair around a stand-alone
+// op and the two boundaries inside the three-kernel fine stage
+enum Event { EV_START, EV_SPECTROGRAM, EV_SYNC, EV_CYCLE_SPECTRUM, EV_PASS0, EV_FINE, EV_PASS234, EV_OSD, EV_RECORDS,
+             EV_OP_BEGIN, EV_OP_END, EV_TSCAN_END, EV_FSCAN_END, EV_COUNT };
+
+// `which` of ft8_last_kernel_ms
+enum KernelMs { MS_TOTAL, MS_SPECTROGRAM, MS_SYNC, MS_CYCLE_SPECTRUM, MS_PASS0, MS_FINE, MS_PASS234, MS_OSD, MS_RECORDS,
+                MS_FINE_TSCAN, MS_FINE_FSCAN, MS_FINE_FINAL, MS_COUNT };
 
 struct ft8_handle {
     int device = 0;
@@ -39,46 +83,43 @@ struct ft8_handle {
     ft8_cfg cfg{};
     std::string err;
     // constant-like tables in global memory
-    float* d_hann = nullptr;
-    float2 *d_W1920 = nullptr, *d_W3840 = nullptr, *d_W3200 = nullptr, *d_W375 = nullptr, *d_W256 = nullptr,
-           *d_W96000 = nullptr, *d_W192000 = nullptr, *d_W32 = nullptr;
-    float2 *d_TS = nullptr, *d_TF = nullptr, *d_TC = nullptr, *d_T256 = nullptr, *d_W96000T = nullptr;   // per-pass twiddle tables [k-1][p]
-    float* d_pulse = nullptr;        // GFSK pulse for the synthetic generator
+    DevBuf<float> d_hann;
+    DevBuf<float2> d_W1920, d_W3840, d_W3200, d_W375, d_W256, d_W192000, d_W32;
+    DevBuf<float2> d_TS, d_TF, d_TC, d_T256, d_W96000T;   // per-pass twiddle tables [k-1][p]
+    DevBuf<float> d_pulse;           // GFSK pulse for the synthetic generator
     // tensor-core frequency scan (fine_tc.cuh): B operand (E | M, tf32 hi/lo), half-sample phase table, per-item intermediates
-    float* d_bmat = nullptr; float2* d_w6400 = nullptr;
-    float2* d_zwin = nullptr; TScanOut* d_tso = nullptr; int32_t* d_ff = nullptr; size_t fine_tmp_items = 0;
-    int32_t* d_amb = nullptr;         // [fine_tmp_items + 1]: near-tie candidates of the frequency scan ([0] = count, list from [1])
+    DevBuf<float> d_bmat; DevBuf<float2> d_w6400;
+    DevBuf<float2> d_zwin; DevBuf<TScanOut> d_tso; DevBuf<int32_t> d_ff;
+    DevBuf<int32_t> d_amb;           // [items + 1]: near-tie candidates of the frequency scan ([0] = count, list from [1])
     // batch scratch
     size_t cap_cycles = 0, cap_slots = 0;
-    void* d_audio = nullptr; size_t audio_bytes = 0;
+    DevBuf<char> d_audio;
     // prefetch slot (ft8_prefetch_audio): the NEXT batch's audio is copied here while the current batch is decoded
-    void* d_audio_pf = nullptr; size_t audio_pf_bytes = 0;
+    DevBuf<char> d_audio_pf;
     const void* pf_host = nullptr; int pf_B = 0, pf_dtype = -1;
     cudaEvent_t pf_ev = nullptr;
-    float* d_grid = nullptr;
+    DevBuf<float> d_grid;
     // live mode (ft8_decode_cycles_live): the reference's two-cycle waterfall ring per stream + the previous cycle's last window
     // (float32 whatever the input dtype; zero for a stream that has no previous cycle)
-    float* d_ring = nullptr; float* d_tail = nullptr;
-    float2* d_Y = nullptr; size_t y_cycles = 0;
-    float2* d_spec = nullptr;
-    float* d_best_score = nullptr; int16_t* d_best_h0 = nullptr;
-    int16_t *d_f0 = nullptr, *d_h0 = nullptr; float* d_score = nullptr; int32_t* d_ncand = nullptr;
-    int32_t* d_cycle_of = nullptr;
-    uint8_t* d_status = nullptr; float* d_llr_grid = nullptr; float* d_grid_sd = nullptr; int8_t* d_grid_snr = nullptr;
-    float* d_llr_fine = nullptr; FineOut* d_fine = nullptr; float* d_saved = nullptr; uint8_t* d_saved_n = nullptr;
-    uint8_t* d_saved_ap = nullptr; uint32_t* d_bits = nullptr; uint8_t *d_ripass = nullptr, *d_rap = nullptr, *d_rmethod = nullptr;
-    uint16_t* d_rnits = nullptr; int32_t* d_osd_found = nullptr; uint32_t* d_osd_bits = nullptr;
-    int32_t *d_list_fine = nullptr, *d_list_osd = nullptr, *d_counts = nullptr;   // counts: [0] fine, [1] osd, [2] records
-    DevStats* d_stats = nullptr;
-    ft8_record* d_rec = nullptr;
-    int32_t *d_rec_n = nullptr, *d_rec_base = nullptr;   // per-cycle record counts / offsets
-    int32_t* h_counts = nullptr;      // pinned
+    DevBuf<float> d_ring, d_tail;
+    DevBuf<float2> d_Y; size_t y_cycles = 0;
+    DevBuf<float2> d_spec;
+    DevBuf<float> d_best_score; DevBuf<int16_t> d_best_h0;
+    DevBuf<int16_t> d_f0, d_h0; DevBuf<float> d_score; DevBuf<int32_t> d_ncand;
+    DevBuf<int32_t> d_cycle_of;
+    DevBuf<uint8_t> d_status; DevBuf<float> d_llr_grid, d_grid_sd; DevBuf<int8_t> d_grid_snr;
+    DevBuf<float> d_llr_fine; DevBuf<FineOut> d_fine; DevBuf<float> d_saved; DevBuf<uint8_t> d_saved_n;
+    DevBuf<uint8_t> d_saved_ap; DevBuf<uint32_t> d_bits; DevBuf<uint8_t> d_ripass, d_rap, d_rmethod;
+    DevBuf<uint16_t> d_rnits; DevBuf<int32_t> d_osd_found; DevBuf<uint32_t> d_osd_bits;
+    DevBuf<int32_t> d_list_fine, d_list_osd, d_counts;   // d_counts: [CNT_SLOTS]
+    DevBuf<DevStats> d_stats;
+    DevBuf<ft8_record> d_rec;
+    DevBuf<int32_t> d_rec_n, d_rec_base;   // per-cycle record counts / offsets
+    int32_t* h_counts = nullptr;      // pinned [CNT_SLOTS]
     DevStats* h_stats = nullptr;      // pinned
-    // generic arena for the stand-alone stage ops
-    void* arena = nullptr; size_t arena_bytes = 0;
-    cudaEvent_t ev[14] = {};          // ev[0..8]: stage boundaries of ft8_decode_cycles; ev[10], ev[11]: stand-alone ops;
-                                      // ev[12], ev[13]: between the three kernels of the fine stage
-    float last_ms[12] = {};           // see ft8_last_kernel_ms
+    DevBuf<char> arena;               // host buffers and scratch of the stand-alone stage ops (Staging)
+    cudaEvent_t ev[EV_COUNT] = {};
+    float last_ms[MS_COUNT] = {};
     ft8_stats stats{};
 };
 
@@ -119,10 +160,10 @@ static void append_pass_table(std::vector<float2>& out, int n, int R, int S) {
         for (int p = 0; p < M; ++p) out.push_back(twiddle1(n, (long long)p * k * S));
 }
 
-template <typename T> static cudaError_t upload(T** dst, const std::vector<T>& v) {
-    cudaError_t e = cudaMalloc((void**)dst, v.size() * sizeof(T));
+template <typename T> static cudaError_t upload(DevBuf<T>& dst, const std::vector<T>& v) {
+    cudaError_t e = dst.ensure(v.size());
     if (e != cudaSuccess) return e;
-    return cudaMemcpy(*dst, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice);
+    return cudaMemcpy(dst, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice);
 }
 
 static uint32_t crc14_bits(const uint8_t* msg77) {      // decoders.py:123-129
@@ -234,24 +275,6 @@ static std::vector<float> fscan_bmat() {
     return out;
 }
 
-template <typename T> static cudaError_t dmalloc(T** p, size_t n) { return cudaMalloc((void**)p, n * sizeof(T)); }
-
-static int ensure_arena(ft8_handle* h, size_t bytes) {
-    if (bytes <= h->arena_bytes) return FT8_OK;
-    if (h->arena) { CK(cudaStreamSynchronize(h->stream)); CK(cudaFree(h->arena)); h->arena = nullptr; h->arena_bytes = 0; }
-    CK(cudaMalloc(&h->arena, bytes));
-    h->arena_bytes = bytes;
-    return FT8_OK;
-}
-
-static int ensure_audio(ft8_handle* h, size_t bytes) {
-    if (bytes <= h->audio_bytes) return FT8_OK;
-    if (h->d_audio) { CK(cudaStreamSynchronize(h->stream)); CK(cudaFree(h->d_audio)); h->d_audio = nullptr; h->audio_bytes = 0; }
-    CK(cudaMalloc(&h->d_audio, bytes));
-    h->audio_bytes = bytes;
-    return FT8_OK;
-}
-
 extern "C" void ft8_default_cfg(ft8_cfg* cfg) {
     if (!cfg) return;
     memset(cfg, 0, sizeof(*cfg));
@@ -280,7 +303,6 @@ extern "C" int ft8_create(int device, const ft8_cfg* cfg_in, ft8_handle** out) {
     if (cfg.max_cands > N_F0) cfg.max_cands = N_F0;
     if (cfg.osd_singleflips < 0 || cfg.osd_singleflips > OSD_MAX_FLIPS || cfg.osd_doubleflips < 0)
         return fail(nullptr, FT8_E_BADARG, "ft8_create: osd flips out of range");
-    if (cfg.max_codewords <= 0) cfg.max_codewords = 1 << 16;
     if (cfg.search_f0_lo == 0 && cfg.search_f0_hi == 0) { cfg.search_f0_lo = F0_LO; cfg.search_f0_hi = F0_LO + N_F0; }
     if (cfg.search_h0_lo == 0 && cfg.search_h0_hi == 0) { cfg.search_h0_lo = H0_LO; cfg.search_h0_hi = H0_LO + N_H0; }
     if (cfg.search_f0_lo < F0_LO || cfg.search_f0_hi > F0_LO + N_F0 || cfg.search_f0_lo >= cfg.search_f0_hi ||
@@ -315,14 +337,14 @@ extern "C" int ft8_create(int device, const ft8_cfg* cfg_in, ft8_handle** out) {
             const double n = (double)(1 - NFFT_S + 2 * i);
             w[i] = (float)(0.5 + 0.5 * cos(M_PI * n / (double)(NFFT_S - 1)));
         }
-        CKC(upload(&h->d_hann, w));
-        CKC(upload(&h->d_W1920, twiddles(1920, 1920)));
-        CKC(upload(&h->d_W3840, twiddles(3840, 1921)));
-        CKC(upload(&h->d_W3200, twiddles(3200, 3200)));
-        CKC(upload(&h->d_W375, twiddles(375, 375)));
-        CKC(upload(&h->d_W256, twiddles(256, 256)));
-        CKC(upload(&h->d_W192000, twiddles(192000, 96001)));
-        CKC(upload(&h->d_W32, twiddles(32, 32)));
+        CKC(upload(h->d_hann, w));
+        CKC(upload(h->d_W1920, twiddles(1920, 1920)));
+        CKC(upload(h->d_W3840, twiddles(3840, 1921)));
+        CKC(upload(h->d_W3200, twiddles(3200, 3200)));
+        CKC(upload(h->d_W375, twiddles(375, 375)));
+        CKC(upload(h->d_W256, twiddles(256, 256)));
+        CKC(upload(h->d_W192000, twiddles(192000, 96001)));
+        CKC(upload(h->d_W32, twiddles(32, 32)));
         {   // per-pass tables (coalesced twiddle loads), one buffer per kernel
             std::vector<float2> ts, tf, tc, t256, w96t;
             append_pass_table(ts, 1920, 15, 1); append_pass_table(ts, 1920, 8, 15);                              // SP_T8_OFF
@@ -333,21 +355,21 @@ extern "C" int ft8_create(int device, const ft8_cfg* cfg_in, ft8_handle** out) {
             for (int k1 = 0; k1 < CS_N1; ++k1)
                 for (int n2 = 0; n2 < CS_N2; ++n2) w96t.push_back(twiddle1(96000, (long long)n2 * k1));
             if ((int)ts.size() != SP_T8_OFF + 7 * 16 || (int)tf.size() != FINE_TF_LEN || (int)tc.size() != 370) { ft8_destroy(h); return fail(nullptr, FT8_E_CUDA, "twiddle table layout"); }
-            CKC(upload(&h->d_TS, ts)); CKC(upload(&h->d_TF, tf)); CKC(upload(&h->d_TC, tc)); CKC(upload(&h->d_T256, t256));
-            CKC(upload(&h->d_W96000T, w96t));
+            CKC(upload(h->d_TS, ts)); CKC(upload(h->d_TF, tf)); CKC(upload(h->d_TC, tc)); CKC(upload(h->d_T256, t256));
+            CKC(upload(h->d_W96000T, w96t));
         }
-        CKC(upload(&h->d_pulse, synth_pulse_table()));
-        CKC(upload(&h->d_bmat, fscan_bmat()));
+        CKC(upload(h->d_pulse, synth_pulse_table()));
+        CKC(upload(h->d_bmat, fscan_bmat()));
         {
             std::vector<float2> w(FS_W_LEN);
             for (int g = 0; g < FS_W_LEN; ++g) { const double a = 2.0 * M_PI * (double)g / (double)FS_W_LEN; w[g] = make_float2((float)cos(a), (float)sin(a)); }
-            CKC(upload(&h->d_w6400, w));
+            CKC(upload(h->d_w6400, w));
         }
     }
     const size_t B = (size_t)cfg.max_cycles, K = (size_t)cfg.max_cands, N = B * K;
     h->cap_cycles = B;
     h->cap_slots = N;
-    CKC(dmalloc(&h->d_grid, B * GRID_ROWS * GRID_COLS));
+    CKC(h->d_grid.ensure(B * GRID_ROWS * GRID_COLS));
     // four-step scratch Y: 768 KB per cycle, written by k_cs_cols and read back by k_cs_rows, in chunks of up to 1024 cycles.
     // Smaller, L2-resident chunks (VERDICT r1 item 7) were measured and are SLOWER: 3.18 ms per 4096 cycles at 1024, 3.50 at 256,
     // 3.88 at 128, 4.20 at 64, 5.00 at 32 (profiles/r02_experiments.md) -- both kernels sit on the L1/shared data pipe, not on
@@ -355,33 +377,31 @@ extern "C" int ft8_create(int device, const ft8_cfg* cfg_in, ft8_handle** out) {
     size_t ych = 1024;
     if (const char* e = getenv("FT8_Y_CYCLES")) ych = (size_t)std::max(1, atoi(e));
     h->y_cycles = std::min<size_t>(B, ych);
-    CKC(dmalloc(&h->d_Y, h->y_cycles * CS_N));
-    CKC(dmalloc(&h->d_spec, B * FINE_SPEC_STRIDE));
-    CKC(dmalloc(&h->d_best_score, B * N_F0 * SY_HS));
-    CKC(dmalloc(&h->d_best_h0, B * N_F0 * SY_HS));
-    CKC(dmalloc(&h->d_f0, N)); CKC(dmalloc(&h->d_h0, N)); CKC(dmalloc(&h->d_score, N)); CKC(dmalloc(&h->d_ncand, B));
-    CKC(dmalloc(&h->d_cycle_of, N));
-    CKC(dmalloc(&h->d_status, N)); CKC(dmalloc(&h->d_llr_grid, N * 174)); CKC(dmalloc(&h->d_grid_sd, N)); CKC(dmalloc(&h->d_grid_snr, N));
-    CKC(dmalloc(&h->d_llr_fine, N * 174)); CKC(dmalloc(&h->d_fine, N)); CKC(dmalloc(&h->d_saved, N * 5 * 174));
-    CKC(dmalloc(&h->d_saved_n, N)); CKC(dmalloc(&h->d_saved_ap, N * 5)); CKC(dmalloc(&h->d_bits, N * 3));
-    CKC(dmalloc(&h->d_ripass, N)); CKC(dmalloc(&h->d_rap, N)); CKC(dmalloc(&h->d_rmethod, N)); CKC(dmalloc(&h->d_rnits, N));
-    CKC(dmalloc(&h->d_osd_found, N * 10)); CKC(dmalloc(&h->d_osd_bits, N * 30));
-    CKC(dmalloc(&h->d_list_fine, N)); CKC(dmalloc(&h->d_list_osd, N)); CKC(dmalloc(&h->d_counts, 8));
-    CKC(dmalloc(&h->d_stats, 1)); CKC(dmalloc(&h->d_rec, N)); CKC(dmalloc(&h->d_rec_n, B)); CKC(dmalloc(&h->d_rec_base, B));
-    CKC(cudaMallocHost((void**)&h->h_counts, 8 * sizeof(int32_t)));
+    CKC(h->d_Y.ensure(h->y_cycles * CS_N));
+    CKC(h->d_spec.ensure(B * FINE_SPEC_STRIDE));
+    CKC(h->d_best_score.ensure(B * N_F0 * SY_HS));
+    CKC(h->d_best_h0.ensure(B * N_F0 * SY_HS));
+    CKC(h->d_f0.ensure(N)); CKC(h->d_h0.ensure(N)); CKC(h->d_score.ensure(N)); CKC(h->d_ncand.ensure(B));
+    CKC(h->d_status.ensure(N)); CKC(h->d_llr_grid.ensure(N * 174)); CKC(h->d_grid_sd.ensure(N)); CKC(h->d_grid_snr.ensure(N));
+    CKC(h->d_llr_fine.ensure(N * 174)); CKC(h->d_fine.ensure(N)); CKC(h->d_saved.ensure(N * 5 * 174));
+    CKC(h->d_saved_n.ensure(N)); CKC(h->d_saved_ap.ensure(N * 5)); CKC(h->d_bits.ensure(N * 3));
+    CKC(h->d_ripass.ensure(N)); CKC(h->d_rap.ensure(N)); CKC(h->d_rmethod.ensure(N)); CKC(h->d_rnits.ensure(N));
+    CKC(h->d_osd_found.ensure(N * 10)); CKC(h->d_osd_bits.ensure(N * 30));
+    CKC(h->d_list_fine.ensure(N)); CKC(h->d_list_osd.ensure(N)); CKC(h->d_counts.ensure(CNT_SLOTS));
+    CKC(h->d_stats.ensure(1)); CKC(h->d_rec.ensure(N)); CKC(h->d_rec_n.ensure(B)); CKC(h->d_rec_base.ensure(B));
+    CKC(cudaMallocHost((void**)&h->h_counts, CNT_SLOTS * sizeof(int32_t)));
     CKC(cudaMallocHost((void**)&h->h_stats, sizeof(DevStats)));
     {
         std::vector<int32_t> co(N);
         for (size_t i = 0; i < N; ++i) co[i] = (int32_t)(i / K);
-        CKC(cudaMemcpy(h->d_cycle_of, co.data(), N * sizeof(int32_t), cudaMemcpyHostToDevice));
+        CKC(upload(h->d_cycle_of, co));
     }
     CKC(cudaFuncSetAttribute(k_fine, cudaFuncAttributeMaxDynamicSharedMemorySize, FINE_SMEM_BYTES));
     CKC(cudaFuncSetAttribute(k_fine_tscan<FT_NT, FT_CTAS>, cudaFuncAttributeMaxDynamicSharedMemorySize, FT_SMEM_BYTES));
     CKC(cudaFuncSetAttribute(k_fine_final<FT_NT, FF_CTAS>, cudaFuncAttributeMaxDynamicSharedMemorySize, FF_SMEM_BYTES));
     CKC(cudaFuncSetAttribute(k_fscan_mma, cudaFuncAttributeMaxDynamicSharedMemorySize, FS_SMEM_BYTES));
     if (cfg.fine_mode == 0) {
-        h->fine_tmp_items = N;
-        CKC(dmalloc(&h->d_zwin, N * FS_WIN)); CKC(dmalloc(&h->d_tso, N)); CKC(dmalloc(&h->d_ff, N)); CKC(dmalloc(&h->d_amb, N + 1));
+        CKC(h->d_zwin.ensure(N * FS_WIN)); CKC(h->d_tso.ensure(N)); CKC(h->d_ff.ensure(N)); CKC(h->d_amb.ensure(N + 1));
     }
     {
         const int sp_smem = SP_ROWS * SP_BUFS * SP_BUF_LEN * (int)sizeof(float2);
@@ -401,21 +421,15 @@ extern "C" void ft8_destroy(ft8_handle* h) {
     if (!h) return;
     cudaSetDevice(h->device);
     if (h->stream) cudaStreamSynchronize(h->stream);
-    void* ptrs[] = {h->d_TS, h->d_TF, h->d_TC, h->d_T256, h->d_W96000T, h->d_hann, h->d_W1920, h->d_W3840, h->d_W3200, h->d_W375, h->d_W256, h->d_W96000, h->d_W192000, h->d_W32,
-                    h->d_pulse, h->d_ring, h->d_tail, h->d_bmat, h->d_w6400, h->d_zwin, h->d_tso, h->d_ff, h->d_amb, h->d_audio, h->d_grid, h->d_Y, h->d_spec, h->d_best_score, h->d_best_h0, h->d_f0, h->d_h0, h->d_score,
-                    h->d_ncand, h->d_cycle_of, h->d_status, h->d_llr_grid, h->d_grid_sd, h->d_grid_snr, h->d_llr_fine, h->d_fine,
-                    h->d_saved, h->d_saved_n, h->d_saved_ap, h->d_bits, h->d_ripass, h->d_rap, h->d_rmethod, h->d_rnits,
-                    h->d_osd_found, h->d_osd_bits, h->d_list_fine, h->d_list_osd, h->d_counts, h->d_stats, h->d_rec, h->d_rec_n, h->d_rec_base, h->arena};
-    for (void* p : ptrs) if (p) cudaFree(p);
-    if (h->h_counts) cudaFreeHost(h->h_counts);
-    if (h->h_stats) cudaFreeHost(h->h_stats);
+    if (h->copy_stream) cudaStreamSynchronize(h->copy_stream);
     for (auto& ev : h->ev) if (ev) cudaEventDestroy(ev);
     for (auto& ev : h->chunk_ev) if (ev) cudaEventDestroy(ev);
     if (h->pf_ev) cudaEventDestroy(h->pf_ev);
-    if (h->d_audio_pf) cudaFree(h->d_audio_pf);
     if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
     if (h->stream) cudaStreamDestroy(h->stream);
-    delete h;
+    if (h->h_counts) cudaFreeHost(h->h_counts);
+    if (h->h_stats) cudaFreeHost(h->h_stats);
+    delete h;                        // frees the device buffers
 }
 
 extern "C" const char* ft8_last_error(ft8_handle* h) { return h ? h->err.c_str() : g_create_error.c_str(); }
@@ -445,7 +459,7 @@ extern "C" int ft8_get_stats(ft8_handle* h, ft8_stats* out) {
     return FT8_OK;
 }
 extern "C" int ft8_last_kernel_ms(ft8_handle* h, int which, float* ms) {
-    if (!h || !ms || which < 0 || which > 11) return FT8_E_BADARG;
+    if (!h || !ms || which < 0 || which >= MS_COUNT) return FT8_E_BADARG;
     *ms = h->last_ms[which];
     return FT8_OK;
 }
@@ -523,58 +537,89 @@ static int launch_fine(ft8_handle* h, const float2* spec, int spec_stride, const
         return FT8_OK;
     }
     const size_t need = list ? h->cap_slots : (size_t)n_direct;
-    if (need > h->fine_tmp_items) {
-        CK(cudaStreamSynchronize(h->stream));
-        if (h->d_zwin) CK(cudaFree(h->d_zwin)); if (h->d_tso) CK(cudaFree(h->d_tso)); if (h->d_ff) CK(cudaFree(h->d_ff));
-        if (h->d_amb) CK(cudaFree(h->d_amb));
-        h->d_zwin = nullptr; h->d_tso = nullptr; h->d_ff = nullptr; h->d_amb = nullptr; h->fine_tmp_items = 0;
-        CK(dmalloc(&h->d_zwin, need * FS_WIN)); CK(dmalloc(&h->d_tso, need)); CK(dmalloc(&h->d_ff, need)); CK(dmalloc(&h->d_amb, need + 1));
-        h->fine_tmp_items = need;
-    }
+    CK(h->d_zwin.ensure(need * FS_WIN, h->stream)); CK(h->d_tso.ensure(need, h->stream)); CK(h->d_ff.ensure(need, h->stream));
+    CK(h->d_amb.ensure(need + 1, h->stream));
     const int nbt = list ? persistent_blocks(h, FT_CTAS) : std::min(persistent_blocks(h, FT_CTAS), n_direct);
     const int nb3 = list ? persistent_blocks(h, FF_CTAS) : std::min(persistent_blocks(h, FF_CTAS), n_direct);
     k_fine_tscan<FT_NT, FT_CTAS><<<nbt, FT_NT, FT_SMEM_BYTES, h->stream>>>(spec, spec_stride, list, count, n_direct, cycle_of, f0, h0, h->d_TF, h->d_tso, h->d_zwin);
     CK(cudaGetLastError());
-    CK(cudaEventRecord(h->ev[12], h->stream));
+    CK(cudaEventRecord(h->ev[EV_TSCAN_END], h->stream));
     const int nb1 = list ? h->n_sm : std::min(h->n_sm, (n_direct + FS_CAND - 1) / FS_CAND);
     CK(cudaMemsetAsync(h->d_amb, 0, sizeof(int32_t), h->stream));
     k_fscan_mma<<<nb1, FS_NT, FS_SMEM_BYTES, h->stream>>>(spec, spec_stride, list, count, n_direct, cycle_of, f0, h0, h->d_tso, h->d_zwin,
                                                          h->d_bmat, h->d_w6400, h->d_ff, h->d_amb + 1, h->d_amb);
     CK(cudaGetLastError());
-    CK(cudaEventRecord(h->ev[13], h->stream));
+    CK(cudaEventRecord(h->ev[EV_FSCAN_END], h->stream));
     k_fine_final<FT_NT, FF_CTAS><<<nb3, FT_NT, FF_SMEM_BYTES, h->stream>>>(spec, spec_stride, list, count, n_direct, cycle_of, f0, h0, h->d_TF, h->d_tso, h->d_ff,
                                                             fo, llr, sig_grid);
     CK(cudaGetLastError());
     // near-tie candidates of the frequency scan: decided by the literal nine-transform kernel (overwrites their results)
     k_fine<<<persistent_blocks(h, 2), FINE_NT, FINE_SMEM_BYTES, h->stream>>>(spec, spec_stride, h->d_amb + 1, h->d_amb, 0, cycle_of, f0, h0, h->d_TF, fo, llr, sig_grid);
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(h->d_counts + 3, h->d_amb, sizeof(int32_t), cudaMemcpyDeviceToDevice, h->stream));      // statistics: counts[3]
+    CK(cudaMemcpyAsync(h->d_counts + CNT_NEAR_TIE, h->d_amb, sizeof(int32_t), cudaMemcpyDeviceToDevice, h->stream));
     return FT8_OK;
 }
 static int fine_launches(ft8_handle* h) { return h->cfg.fine_mode == 1 ? 1 : 4; }
-
-// copy helpers honouring the mem flag
-static int to_device(ft8_handle* h, void* d, const void* src, size_t bytes, int mem) {
-    CK(cudaMemcpyAsync(d, src, bytes, mem == FT8_MEM_HOST ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, h->stream));
-    return FT8_OK;
-}
-static int from_device(ft8_handle* h, void* dst, const void* d, size_t bytes, int mem) {
-    CK(cudaMemcpyAsync(dst, d, bytes, mem == FT8_MEM_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, h->stream));
-    return FT8_OK;
-}
 
 #define ENTER(h)                                  \
     if (!(h)) return FT8_E_BADARG;                \
     CK(cudaSetDevice((h)->device));
 #define TRY(x) do { int r__ = (x); if (r__ != FT8_OK) return r__; } while (0)
 
-static int stage_audio(ft8_handle* h, const void* audio, int dtype, int B, int mem, const void** d_audio) {
+static int check_dtype(ft8_handle* h, int dtype) {
     if (dtype != FT8_AUDIO_I16 && dtype != FT8_AUDIO_F32) return fail(h, FT8_E_BADARG, "audio_dtype must be FT8_AUDIO_I16 or FT8_AUDIO_F32");
-    if (mem == FT8_MEM_DEVICE) { *d_audio = audio; return FT8_OK; }
-    const size_t bytes = (size_t)B * CYCLE_SAMPLES * (dtype == FT8_AUDIO_I16 ? 2 : 4);
-    TRY(ensure_audio(h, bytes));
-    TRY(to_device(h, h->d_audio, audio, bytes, mem));
-    *d_audio = h->d_audio;
+    return FT8_OK;
+}
+static size_t sample_bytes(int dtype) { return dtype == FT8_AUDIO_I16 ? 2 : 4; }
+
+// Caller buffers of one stand-alone op.  With FT8_MEM_DEVICE a caller buffer is used in place; with FT8_MEM_HOST it gets a
+// slice of the handle's arena: begin() copies the inputs in and finish() copies the outputs back before its final
+// synchronise.  Scratch is always a slice of the arena.  begin() sizes the arena from the declarations and grows it, which
+// frees the old arena, so every buffer is declared before begin() and the declared pointers are set by it.  A NULL caller
+// buffer (an optional output) stays NULL.
+class Staging {
+  public:
+    Staging(ft8_handle* h, int mem) : h_(h), host_(mem == FT8_MEM_HOST) {}
+    template <typename T> void in(const T*& dev, const void* user, size_t bytes) { add(dev, user, bytes, true, false); }
+    template <typename T> void out(T*& dev, void* user, size_t bytes) { add(dev, user, bytes, false, true); }
+    template <typename T> void inout(T*& dev, void* user, size_t bytes) { add(dev, user, bytes, true, true); }
+    template <typename T> void scratch(T*& dev, size_t bytes) { add(dev, nullptr, bytes, false, false); }
+
+    int begin() {
+        ft8_handle* h = h_;
+        CK(h->arena.ensure(bytes_, h->stream));
+        for (const Slot& s : slots_) {
+            char* p = h->arena + s.off;
+            memcpy(s.dev, &p, sizeof(p));
+            if (s.in) CK(cudaMemcpyAsync(p, s.user, s.bytes, cudaMemcpyHostToDevice, h->stream));
+        }
+        return FT8_OK;
+    }
+    int finish() {
+        ft8_handle* h = h_;
+        for (const Slot& s : slots_)
+            if (s.out) CK(cudaMemcpyAsync((void*)s.user, h->arena + s.off, s.bytes, cudaMemcpyDeviceToHost, h->stream));
+        CK(cudaStreamSynchronize(h->stream));
+        return FT8_OK;
+    }
+
+  private:
+    struct Slot { void* dev; const void* user; size_t off, bytes; bool in, out; };
+    template <typename P> void add(P& dev, const void* user, size_t bytes, bool in, bool out) {
+        if ((in || out) && (!host_ || !user)) { dev = (P)user; return; }
+        const size_t off = (bytes_ + 255) & ~(size_t)255;
+        slots_.push_back({&dev, user, off, bytes, in, out});
+        bytes_ = off + bytes;
+    }
+    ft8_handle* h_;
+    bool host_;
+    std::vector<Slot> slots_;
+    size_t bytes_ = 0;
+};
+
+// copy of a handle-owned device array to a caller buffer
+static int from_device(ft8_handle* h, void* dst, const void* d, size_t bytes, int mem) {
+    CK(cudaMemcpyAsync(dst, d, bytes, mem == FT8_MEM_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, h->stream));
     return FT8_OK;
 }
 
@@ -583,39 +628,41 @@ extern "C" int ft8_spectrogram(ft8_handle* h, const void* audio, int audio_dtype
     ENTER(h);
     if (!audio || !grid_db || B <= 0) return fail(h, FT8_E_BADARG, "ft8_spectrogram: bad argument");
     if ((size_t)B > h->cap_cycles) return fail(h, FT8_E_CAPACITY, "ft8_spectrogram: B exceeds cfg.max_cycles");
-    const void* da;
-    TRY(stage_audio(h, audio, audio_dtype, B, mem, &da));
-    float* dg = mem == FT8_MEM_DEVICE ? grid_db : h->d_grid;
-    CK(cudaEventRecord(h->ev[10], h->stream));
+    TRY(check_dtype(h, audio_dtype));
+    const char* da; float* dg;
+    Staging st(h, mem);
+    st.in(da, audio, (size_t)B * CYCLE_SAMPLES * sample_bytes(audio_dtype));
+    st.out(dg, grid_db, (size_t)B * GRID_ROWS * GRID_COLS * sizeof(float));
+    TRY(st.begin());
+    CK(cudaEventRecord(h->ev[EV_OP_BEGIN], h->stream));
     TRY(launch_spectrogram(h, da, audio_dtype, B, dg));
-    CK(cudaEventRecord(h->ev[11], h->stream));
-    if (mem == FT8_MEM_HOST) TRY(from_device(h, grid_db, dg, (size_t)B * GRID_ROWS * GRID_COLS * sizeof(float), mem));
-    CK(cudaStreamSynchronize(h->stream));
-    CK(cudaEventElapsedTime(&h->last_ms[1], h->ev[10], h->ev[11]));
+    CK(cudaEventRecord(h->ev[EV_OP_END], h->stream));
+    TRY(st.finish());
+    CK(cudaEventElapsedTime(&h->last_ms[MS_SPECTROGRAM], h->ev[EV_OP_BEGIN], h->ev[EV_OP_END]));
     return FT8_OK;
 }
 
 extern "C" int ft8_hop_spectrum(ft8_handle* h, const void* audio_buffer, int audio_dtype, float* row_db, int mem) {
     ENTER(h);
     if (!audio_buffer || !row_db) return fail(h, FT8_E_BADARG, "ft8_hop_spectrum: bad argument");
-    if (audio_dtype != FT8_AUDIO_I16 && audio_dtype != FT8_AUDIO_F32) return fail(h, FT8_E_BADARG, "audio_dtype must be FT8_AUDIO_I16 or FT8_AUDIO_F32");
-    const size_t esz = audio_dtype == FT8_AUDIO_I16 ? 2 : 4;
+    TRY(check_dtype(h, audio_dtype));
+    const size_t esz = sample_bytes(audio_dtype);
     const void* da = audio_buffer;
     if (mem == FT8_MEM_HOST) {
         // only the last 3840 samples are read (receiver.py:289): stage those 15 KB at their place in a cycle-sized buffer,
         // not the whole 720 KB ring, every 40 ms hop
-        TRY(ensure_audio(h, (size_t)CYCLE_SAMPLES * esz));
+        CK(h->d_audio.ensure((size_t)CYCLE_SAMPLES * esz, h->stream));
         const size_t off = (size_t)(CYCLE_SAMPLES - NFFT_S) * esz;
-        TRY(to_device(h, (char*)h->d_audio + off, (const char*)audio_buffer + off, (size_t)NFFT_S * esz, mem));
+        CK(cudaMemcpyAsync(h->d_audio + off, (const char*)audio_buffer + off, (size_t)NFFT_S * esz, cudaMemcpyHostToDevice, h->stream));
         da = h->d_audio;
     }
-    float* dr = row_db;
-    if (mem == FT8_MEM_HOST) { TRY(ensure_arena(h, GRID_COLS * sizeof(float))); dr = (float*)h->arena; }
+    float* dr;
+    Staging st(h, mem);
+    st.out(dr, row_db, GRID_COLS * sizeof(float));
+    TRY(st.begin());
     // the window over the last 3840 samples of a 180000-sample buffer is row 375 of that buffer's waterfall
     TRY(launch_spectrogram(h, da, audio_dtype, 1, dr, 375, 375, 1, 375, 0));
-    if (mem == FT8_MEM_HOST) TRY(from_device(h, row_db, dr, GRID_COLS * sizeof(float), mem));
-    CK(cudaStreamSynchronize(h->stream));
-    return FT8_OK;
+    return st.finish();
 }
 
 extern "C" int ft8_sync(ft8_handle* h, const float* grid_db, int grid_rows, int B, int odd_even, int16_t* cand_f0,
@@ -624,86 +671,63 @@ extern "C" int ft8_sync(ft8_handle* h, const float* grid_db, int grid_rows, int 
     if (!grid_db || !cand_f0 || !cand_h0 || !cand_score || !n_cand || B <= 0) return fail(h, FT8_E_BADARG, "ft8_sync: bad argument");
     if (grid_rows != GRID_ROWS && grid_rows != LIVE_ROWS) return fail(h, FT8_E_BADARG, "ft8_sync: grid_rows must be 376 or 750");
     if ((size_t)B > h->cap_cycles) return fail(h, FT8_E_CAPACITY, "ft8_sync: B exceeds cfg.max_cycles");
+    if (payload_db && mem == FT8_MEM_HOST && grid_rows != GRID_ROWS)
+        return fail(h, FT8_E_BADARG, "ft8_sync: payload_db with a host 750-row grid is not supported; pass grid_rows=376 or device memory");
     const size_t K = h->cfg.max_cands, N = (size_t)B * K;
-    const float* dg = grid_db;
-    if (mem == FT8_MEM_HOST) {
-        const size_t bytes = (size_t)B * grid_rows * GRID_COLS * sizeof(float);
-        if (grid_rows == GRID_ROWS) { TRY(to_device(h, h->d_grid, grid_db, bytes, mem)); dg = h->d_grid; }
-        else { TRY(ensure_arena(h, bytes)); TRY(to_device(h, h->arena, grid_db, bytes, mem)); dg = (const float*)h->arena; }
-    }
+    const float* dg; float* d_pay;
+    Staging st(h, mem);
+    st.in(dg, grid_db, (size_t)B * grid_rows * GRID_COLS * sizeof(float));
+    st.out(d_pay, payload_db, N * 58 * 8 * sizeof(float));
+    TRY(st.begin());
     CK(cudaMemsetAsync(h->d_f0, 0, N * 2, h->stream));
     CK(cudaMemsetAsync(h->d_h0, 0, N * 2, h->stream));
     CK(cudaMemsetAsync(h->d_score, 0, N * 4, h->stream));
-    CK(cudaEventRecord(h->ev[10], h->stream));
+    CK(cudaEventRecord(h->ev[EV_OP_BEGIN], h->stream));
     TRY(launch_sync(h, dg, grid_rows, B, odd_even));
-    CK(cudaEventRecord(h->ev[11], h->stream));
-    float* d_pay = nullptr;
+    CK(cudaEventRecord(h->ev[EV_OP_END], h->stream));
     if (payload_db) {
-        if (mem == FT8_MEM_DEVICE) d_pay = payload_db;
-        else {
-            // the arena may hold the live grid: place the payload scratch after it
-            const size_t gbytes = (grid_rows == GRID_ROWS) ? 0 : (size_t)B * grid_rows * GRID_COLS * sizeof(float);
-            if (gbytes) return fail(h, FT8_E_BADARG, "ft8_sync: payload_db with a host 750-row grid is not supported; pass grid_rows=376 or device memory");
-            TRY(ensure_arena(h, N * 58 * 8 * sizeof(float)));
-            d_pay = (float*)h->arena;
-        }
         CK(cudaMemsetAsync(d_pay, 0, N * 58 * 8 * sizeof(float), h->stream));
         CK(cudaMemsetAsync(h->d_stats, 0, sizeof(DevStats), h->stream));
-        CK(cudaMemsetAsync(h->d_counts, 0, 8 * sizeof(int32_t), h->stream));
+        CK(cudaMemsetAsync(h->d_counts, 0, CNT_SLOTS * sizeof(int32_t), h->stream));
         k_pass0<<<persistent_blocks(h, 8), WARPS_PER_CTA * 32, sizeof(PassSmem), h->stream>>>(
-            cand_state(h), (int)N, dg, grid_rows, odd_even ? 375 : 0, h->cfg.llr_sd_min, d_pay, 1, h->d_list_fine, h->d_counts, h->d_counts + 6, h->d_stats);
+            cand_state(h), (int)N, dg, grid_rows, odd_even ? 375 : 0, h->cfg.llr_sd_min, d_pay, 1, h->d_list_fine,
+            h->d_counts + CNT_FINE, h->d_counts + CNT_CURSOR_PASS0, h->d_stats);
         CK(cudaGetLastError());
     }
     TRY(from_device(h, cand_f0, h->d_f0, N * 2, mem));
     TRY(from_device(h, cand_h0, h->d_h0, N * 2, mem));
     TRY(from_device(h, cand_score, h->d_score, N * 4, mem));
     TRY(from_device(h, n_cand, h->d_ncand, (size_t)B * 4, mem));
-    if (payload_db && mem == FT8_MEM_HOST) TRY(from_device(h, payload_db, d_pay, N * 58 * 8 * sizeof(float), mem));
-    CK(cudaStreamSynchronize(h->stream));
-    CK(cudaEventElapsedTime(&h->last_ms[2], h->ev[10], h->ev[11]));
+    TRY(st.finish());
+    CK(cudaEventElapsedTime(&h->last_ms[MS_SYNC], h->ev[EV_OP_BEGIN], h->ev[EV_OP_END]));
     return FT8_OK;
 }
-
-// carve typed sub-buffers out of the arena
-struct Carver {
-    char* base; size_t off = 0;
-    template <typename T> T* take(size_t n) { off = (off + 255) & ~(size_t)255; T* p = (T*)(base + off); off += n * sizeof(T); return p; }
-};
 
 extern "C" int ft8_llr(ft8_handle* h, const float* payload_db, int N, float* llr, float* sd, int32_t* snr, int mem) {
     ENTER(h);
     if (!payload_db || !llr || !sd || !snr || N <= 0) return fail(h, FT8_E_BADARG, "ft8_llr: bad argument");
-    const float* dp = payload_db; float* dl = llr; float* ds = sd; int32_t* dn = snr;
-    if (mem == FT8_MEM_HOST) {
-        TRY(ensure_arena(h, (size_t)N * (464 + 174 + 2) * 4 + 4096));
-        Carver c{(char*)h->arena};
-        float* p = c.take<float>((size_t)N * 464); dl = c.take<float>((size_t)N * 174); ds = c.take<float>(N); dn = c.take<int32_t>(N);
-        TRY(to_device(h, p, payload_db, (size_t)N * 464 * 4, mem));
-        dp = p;
-    }
+    const float* dp; float *dl, *ds; int32_t* dn;
+    Staging st(h, mem);
+    st.in(dp, payload_db, (size_t)N * 464 * 4);
+    st.out(dl, llr, (size_t)N * 174 * 4); st.out(ds, sd, (size_t)N * 4); st.out(dn, snr, (size_t)N * 4);
+    TRY(st.begin());
     k_llr_batch<<<std::min(persistent_blocks(h, 8), (N + WARPS_PER_CTA - 1) / WARPS_PER_CTA), WARPS_PER_CTA * 32, 0, h->stream>>>(dp, N, dl, ds, dn);
     CK(cudaGetLastError());
-    if (mem == FT8_MEM_HOST) {
-        TRY(from_device(h, llr, dl, (size_t)N * 174 * 4, mem));
-        TRY(from_device(h, sd, ds, (size_t)N * 4, mem));
-        TRY(from_device(h, snr, dn, (size_t)N * 4, mem));
-    }
-    CK(cudaStreamSynchronize(h->stream));
-    return FT8_OK;
+    return st.finish();
 }
 
 extern "C" int ft8_cycle_spectrum(ft8_handle* h, const void* audio, int audio_dtype, int B, float* spec, int mem) {
     ENTER(h);
     if (!audio || !spec || B <= 0) return fail(h, FT8_E_BADARG, "ft8_cycle_spectrum: bad argument");
     if ((size_t)B > h->cap_cycles) return fail(h, FT8_E_CAPACITY, "ft8_cycle_spectrum: B exceeds cfg.max_cycles");
-    const void* da;
-    TRY(stage_audio(h, audio, audio_dtype, B, mem, &da));
-    float2* ds = (float2*)spec;
-    if (mem == FT8_MEM_HOST) { TRY(ensure_arena(h, (size_t)B * FT8_SPEC_BINS * sizeof(float2))); ds = (float2*)h->arena; }
+    TRY(check_dtype(h, audio_dtype));
+    const char* da; float2* ds;
+    Staging st(h, mem);
+    st.in(da, audio, (size_t)B * CYCLE_SAMPLES * sample_bytes(audio_dtype));
+    st.out(ds, spec, (size_t)B * FT8_SPEC_BINS * sizeof(float2));
+    TRY(st.begin());
     TRY(launch_cycle_spectrum(h, da, audio_dtype, B, ds, FT8_SPEC_BINS, FT8_SPEC_BINS - 1));
-    if (mem == FT8_MEM_HOST) TRY(from_device(h, spec, ds, (size_t)B * FT8_SPEC_BINS * sizeof(float2), mem));
-    CK(cudaStreamSynchronize(h->stream));
-    return FT8_OK;
+    return st.finish();
 }
 
 // ft8_fine helpers: range check of caller-supplied candidates on the device (works for host and device callers alike)
@@ -725,70 +749,46 @@ extern "C" int ft8_fine(ft8_handle* h, const float* spec, int B, const int32_t* 
     ENTER(h);
     if (!spec || !cycle_of || !f0_idx || !h0_idx || !ttweak || !ftweak || !nsync || !llr || !sd || !snr || N <= 0 || B <= 0)
         return fail(h, FT8_E_BADARG, "ft8_fine: bad argument");
-    const size_t specn = (size_t)B * FT8_SPEC_BINS;
-    size_t need = specn * 8 + (size_t)N * (4 + 2 + 2 + sizeof(FineOut) + 174 * 4 + 632 * 4 + 5 * 4) + 16 * 256;
-    TRY(ensure_arena(h, need));
-    Carver c{(char*)h->arena};
-    float2* dspec = c.take<float2>(specn);
-    int32_t* dco = c.take<int32_t>(N); int16_t* df0 = c.take<int16_t>(N); int16_t* dh0 = c.take<int16_t>(N);
-    FineOut* dfo = c.take<FineOut>(N); float* dllr = c.take<float>((size_t)N * 174); float* dsg = c.take<float>((size_t)N * 632);
-    int32_t* dtt = c.take<int32_t>(N); int32_t* dff = c.take<int32_t>(N); int32_t* dns = c.take<int32_t>(N);
-    float* dsd = c.take<float>(N); int32_t* dsn = c.take<int32_t>(N); int32_t* dbad = c.take<int32_t>(1);
-    const float2* sp = (const float2*)spec;
-    if (mem == FT8_MEM_HOST) { TRY(to_device(h, dspec, spec, specn * 8, mem)); sp = dspec; }
-    TRY(to_device(h, dco, cycle_of, (size_t)N * 4, mem));
-    TRY(to_device(h, df0, f0_idx, (size_t)N * 2, mem));
-    TRY(to_device(h, dh0, h0_idx, (size_t)N * 2, mem));
+    const float2* sp; const int32_t* dco; const int16_t *df0, *dh0; FineOut* dfo;
+    int32_t *dtt, *dff, *dns, *dsn; float *dsd, *dllr, *dsg;
+    Staging st(h, mem);
+    st.in(sp, spec, (size_t)B * FT8_SPEC_BINS * sizeof(float2));
+    st.in(dco, cycle_of, (size_t)N * 4); st.in(df0, f0_idx, (size_t)N * 2); st.in(dh0, h0_idx, (size_t)N * 2);
+    st.scratch(dfo, (size_t)N * sizeof(FineOut));
+    st.out(dtt, ttweak, (size_t)N * 4); st.out(dff, ftweak, (size_t)N * 4); st.out(dns, nsync, (size_t)N * 4);
+    st.out(dsd, sd, (size_t)N * 4); st.out(dsn, snr, (size_t)N * 4);
+    st.out(dllr, llr, (size_t)N * 174 * 4); st.out(dsg, signal_grid, (size_t)N * 632 * 4);
+    TRY(st.begin());
     // candidates are range-checked on the device before anything gathers with them (host AND device callers)
-    CK(cudaMemsetAsync(dbad, 0, 4, h->stream));
-    k_fine_validate<<<(N + 255) / 256, 256, 0, h->stream>>>(dco, df0, dh0, N, B, dbad);
+    CK(cudaMemsetAsync(h->d_counts + CNT_FINE_BAD, 0, 4, h->stream));
+    k_fine_validate<<<(N + 255) / 256, 256, 0, h->stream>>>(dco, df0, dh0, N, B, h->d_counts + CNT_FINE_BAD);
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(h->h_counts + 3, dbad, 4, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(h->h_counts + CNT_FINE_BAD, h->d_counts + CNT_FINE_BAD, 4, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
-    if (h->h_counts[3] != 0)
+    if (h->h_counts[CNT_FINE_BAD] != 0)
         return fail(h, FT8_E_BADARG, "ft8_fine: candidate outside the supported range (-100 <= h0 <= 200, 4 <= f0 <= 1880, 0 <= cycle_of < B)");
-    float* out_llr = mem == FT8_MEM_HOST ? dllr : llr;
-    float* out_sg = signal_grid ? (mem == FT8_MEM_HOST ? dsg : signal_grid) : nullptr;
-    TRY(launch_fine(h, sp, FT8_SPEC_BINS, nullptr, nullptr, N, dco, df0, dh0, dfo, out_llr, out_sg));
-    const bool host = mem == FT8_MEM_HOST;
-    k_fine_unpack<<<(N + 255) / 256, 256, 0, h->stream>>>(dfo, N, host ? dtt : ttweak, host ? dff : ftweak, host ? dns : nsync,
-                                                          host ? dsd : sd, host ? dsn : snr);
+    TRY(launch_fine(h, sp, FT8_SPEC_BINS, nullptr, nullptr, N, dco, df0, dh0, dfo, dllr, dsg));
+    k_fine_unpack<<<(N + 255) / 256, 256, 0, h->stream>>>(dfo, N, dtt, dff, dns, dsd, dsn);
     CK(cudaGetLastError());
-    if (host) {
-        TRY(from_device(h, ttweak, dtt, (size_t)N * 4, mem)); TRY(from_device(h, ftweak, dff, (size_t)N * 4, mem));
-        TRY(from_device(h, nsync, dns, (size_t)N * 4, mem)); TRY(from_device(h, sd, dsd, (size_t)N * 4, mem));
-        TRY(from_device(h, snr, dsn, (size_t)N * 4, mem));
-        TRY(from_device(h, llr, dllr, (size_t)N * 174 * 4, mem));
-        if (signal_grid) TRY(from_device(h, signal_grid, dsg, (size_t)N * 632 * 4, mem));
-    }
-    CK(cudaStreamSynchronize(h->stream));
-    return FT8_OK;
+    return st.finish();
 }
 
 extern "C" int ft8_ldpc(ft8_handle* h, float* llr, int N, int max_ncheck0, int max_iters, int32_t* status, int32_t* nits,
                         uint32_t* bits91, int mem) {
     ENTER(h);
     if (!llr || !status || !nits || !bits91 || N <= 0 || max_iters < 0) return fail(h, FT8_E_BADARG, "ft8_ldpc: bad argument");
-    float* dl = llr; int32_t* dst = status; int32_t* dn = nits; uint32_t* db = bits91;
-    if (mem == FT8_MEM_HOST) {
-        TRY(ensure_arena(h, (size_t)N * (174 + 1 + 1 + 3) * 4 + 4096));
-        Carver c{(char*)h->arena};
-        dl = c.take<float>((size_t)N * 174); dst = c.take<int32_t>(N); dn = c.take<int32_t>(N); db = c.take<uint32_t>((size_t)N * 3);
-        TRY(to_device(h, dl, llr, (size_t)N * 174 * 4, mem));
-    }
-    CK(cudaEventRecord(h->ev[10], h->stream));
+    float* dl; int32_t *dst, *dn; uint32_t* db;
+    Staging st(h, mem);
+    st.inout(dl, llr, (size_t)N * 174 * 4);
+    st.out(dst, status, (size_t)N * 4); st.out(dn, nits, (size_t)N * 4); st.out(db, bits91, (size_t)N * 12);
+    TRY(st.begin());
+    CK(cudaEventRecord(h->ev[EV_OP_BEGIN], h->stream));
     k_ldpc_batch<<<std::min(persistent_blocks(h, 8), (N + WARPS_PER_CTA - 1) / WARPS_PER_CTA), WARPS_PER_CTA * 32, sizeof(PassSmem), h->stream>>>(
         dl, N, max_ncheck0, max_iters, dst, dn, db);
     CK(cudaGetLastError());
-    CK(cudaEventRecord(h->ev[11], h->stream));
-    if (mem == FT8_MEM_HOST) {
-        TRY(from_device(h, llr, dl, (size_t)N * 174 * 4, mem));
-        TRY(from_device(h, status, dst, (size_t)N * 4, mem));
-        TRY(from_device(h, nits, dn, (size_t)N * 4, mem));
-        TRY(from_device(h, bits91, db, (size_t)N * 12, mem));
-    }
-    CK(cudaStreamSynchronize(h->stream));
-    CK(cudaEventElapsedTime(&h->last_ms[0], h->ev[10], h->ev[11]));
+    CK(cudaEventRecord(h->ev[EV_OP_END], h->stream));
+    TRY(st.finish());
+    CK(cudaEventElapsedTime(&h->last_ms[MS_TOTAL], h->ev[EV_OP_BEGIN], h->ev[EV_OP_END]));
     return FT8_OK;
 }
 
@@ -797,189 +797,42 @@ extern "C" int ft8_osd(ft8_handle* h, const float* llr, int N, int singleflips, 
     ENTER(h);
     if (!llr || !found || !bits91 || N <= 0 || singleflips < 0 || singleflips > OSD_MAX_FLIPS || doubleflips < 0)
         return fail(h, FT8_E_BADARG, "ft8_osd: bad argument (singleflips must be 0..91)");
-    const float* dl = llr; int32_t* df = found; uint32_t* db = bits91;
-    if (mem == FT8_MEM_HOST) {
-        TRY(ensure_arena(h, (size_t)N * (174 + 1 + 3) * 4 + 4096));
-        Carver c{(char*)h->arena};
-        float* l = c.take<float>((size_t)N * 174); df = c.take<int32_t>(N); db = c.take<uint32_t>((size_t)N * 3);
-        TRY(to_device(h, l, llr, (size_t)N * 174 * 4, mem));
-        dl = l;
-    }
-    CK(cudaEventRecord(h->ev[10], h->stream));
+    const float* dl; int32_t* df; uint32_t* db;
+    Staging st(h, mem);
+    st.in(dl, llr, (size_t)N * 174 * 4);
+    st.out(df, found, (size_t)N * 4); st.out(db, bits91, (size_t)N * 12);
+    TRY(st.begin());
+    CK(cudaEventRecord(h->ev[EV_OP_BEGIN], h->stream));
     k_osd_batch<<<std::min(persistent_blocks(h, 8), (N + WARPS_PER_CTA - 1) / WARPS_PER_CTA), WARPS_PER_CTA * 32, sizeof(OsdSmem), h->stream>>>(
         dl, N, singleflips, doubleflips, df, db);
     CK(cudaGetLastError());
-    CK(cudaEventRecord(h->ev[11], h->stream));
-    if (mem == FT8_MEM_HOST) {
-        TRY(from_device(h, found, df, (size_t)N * 4, mem));
-        TRY(from_device(h, bits91, db, (size_t)N * 12, mem));
-    }
-    CK(cudaStreamSynchronize(h->stream));
-    CK(cudaEventElapsedTime(&h->last_ms[0], h->ev[10], h->ev[11]));
+    CK(cudaEventRecord(h->ev[EV_OP_END], h->stream));
+    TRY(st.finish());
+    CK(cudaEventElapsedTime(&h->last_ms[MS_TOTAL], h->ev[EV_OP_BEGIN], h->ev[EV_OP_END]));
     return FT8_OK;
 }
 
 extern "C" int ft8_crc14(ft8_handle* h, const uint32_t* bits91, int N, int32_t* flags, int mem) {
     ENTER(h);
     if (!bits91 || !flags || N <= 0) return fail(h, FT8_E_BADARG, "ft8_crc14: bad argument");
-    const uint32_t* db = bits91; int32_t* df = flags;
-    if (mem == FT8_MEM_HOST) {
-        TRY(ensure_arena(h, (size_t)N * 16 + 4096));
-        Carver c{(char*)h->arena};
-        uint32_t* b = c.take<uint32_t>((size_t)N * 3); df = c.take<int32_t>(N);
-        TRY(to_device(h, b, bits91, (size_t)N * 12, mem));
-        db = b;
-    }
+    const uint32_t* db; int32_t* df;
+    Staging st(h, mem);
+    st.in(db, bits91, (size_t)N * 12);
+    st.out(df, flags, (size_t)N * 4);
+    TRY(st.begin());
     k_crc_batch<<<std::min(persistent_blocks(h, 8), (N + 127) / 128), 128, 0, h->stream>>>(db, N, df);
     CK(cudaGetLastError());
-    if (mem == FT8_MEM_HOST) TRY(from_device(h, flags, df, (size_t)N * 4, mem));
-    CK(cudaStreamSynchronize(h->stream));
-    return FT8_OK;
+    return st.finish();
 }
 
 // ------------------------------------------------------------------------------------------ whole path
-// Record packaging on the device (R1; receiver.py:51-66, 389-398).  One CTA per cycle orders that cycle's decoded
-// candidates in the reference's emission order -- pass by pass; inside a pass by llr_sd descending (the fine sd from
-// ipass 2 on, all-equal before), ties by candidate rank -- flags later duplicates of a payload (receiver.py:53-55) and
-// writes the records contiguously at base[cycle], so the host only copies.
-constexpr int REC_MAXC = 928, REC_NT = 256;
-
-__global__ void __launch_bounds__(REC_NT) k_rec_count(CandState cs, int32_t* __restrict__ n_per_cycle) {
-    __shared__ int cnt;
-    const int cyc = blockIdx.x;
-    if (threadIdx.x == 0) cnt = 0;
-    __syncthreads();
-    const int n = cs.n_cand[cyc];
-    int c = 0;
-    for (int r = threadIdx.x; r < n; r += REC_NT) c += cs.status[cyc * cs.K + r] == ST_DECODED;
-    if (c) atomicAdd(&cnt, c);
-    __syncthreads();
-    if (threadIdx.x == 0) n_per_cycle[cyc] = cnt;
-}
-
-// exclusive scan of n_per_cycle[B] -> base[B], total -> *total (single CTA)
-__global__ void __launch_bounds__(1024) k_rec_scan(const int32_t* __restrict__ n_per_cycle, int B, int32_t* __restrict__ base,
-                                                   int32_t* __restrict__ total) {
-    __shared__ int warp_sum[32];
-    __shared__ int carry;
-    if (threadIdx.x == 0) carry = 0;
-    __syncthreads();
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    for (int b0 = 0; b0 < B; b0 += 1024) {
-        const int i = b0 + threadIdx.x;
-        const int v = i < B ? n_per_cycle[i] : 0;
-        int x = v;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) { const int y = __shfl_up_sync(0xffffffffu, x, o); if (lane >= o) x += y; }
-        if (lane == 31) warp_sum[w] = x;
-        __syncthreads();
-        if (w == 0) {
-            int s = warp_sum[lane];
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) { const int y = __shfl_up_sync(0xffffffffu, s, o); if (lane >= o) s += y; }
-            warp_sum[lane] = s;
-        }
-        __syncthreads();
-        const int before = carry + (w ? warp_sum[w - 1] : 0) + x - v;
-        if (i < B) base[i] = before;
-        __syncthreads();
-        if (threadIdx.x == 1023) carry = before + v;
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) *total = carry;
-}
-
-__global__ void __launch_bounds__(REC_NT)
-k_rec_write(CandState cs, const FineOut* __restrict__ fine, const int32_t* __restrict__ base, ft8_record* __restrict__ rec,
-            DevStats* __restrict__ stats) {
-    __shared__ uint16_t s_rank[REC_MAXC];      // candidate rank (index inside the cycle) of the i-th decoded candidate
-    __shared__ uint8_t s_ipass[REC_MAXC];
-    __shared__ float s_sd[REC_MAXC];
-    __shared__ uint32_t s_w[REC_MAXC][3];
-    __shared__ int s_n, s_emit;
-    const int cyc = blockIdx.x, lane = threadIdx.x & 31;
-    if (threadIdx.x == 0) { s_n = 0; s_emit = 0; }
-    __syncthreads();
-    const int n = cs.n_cand[cyc];
-    // compaction in candidate order (ballot scan per warp-sized chunk keeps it deterministic)
-    for (int r0 = 0; r0 < n; r0 += REC_NT) {
-        const int r = r0 + threadIdx.x;
-        const bool dec = r < n && cs.status[cyc * cs.K + r] == ST_DECODED;
-        const uint32_t m = __ballot_sync(0xffffffffu, dec);
-        __shared__ int wbase[REC_NT / 32];
-        if (lane == 0) wbase[threadIdx.x >> 5] = __popc(m);
-        __syncthreads();
-        int off = s_n;
-        for (int w = 0; w < (threadIdx.x >> 5); ++w) off += wbase[w];
-        if (dec) {
-            const int i = off + __popc(m & ((1u << lane) - 1u));
-            const int slot = cyc * cs.K + r;
-            s_rank[i] = (uint16_t)r;
-            s_ipass[i] = cs.r_ipass[slot];
-            s_sd[i] = cs.r_ipass[slot] >= 2 ? fine[slot].sd : 0.0f;
-            s_w[i][0] = cs.bits91[3 * slot]; s_w[i][1] = cs.bits91[3 * slot + 1]; s_w[i][2] = cs.bits91[3 * slot + 2] & 0x1FFFu;
-        }
-        __syncthreads();
-        if (threadIdx.x == 0) { int t = 0; for (int w = 0; w < REC_NT / 32; ++w) t += wbase[w]; s_n += t; }
-        __syncthreads();
-    }
-    const int nd = s_n;
-    int emitted_here = 0;
-    for (int i = threadIdx.x; i < nd; i += REC_NT) {
-        const int ip = s_ipass[i];
-        const float sd = s_sd[i];
-        const int rk = s_rank[i];
-        int pos = 0;
-        bool dup = false;
-        for (int j = 0; j < nd; ++j) {
-            const int jp = s_ipass[j];
-            bool before;                      // does j precede i in emission order?
-            if (jp != ip) before = jp < ip;
-            else if (ip >= 2 && s_sd[j] != sd) before = s_sd[j] > sd;
-            else before = s_rank[j] < rk;
-            if (before) {
-                ++pos;
-                dup = dup || (s_w[j][0] == s_w[i][0] && s_w[j][1] == s_w[i][1] && s_w[j][2] == s_w[i][2]);
-            }
-        }
-        const int slot = cyc * cs.K + rk;
-        ft8_record r;
-        memset(&r, 0, sizeof(r));
-        r.bits91[0] = cs.bits91[3 * slot]; r.bits91[1] = cs.bits91[3 * slot + 1]; r.bits91[2] = cs.bits91[3 * slot + 2];
-        r.cycle = cyc; r.cand = (int16_t)rk; r.f0_idx = cs.f0[slot]; r.h0_idx = cs.h0[slot];
-        r.ipass = (uint8_t)ip; r.ap = cs.r_ap[slot]; r.method = cs.r_method[slot]; r.n_its = cs.r_nits[slot];
-        r.score = cs.score[slot]; r.grid_sd = cs.grid_sd[slot];
-        r.emitted = dup ? 0 : 1;
-        emitted_here += dup ? 0 : 1;
-        // float(h0/25) and 3.125*f0 like receiver.py:350-351 (python floats; rounded to fp32 for the record)
-        double tsec = (double)r.h0_idx / 25.0, fhz = 3.125 * (double)r.f0_idx;
-        if (ip >= 2) {
-            const FineOut fo = fine[slot];
-            r.ttweak = (int8_t)fo.tt; r.ftweak = (int8_t)fo.ff; r.nsync = (uint8_t)fo.nsync; r.fine_sd = fo.sd; r.snr = (int8_t)fo.snr;
-            tsec += (double)fo.tt / 200.0; fhz += (double)fo.ff / 16.0;
-        } else {
-            r.nsync = 100; r.fine_sd = nanf(""); r.snr = cs.grid_snr[slot];
-        }
-        r.tsec = (float)tsec; r.fHz = (float)fhz;
-        rec[base[cyc] + pos] = r;
-    }
-    if (emitted_here) atomicAdd(&s_emit, emitted_here);
-    __syncthreads();
-    if (threadIdx.x == 0 && s_emit) atomicAdd(&stats->emitted, (unsigned long long)s_emit);
-}
-
 extern "C" int ft8_prefetch_audio(ft8_handle* h, const void* audio_host, int audio_dtype, int B) {
     ENTER(h);
     if (!audio_host || B <= 0 || (audio_dtype != FT8_AUDIO_I16 && audio_dtype != FT8_AUDIO_F32))
         return fail(h, FT8_E_BADARG, "ft8_prefetch_audio: bad argument");
     if ((size_t)B > h->cap_cycles) return fail(h, FT8_E_CAPACITY, "ft8_prefetch_audio: B exceeds cfg.max_cycles");
-    const size_t bytes = (size_t)B * CYCLE_SAMPLES * (audio_dtype == FT8_AUDIO_I16 ? 2 : 4);
-    if (bytes > h->audio_pf_bytes) {
-        if (h->d_audio_pf) { CK(cudaStreamSynchronize(h->copy_stream)); CK(cudaStreamSynchronize(h->stream)); CK(cudaFree(h->d_audio_pf)); }
-        h->d_audio_pf = nullptr; h->audio_pf_bytes = 0;
-        CK(cudaMalloc(&h->d_audio_pf, bytes));
-        h->audio_pf_bytes = bytes;
-    }
+    const size_t bytes = (size_t)B * CYCLE_SAMPLES * sample_bytes(audio_dtype);
+    CK(h->d_audio_pf.ensure(bytes, h->copy_stream, h->stream));
     // the slot may still be read by kernels of the call that consumed the previous prefetch (same stream order)
     CK(cudaEventRecord(h->pf_ev, h->stream));
     CK(cudaStreamWaitEvent(h->copy_stream, h->pf_ev, 0));
@@ -1009,6 +862,76 @@ __global__ void k_fill(float* p, size_t n, float v) {
     for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) p[i] = v;
 }
 
+// A fresh ring is all 1.0 like np.ones (receiver.py:238).  A stream without a previous cycle reads zeros before its first
+// sample, as a fresh Receiver does; so does a stream that joins a later call with a larger B.
+static int clear_live(ft8_handle* h) {
+    k_fill<<<h->n_sm * 8, 256, 0, h->stream>>>(h->d_ring, h->cap_cycles * (size_t)LIVE_ROWS * GRID_COLS, 1.0f);
+    CK(cudaGetLastError());
+    CK(cudaMemsetAsync(h->d_tail, 0, h->cap_cycles * (size_t)NFFT_S * sizeof(float), h->stream));
+    return FT8_OK;
+}
+
+// Decode prologue.  A pending prefetch is consumed only by the streaming entry (consume_pf), whose caller named this very
+// buffer as the next batch and so promises it has not been rewritten since; every other call drops it -- after waiting for
+// its copy, which may still be reading the caller's host buffer.  *d_audio is where the batch is on the device (for host
+// audio that was not prefetched: where it is to be copied); *prefetched says whether it came from the prefetch.
+static int take_audio(ft8_handle* h, const void* audio, int dtype, int B, int mem, bool consume_pf, const void** d_audio,
+                      bool* prefetched) {
+    *prefetched = consume_pf && mem == FT8_MEM_HOST && h->pf_host == audio && h->pf_B == B && h->pf_dtype == dtype;
+    if (!*prefetched && h->pf_host) CK(cudaStreamSynchronize(h->copy_stream));
+    h->pf_host = nullptr;                        // a pending prefetch this call does not consume is dropped, never decoded later
+    *d_audio = audio;
+    if (*prefetched) {
+        // this batch was copied by ft8_prefetch_audio while the previous call was computing: swap it in and go on as if
+        // the audio were device-resident
+        std::swap(h->d_audio, h->d_audio_pf);
+        CK(cudaStreamWaitEvent(h->stream, h->pf_ev, 0));
+        *d_audio = h->d_audio;
+    } else if (mem == FT8_MEM_HOST) {
+        CK(h->d_audio.ensure((size_t)B * CYCLE_SAMPLES * sample_bytes(dtype), h->stream));
+        *d_audio = h->d_audio;
+    }
+    return FT8_OK;
+}
+
+// Decode epilogue: counts, records and statistics back to the host.  Records are cycle-major, so when rec_capacity cuts
+// them the per-cycle counts are trimmed to what was copied.
+static int finish_decode(ft8_handle* h, int B, ft8_record* rec, int rec_capacity, int32_t* n_rec, int launches) {
+    CK(cudaMemcpyAsync(h->h_counts, h->d_counts, (CNT_NEAR_TIE + 1) * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(h->h_stats, h->d_stats, sizeof(DevStats), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(n_rec, h->d_rec_n, (size_t)B * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    const int nrec = h->h_counts[CNT_RECORDS];
+    const int ncopy = std::min(nrec, rec_capacity);
+    if (ncopy > 0) {
+        CK(cudaMemcpyAsync(rec, h->d_rec, (size_t)ncopy * sizeof(ft8_record), cudaMemcpyDeviceToHost, h->stream));
+        CK(cudaStreamSynchronize(h->stream));
+    }
+    const bool overflow = nrec > rec_capacity;
+    if (overflow) {
+        int left = rec_capacity;
+        for (int b = 0; b < B; ++b) { const int t = std::min(n_rec[b], left); n_rec[b] = t; left -= t; }
+    }
+    const int64_t emitted = (int64_t)h->h_stats->emitted;
+    CK(cudaEventElapsedTime(&h->last_ms[MS_TOTAL], h->ev[EV_START], h->ev[EV_RECORDS]));
+    for (int i = MS_SPECTROGRAM; i <= MS_RECORDS; ++i) CK(cudaEventElapsedTime(&h->last_ms[i], h->ev[i - 1], h->ev[i]));
+    h->last_ms[MS_FINE_TSCAN] = h->last_ms[MS_FINE_FSCAN] = h->last_ms[MS_FINE_FINAL] = 0.0f;
+    if (h->cfg.fine_mode == 0) {
+        CK(cudaEventElapsedTime(&h->last_ms[MS_FINE_TSCAN], h->ev[EV_PASS0], h->ev[EV_TSCAN_END]));
+        CK(cudaEventElapsedTime(&h->last_ms[MS_FINE_FSCAN], h->ev[EV_TSCAN_END], h->ev[EV_FSCAN_END]));
+        CK(cudaEventElapsedTime(&h->last_ms[MS_FINE_FINAL], h->ev[EV_FSCAN_END], h->ev[EV_FINE]));
+    }
+    ft8_stats& s = h->stats;
+    memset(&s, 0, sizeof(s));
+    s.cycles = B; s.candidates = (int64_t)h->h_stats->candidates; s.stopped_sd = (int64_t)h->h_stats->stopped_sd;
+    s.fine_evals = (int64_t)h->h_stats->fine_evals; s.fine_pass = (int64_t)h->h_stats->fine_pass;
+    s.ldpc_calls = (int64_t)h->h_stats->ldpc_calls; s.ldpc_iters = (int64_t)h->h_stats->ldpc_iters;
+    s.osd_calls = (int64_t)h->h_stats->osd_calls; s.decoded = nrec; s.emitted = emitted; s.kernel_launches = launches;
+    s.fine_rechecked = h->cfg.fine_mode == 0 ? h->h_counts[CNT_NEAR_TIE] : 0;
+    if (overflow) return fail(h, FT8_E_CAPACITY, "ft8_decode_cycles: rec_capacity too small (records truncated)");
+    return FT8_OK;
+}
+
 static int decode_cycles_core(ft8_handle* h, const void* audio, int audio_dtype, int B, int odd_even, ft8_record* rec,
                               int rec_capacity, int32_t* n_rec, int mem, const void* next_audio_host, bool consume_pf,
                               bool live = false) {
@@ -1021,166 +944,103 @@ static int decode_cycles_core(ft8_handle* h, const void* audio, int audio_dtype,
     // Live mode: stream b keeps the reference's 750-row two-cycle ring (receiver.py:238, 295-306); this call's rows go to the
     // half odd_even selects, rows of the other half still hold the previous cycle, and the first hops' windows reach back into
     // the previous cycle's last samples -- so candidates with h0 < -32 read real rows, exactly as a live Receiver does.
-    if (audio_dtype != FT8_AUDIO_I16 && audio_dtype != FT8_AUDIO_F32) return fail(h, FT8_E_BADARG, "audio_dtype must be FT8_AUDIO_I16 or FT8_AUDIO_F32");
-    const size_t esz = audio_dtype == FT8_AUDIO_I16 ? 2 : 4;
+    TRY(check_dtype(h, audio_dtype));
+    const size_t esz = sample_bytes(audio_dtype);
     const int cycle_h0 = live ? (odd_even ? 375 : 0) : 0;
     const int grows = live ? LIVE_ROWS : GRID_ROWS;
     float* gbase = h->d_grid;
-    const float* tail = nullptr;
     if (live) {
         if (!h->d_ring) {
-            const size_t n = h->cap_cycles * (size_t)LIVE_ROWS * GRID_COLS;
-            CK(dmalloc(&h->d_ring, n));
-            k_fill<<<h->n_sm * 8, 256, 0, h->stream>>>(h->d_ring, n, 1.0f);           // np.ones (receiver.py:238)
-            CK(cudaGetLastError());
-            // a stream without a previous cycle reads zeros before its first sample, as a fresh Receiver does; so does a
-            // stream that joins a later call with a larger B
-            CK(dmalloc(&h->d_tail, h->cap_cycles * (size_t)NFFT_S));
-            CK(cudaMemsetAsync(h->d_tail, 0, h->cap_cycles * (size_t)NFFT_S * sizeof(float), h->stream));
+            CK(h->d_ring.ensure(h->cap_cycles * (size_t)LIVE_ROWS * GRID_COLS, h->stream));
+            CK(h->d_tail.ensure(h->cap_cycles * (size_t)NFFT_S, h->stream));
+            TRY(clear_live(h));
         }
         gbase = h->d_ring;
-        tail = h->d_tail;
     }
-    const void* da = audio;
-    // A pending prefetch is consumed only by the streaming entry (consume_pf), whose caller named this very buffer as the
-    // next batch and so promises it has not been rewritten since; every other call drops it -- after waiting for its copy,
-    // which may still be reading the caller's host buffer.
-    const bool prefetched = consume_pf && mem == FT8_MEM_HOST && h->pf_host == audio && h->pf_B == B && h->pf_dtype == audio_dtype;
-    if (!prefetched && h->pf_host) CK(cudaStreamSynchronize(h->copy_stream));
-    if (prefetched) {
-        // this batch was copied by ft8_prefetch_audio while the previous call was computing: swap it in and go on as if
-        // the audio were device-resident
-        std::swap(h->d_audio, h->d_audio_pf);
-        std::swap(h->audio_bytes, h->audio_pf_bytes);
-        h->pf_host = nullptr;
-        CK(cudaStreamWaitEvent(h->stream, h->pf_ev, 0));
-        da = h->d_audio;
-        mem = FT8_MEM_DEVICE;
-    } else {
-        h->pf_host = nullptr;                    // a pending prefetch this call does not consume is dropped, never decoded later
-        if (mem == FT8_MEM_HOST) { TRY(ensure_audio(h, (size_t)B * CYCLE_SAMPLES * esz)); da = h->d_audio; }
-    }
+    const void* da;
+    bool prefetched;
+    TRY(take_audio(h, audio, audio_dtype, B, mem, consume_pf, &da, &prefetched));
+    const bool copy = mem == FT8_MEM_HOST && !prefetched;
     // streaming callers name the next batch: its copy is queued now and runs underneath this batch's kernels
     // (after this batch's own copies when it was not prefetched itself, so that they are not queued behind it)
     if (next_audio_host && prefetched) TRY(ft8_prefetch_audio(h, next_audio_host, audio_dtype, B));
     int launches = 0;
-    CK(cudaMemsetAsync(h->d_counts, 0, 8 * sizeof(int32_t), h->stream));   // [0] fine list, [1] osd list, [2] records, [4],[5] work cursors
+    CK(cudaMemsetAsync(h->d_counts, 0, CNT_SLOTS * sizeof(int32_t), h->stream));
     CK(cudaMemsetAsync(h->d_stats, 0, sizeof(DevStats), h->stream));
-    CK(cudaEventRecord(h->ev[0], h->stream));
-    if (mem == FT8_MEM_HOST && B > 64) {
-        // host audio: copy in chunks on the copy stream; S1, S2 and F1 of a chunk start as soon as it has landed,
-        // so the PCIe transfer hides behind the front-end kernels (stage timers then cover the whole front end as "S1")
-        // up to 16 equal chunks (measured best for a single handle: 28.6 k cycles/s vs 27.3-28.0 k for growing chunks);
-        // callers that stream batch after batch should use ft8_prefetch_audio, which hides the whole transfer
-        int cb[16], cn[16];
-        const int nchunk = std::min(16, (B + 255) / 256);
-        const int per = (B + nchunk - 1) / nchunk;
-        for (int c = 0; c < nchunk; ++c) { cb[c] = c * per; cn[c] = std::max(0, std::min(per, B - c * per)); }
+    CK(cudaEventRecord(h->ev[EV_START], h->stream));
+    // Front end (S1, S2, F1) chunk by chunk.  Host audio is copied on the copy stream in up to 16 equal chunks, and a chunk's
+    // kernels start as soon as it has landed, so the PCIe transfer hides behind the front end of the chunks before it
+    // (measured best for a single handle: 28.6 k cycles/s vs 27.3-28.0 k for growing chunks); callers that stream batch
+    // after batch should use ft8_prefetch_audio, which hides the whole transfer.  Device-resident or prefetched audio is one
+    // chunk.  With one chunk the stage events fall between S1, S2 and F1; with several, stage 1 covers the whole front end.
+    const int nchunk = copy ? std::min(16, (B + 255) / 256) : 1;
+    const int per = (B + nchunk - 1) / nchunk;
+    if (copy) {
         CK(cudaEventRecord(h->chunk_ev[0], h->stream));
         CK(cudaStreamWaitEvent(h->copy_stream, h->chunk_ev[0], 0));        // previous users of d_audio on the main stream are done
-        for (int c = 0; c < nchunk; ++c) {
-            if (cn[c] <= 0) continue;
-            const size_t off = (size_t)cb[c] * CYCLE_SAMPLES * esz;
-            CK(cudaMemcpyAsync((char*)h->d_audio + off, (const char*)audio + off, (size_t)cn[c] * CYCLE_SAMPLES * esz, cudaMemcpyHostToDevice, h->copy_stream));
+        for (int c = 0, b0 = 0; b0 < B; ++c, b0 += per) {
+            const size_t off = (size_t)b0 * CYCLE_SAMPLES * esz;
+            CK(cudaMemcpyAsync(h->d_audio + off, (const char*)audio + off, (size_t)std::min(per, B - b0) * CYCLE_SAMPLES * esz,
+                               cudaMemcpyHostToDevice, h->copy_stream));
             CK(cudaEventRecord(h->chunk_ev[c], h->copy_stream));
         }
-        for (int c = 0; c < nchunk; ++c) {
-            const int b0 = cb[c], nb = cn[c];
-            if (nb <= 0) continue;
-            const char* a = (const char*)h->d_audio + (size_t)b0 * CYCLE_SAMPLES * esz;
-            CK(cudaStreamWaitEvent(h->stream, h->chunk_ev[c], 0));
-            float* gc = gbase + (size_t)b0 * grows * GRID_COLS;
-            const float* tc = tail ? tail + (size_t)b0 * NFFT_S : nullptr;
-            if (live) TRY(launch_spectrogram(h, a, audio_dtype, nb, gc, 1, 375, LIVE_ROWS, -cycle_h0, 0, tc, 1));
-            else TRY(launch_spectrogram(h, a, audio_dtype, nb, gc));
-            ++launches;
-            TRY(launch_sync(h, gc, grows, nb, live ? odd_even : 0, b0)); launches += 2;
-            TRY(launch_cycle_spectrum(h, a, audio_dtype, nb, h->d_spec + (size_t)b0 * FINE_SPEC_STRIDE, FINE_SPEC_STRIDE, FINE_SPEC_STRIDE - 1));
-            launches += 2 * ((nb + (int)h->y_cycles - 1) / (int)h->y_cycles);
-        }
-        CK(cudaEventRecord(h->ev[1], h->stream));
-        CK(cudaEventRecord(h->ev[2], h->stream));
-        CK(cudaEventRecord(h->ev[3], h->stream));
-    } else {
-        if (mem == FT8_MEM_HOST) TRY(to_device(h, h->d_audio, audio, (size_t)B * CYCLE_SAMPLES * esz, mem));
-        // S1
-        if (live) TRY(launch_spectrogram(h, da, audio_dtype, B, gbase, 1, 375, LIVE_ROWS, -cycle_h0, 0, tail, 1));
-        else TRY(launch_spectrogram(h, da, audio_dtype, B, gbase));
-        ++launches;
-        CK(cudaEventRecord(h->ev[1], h->stream));
-        // S2
-        TRY(launch_sync(h, gbase, grows, B, live ? odd_even : 0)); launches += 2;
-        CK(cudaEventRecord(h->ev[2], h->stream));
-        // F1 (independent of S1/S2; same stream)
-        TRY(launch_cycle_spectrum(h, da, audio_dtype, B, h->d_spec, FINE_SPEC_STRIDE, FINE_SPEC_STRIDE - 1));
-        launches += 2 * ((B + (int)h->y_cycles - 1) / (int)h->y_cycles);
-        CK(cudaEventRecord(h->ev[3], h->stream));
     }
+    for (int c = 0, b0 = 0; b0 < B; ++c, b0 += per) {
+        const int nb = std::min(per, B - b0);
+        const char* a = (const char*)da + (size_t)b0 * CYCLE_SAMPLES * esz;
+        if (copy) CK(cudaStreamWaitEvent(h->stream, h->chunk_ev[c], 0));
+        float* gc = gbase + (size_t)b0 * grows * GRID_COLS;
+        if (live) TRY(launch_spectrogram(h, a, audio_dtype, nb, gc, 1, 375, LIVE_ROWS, -cycle_h0, 0, h->d_tail + (size_t)b0 * NFFT_S, 1));
+        else TRY(launch_spectrogram(h, a, audio_dtype, nb, gc));
+        ++launches;
+        if (nchunk == 1) CK(cudaEventRecord(h->ev[EV_SPECTROGRAM], h->stream));
+        TRY(launch_sync(h, gc, grows, nb, live ? odd_even : 0, b0)); launches += 2;
+        if (nchunk == 1) CK(cudaEventRecord(h->ev[EV_SYNC], h->stream));
+        // F1 (independent of S1/S2; same stream)
+        TRY(launch_cycle_spectrum(h, a, audio_dtype, nb, h->d_spec + (size_t)b0 * FINE_SPEC_STRIDE, FINE_SPEC_STRIDE, FINE_SPEC_STRIDE - 1));
+        launches += 2 * ((nb + (int)h->y_cycles - 1) / (int)h->y_cycles);
+    }
+    if (nchunk > 1) {
+        CK(cudaEventRecord(h->ev[EV_SPECTROGRAM], h->stream));
+        CK(cudaEventRecord(h->ev[EV_SYNC], h->stream));
+    }
+    CK(cudaEventRecord(h->ev[EV_CYCLE_SPECTRUM], h->stream));
     if (next_audio_host && !prefetched) TRY(ft8_prefetch_audio(h, next_audio_host, audio_dtype, B));
-    if (live) { TRY(save_tails(h, mem == FT8_MEM_HOST ? h->d_audio : da, audio_dtype, B)); ++launches; }   // after S1 has read the old tails
+    if (live) { TRY(save_tails(h, da, audio_dtype, B)); ++launches; }   // after S1 has read the old tails
     CandState cs = cand_state(h);
     // ipass 0
     k_pass0<<<persistent_blocks(h, 8), WARPS_PER_CTA * 32, sizeof(PassSmem), h->stream>>>(
-        cs, N, gbase, grows, cycle_h0, h->cfg.llr_sd_min, nullptr, 0, h->d_list_fine, h->d_counts + 0, h->d_counts + 6, h->d_stats);
+        cs, N, gbase, grows, cycle_h0, h->cfg.llr_sd_min, nullptr, 0, h->d_list_fine, h->d_counts + CNT_FINE,
+        h->d_counts + CNT_CURSOR_PASS0, h->d_stats);
     CK(cudaGetLastError()); ++launches;
-    CK(cudaEventRecord(h->ev[4], h->stream));
+    CK(cudaEventRecord(h->ev[EV_PASS0], h->stream));
     // ipass 1
-    TRY(launch_fine(h, h->d_spec, FINE_SPEC_STRIDE, h->d_list_fine, h->d_counts + 0, 0, h->d_cycle_of, h->d_f0, h->d_h0, h->d_fine,
+    TRY(launch_fine(h, h->d_spec, FINE_SPEC_STRIDE, h->d_list_fine, h->d_counts + CNT_FINE, 0, h->d_cycle_of, h->d_f0, h->d_h0, h->d_fine,
                     h->d_llr_fine, nullptr));
     launches += fine_launches(h);
-    CK(cudaEventRecord(h->ev[5], h->stream));
+    CK(cudaEventRecord(h->ev[EV_FINE], h->stream));
     // ipass 2-4
     k_pass234<<<persistent_blocks(h, 8), WARPS_PER_CTA * 32, sizeof(PassSmem), h->stream>>>(
-        cs, h->d_list_fine, h->d_counts + 0, h->cfg.llr_sd_min, h->d_list_osd, h->d_counts + 1, h->d_counts + 4, h->d_stats);
+        cs, h->d_list_fine, h->d_counts + CNT_FINE, h->cfg.llr_sd_min, h->d_list_osd, h->d_counts + CNT_OSD,
+        h->d_counts + CNT_CURSOR_PASS234, h->d_stats);
     CK(cudaGetLastError()); ++launches;
-    CK(cudaEventRecord(h->ev[6], h->stream));
+    CK(cudaEventRecord(h->ev[EV_PASS234], h->stream));
     // ipass 5-6
     k_osd_items<<<persistent_blocks(h, 8), WARPS_PER_CTA * 32, sizeof(OsdSmem), h->stream>>>(
-        cs, h->d_list_osd, h->d_counts + 1, h->cfg.osd_singleflips, h->cfg.osd_doubleflips, h->d_counts + 5, h->d_stats);
+        cs, h->d_list_osd, h->d_counts + CNT_OSD, h->cfg.osd_singleflips, h->cfg.osd_doubleflips, h->d_counts + CNT_CURSOR_OSD,
+        h->d_stats);
     CK(cudaGetLastError()); ++launches;
-    k_osd_resolve<<<persistent_blocks(h, 2), 128, 0, h->stream>>>(cs, h->d_list_osd, h->d_counts + 1, h->d_stats);
+    k_osd_resolve<<<persistent_blocks(h, 2), 128, 0, h->stream>>>(cs, h->d_list_osd, h->d_counts + CNT_OSD, h->d_stats);
     CK(cudaGetLastError()); ++launches;
-    CK(cudaEventRecord(h->ev[7], h->stream));
+    CK(cudaEventRecord(h->ev[EV_OSD], h->stream));
     k_rec_count<<<B, REC_NT, 0, h->stream>>>(cs, h->d_rec_n);
     CK(cudaGetLastError()); ++launches;
-    k_rec_scan<<<1, 1024, 0, h->stream>>>(h->d_rec_n, B, h->d_rec_base, h->d_counts + 2);
+    k_rec_scan<<<1, 1024, 0, h->stream>>>(h->d_rec_n, B, h->d_rec_base, h->d_counts + CNT_RECORDS);
     CK(cudaGetLastError()); ++launches;
     k_rec_write<<<B, REC_NT, 0, h->stream>>>(cs, h->d_fine, h->d_rec_base, h->d_rec, h->d_stats);
     CK(cudaGetLastError()); ++launches;
-    CK(cudaEventRecord(h->ev[8], h->stream));
-    CK(cudaMemcpyAsync(h->h_counts, h->d_counts, 4 * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaMemcpyAsync(h->h_stats, h->d_stats, sizeof(DevStats), cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaMemcpyAsync(n_rec, h->d_rec_n, (size_t)B * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaStreamSynchronize(h->stream));
-    const int nrec = h->h_counts[2];
-    const int ncopy = std::min(nrec, rec_capacity);
-    if (ncopy > 0) {
-        CK(cudaMemcpyAsync(rec, h->d_rec, (size_t)ncopy * sizeof(ft8_record), cudaMemcpyDeviceToHost, h->stream));
-        CK(cudaStreamSynchronize(h->stream));
-    }
-    const bool overflow = nrec > rec_capacity;
-    if (overflow) {                       // records are cycle-major: trim the per-cycle counts to what was copied
-        int left = rec_capacity;
-        for (int b = 0; b < B; ++b) { const int t = std::min(n_rec[b], left); n_rec[b] = t; left -= t; }
-    }
-    const int64_t emitted = (int64_t)h->h_stats->emitted;
-    CK(cudaEventElapsedTime(&h->last_ms[0], h->ev[0], h->ev[8]));
-    for (int i = 1; i <= 8; ++i) CK(cudaEventElapsedTime(&h->last_ms[i], h->ev[i - 1], h->ev[i]));
-    h->last_ms[9] = h->last_ms[10] = h->last_ms[11] = 0.0f;
-    if (h->cfg.fine_mode == 0) {              // the three kernels of the fine stage: time scan, tensor-core frequency scan, final
-        CK(cudaEventElapsedTime(&h->last_ms[9], h->ev[4], h->ev[12]));
-        CK(cudaEventElapsedTime(&h->last_ms[10], h->ev[12], h->ev[13]));
-        CK(cudaEventElapsedTime(&h->last_ms[11], h->ev[13], h->ev[5]));
-    }
-    ft8_stats& s = h->stats;
-    memset(&s, 0, sizeof(s));
-    s.cycles = B; s.candidates = (int64_t)h->h_stats->candidates; s.stopped_sd = (int64_t)h->h_stats->stopped_sd;
-    s.fine_evals = (int64_t)h->h_stats->fine_evals; s.fine_pass = (int64_t)h->h_stats->fine_pass;
-    s.ldpc_calls = (int64_t)h->h_stats->ldpc_calls; s.ldpc_iters = (int64_t)h->h_stats->ldpc_iters;
-    s.osd_calls = (int64_t)h->h_stats->osd_calls; s.decoded = nrec; s.emitted = emitted; s.kernel_launches = launches;
-    s.fine_rechecked = h->cfg.fine_mode == 0 ? h->h_counts[3] : 0;
-    if (overflow) return fail(h, FT8_E_CAPACITY, "ft8_decode_cycles: rec_capacity too small (records truncated)");
-    return FT8_OK;
+    CK(cudaEventRecord(h->ev[EV_RECORDS], h->stream));
+    return finish_decode(h, B, rec, rec_capacity, n_rec, launches);
 }
 
 extern "C" int ft8_decode_cycles(ft8_handle* h, const void* audio, int audio_dtype, int B, int odd_even, ft8_record* rec,
@@ -1196,11 +1056,7 @@ extern "C" int ft8_decode_cycles_live(ft8_handle* h, const void* audio, int audi
 
 extern "C" int ft8_live_reset(ft8_handle* h) {
     ENTER(h);
-    if (h->d_ring) {
-        k_fill<<<h->n_sm * 8, 256, 0, h->stream>>>(h->d_ring, h->cap_cycles * (size_t)LIVE_ROWS * GRID_COLS, 1.0f);
-        CK(cudaGetLastError());
-        CK(cudaMemsetAsync(h->d_tail, 0, h->cap_cycles * (size_t)NFFT_S * sizeof(float), h->stream));
-    }
+    if (h->d_ring) TRY(clear_live(h));
     CK(cudaStreamSynchronize(h->stream));
     return FT8_OK;
 }
@@ -1217,20 +1073,19 @@ extern "C" int ft8_synth_cycles(ft8_handle* h, const uint8_t* symbols, const flo
     if (!symbols || !f_hz || !dt_s || !amp || !audio || B <= 0 || n_sig < 0 || n_sig > SYNTH_MAX_SIG)
         return fail(h, FT8_E_BADARG, "ft8_synth_cycles: bad argument (n_sig <= 128)");
     const size_t ns = (size_t)B * n_sig;
-    TRY(ensure_arena(h, ns * (79 + 12) + (mem == FT8_MEM_HOST ? (size_t)B * CYCLE_SAMPLES * 2 : 0) + 4096));
-    Carver c{(char*)h->arena};
-    uint8_t* dsym = c.take<uint8_t>(ns * 79); float* df = c.take<float>(ns); float* dd = c.take<float>(ns); float* dam = c.take<float>(ns);
-    int16_t* da = mem == FT8_MEM_HOST ? c.take<int16_t>((size_t)B * CYCLE_SAMPLES) : audio;
-    // parameters are small and always come from the host
+    uint8_t* dsym; float *df, *dd, *dam; int16_t* da;
+    Staging st(h, mem);
+    st.scratch(dsym, ns * 79); st.scratch(df, ns * 4); st.scratch(dd, ns * 4); st.scratch(dam, ns * 4);
+    st.out(da, audio, (size_t)B * CYCLE_SAMPLES * 2);
+    TRY(st.begin());
+    // parameters are small and always copied, from host or device memory
     CK(cudaMemcpyAsync(dsym, symbols, ns * 79, cudaMemcpyDefault, h->stream));
     CK(cudaMemcpyAsync(df, f_hz, ns * 4, cudaMemcpyDefault, h->stream));
     CK(cudaMemcpyAsync(dd, dt_s, ns * 4, cudaMemcpyDefault, h->stream));
     CK(cudaMemcpyAsync(dam, amp, ns * 4, cudaMemcpyDefault, h->stream));
     k_synth<<<dim3((CYCLE_SAMPLES + SYNTH_TILE - 1) / SYNTH_TILE, B), SYNTH_NT, 0, h->stream>>>(dsym, df, dd, dam, n_sig, noise_sigma, seed, h->d_pulse, da);
     CK(cudaGetLastError());
-    if (mem == FT8_MEM_HOST) TRY(from_device(h, audio, da, (size_t)B * CYCLE_SAMPLES * 2, mem));
-    CK(cudaStreamSynchronize(h->stream));
-    return FT8_OK;
+    return st.finish();
 }
 
 template <int N, int NT, bool INV>
@@ -1251,10 +1106,11 @@ extern "C" int ft8_debug_fft(ft8_handle* h, int n, int inverse, const float* in,
     ENTER(h);
     if (!in || !out || batch <= 0) return fail(h, FT8_E_BADARG, "ft8_debug_fft: bad argument");
     const size_t bytes = (size_t)batch * n * sizeof(float2);
-    TRY(ensure_arena(h, 2 * bytes + 512));
-    Carver c{(char*)h->arena};
-    float2* di = c.take<float2>((size_t)batch * n); float2* dout = c.take<float2>((size_t)batch * n);
-    TRY(to_device(h, di, in, bytes, FT8_MEM_HOST));
+    const float2* di; float2* dout;
+    Staging st(h, FT8_MEM_HOST);
+    st.in(di, in, bytes);
+    st.out(dout, out, bytes);
+    TRY(st.begin());
 #define DBG(NN, NT, WT)                                                                                                    \
     if (n == NN) {                                                                                                         \
         if (inverse) k_debug_fft<NN, NT, true><<<batch, NT, NN * sizeof(float2), h->stream>>>(di, dout, WT);               \
@@ -1264,9 +1120,7 @@ extern "C" int ft8_debug_fft(ft8_handle* h, int n, int inverse, const float* in,
     else DBG(32, 32, h->d_W32) else return fail(h, FT8_E_BADARG, "ft8_debug_fft: n must be 32, 256, 375, 1920 or 3200");
 #undef DBG
     CK(cudaGetLastError());
-    TRY(from_device(h, out, dout, bytes, FT8_MEM_HOST));
-    CK(cudaStreamSynchronize(h->stream));
-    return FT8_OK;
+    return st.finish();
 }
 
 #ifdef FS_PROFILE

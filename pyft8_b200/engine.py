@@ -239,6 +239,19 @@ class Engine:
         return flags
 
     # ---- whole path
+    def _outputs(self, B, rec, n):
+        """The record and count outputs of a decode of B cycles: new arrays, or the caller's after checking them (the library
+        writes up to len(rec) 64-byte records into `rec` and B int32 counts into `n`)."""
+        if rec is None:
+            rec = np.zeros(B * self.max_cands, L.RECORD_DTYPE)
+        elif rec.dtype != L.RECORD_DTYPE or not rec.flags.c_contiguous:
+            raise ValueError("rec must be a contiguous RECORD_DTYPE array")
+        if n is None:
+            n = np.zeros(B, np.int32)
+        elif n.dtype != np.int32 or len(n) < B or not n.flags.c_contiguous:
+            raise ValueError("n must be a contiguous int32 array of at least B entries")
+        return rec, n
+
     def decode_cycles(self, audio, odd_even=0, next_audio=None, rec=None, n=None):
         """audio [B,180000] int16/float32 -> (records structured array in emission order, n_rec[B]).
 
@@ -249,14 +262,7 @@ class Engine:
         underneath this batch's kernels and the next call consumes it (ft8_decode_cycles_stream)."""
         a, dt = self._audio(audio)
         B = a.shape[0]
-        if rec is None:
-            rec = np.zeros(B * self.max_cands, L.RECORD_DTYPE)
-        elif rec.dtype != L.RECORD_DTYPE or not rec.flags.c_contiguous:
-            raise ValueError("rec must be a contiguous RECORD_DTYPE array")
-        if n is None:
-            n = np.zeros(B, np.int32)
-        elif n.dtype != np.int32 or len(n) < B or not n.flags.c_contiguous:
-            raise ValueError("n must be a contiguous int32 array of at least B entries")
+        rec, n = self._outputs(B, rec, n)
         cap = len(rec)
         pending = getattr(self, "_pf_ref", None)
         # a prefetched copy is consumed only through the streaming entry, and only for the very array that was named
@@ -280,10 +286,7 @@ class Engine:
         Alternate odd_even 0, 1, 0, ... call after call; live_reset() forgets the history."""
         a, dt = self._audio(audio)
         B = a.shape[0]
-        if rec is None:
-            rec = np.zeros(B * self.max_cands, L.RECORD_DTYPE)
-        if n is None:
-            n = np.zeros(B, np.int32)
+        rec, n = self._outputs(B, rec, n)
         self._check(self._lib.ft8_decode_cycles_live(self._h, _ptr(a), dt, B, int(odd_even), _ptr(rec), len(rec), _ptr(n), L.MEM_HOST))
         return rec[:int(n[:B].sum())], n[:B]
 
@@ -299,11 +302,7 @@ class Engine:
 
     def decode_cycles_dev(self, audio_ptr, dtype, B, odd_even=0, rec=None, n=None):
         """Same, with audio already resident on this engine's device (raw pointer)."""
-        cap = B * self.max_cands
-        if rec is None:
-            rec = np.zeros(cap, L.RECORD_DTYPE)
-        if n is None:
-            n = np.zeros(B, np.int32)
+        rec, n = self._outputs(B, rec, n)
         self._check(self._lib.ft8_decode_cycles(self._h, C.c_void_p(audio_ptr), dtype, B, int(odd_even), _ptr(rec), len(rec),
                                                 _ptr(n), L.MEM_DEVICE))
         return rec[:int(n[:B].sum())], n[:B]
