@@ -131,6 +131,7 @@ void* ft8_stream(ft8_handle* h);
  * 5 fine sync, 6 passes 2-4 (LDPC), 7 passes 5-6 (OSD), 8 record collection, 9 / 10 / 11 the three kernels of the fine stage
  * (time scan, tensor-core frequency scan, final transform; 0 with fine_mode 1).  Host audio of more than 256 cycles that was
  * not prefetched is copied and processed in chunks: then 1 covers the whole front end (1-3) and 2 and 3 are 0.
+ * After ft8_decode_cycles_live_seq: 0 = the whole call (all its pieces), 1-11 = the sums of those entries over the pieces.
  * After a stand-alone ft8_spectrogram / ft8_sync call: 1 / 2 = that kernel.  After ft8_ldpc / ft8_osd: 0 = that kernel. */
 int  ft8_last_kernel_ms(ft8_handle* h, int which, float* ms);
 
@@ -195,6 +196,20 @@ int ft8_decode_cycles(ft8_handle* h, const void* audio, int audio_dtype, int B, 
 int ft8_decode_cycles_live(ft8_handle* h, const void* audio, int audio_dtype, int B, int odd_even,
                            ft8_record* rec, int rec_capacity, int32_t* n_rec, int mem);
 int ft8_live_reset(ft8_handle* h);
+
+/* C consecutive live cycles of B streams in one call.  audio is [C][B][180000] (time-major: audio + c*B*180000 is the
+ * batch a c-th ft8_decode_cycles_live call would get), so one stream's recording (B = 1) is one contiguous array.
+ * Equivalent to, and bit-identical with:
+ *     for c in 0..C-1: ft8_decode_cycles_live(h, audio + c*B*180000, audio_dtype, B, odd_even ^ (c & 1), ...)
+ * records concatenated in that order, n_rec[C][B], and ft8_record.cycle = c*B + b.  The handle's live state (both ring
+ * halves and the tail of each stream b < B) is left exactly as those C calls leave it, so ft8_decode_cycles_live and this
+ * entry can follow each other in any order.  C*B may exceed cfg.max_cycles; B may not (FT8_E_CAPACITY).  The call works in
+ * pieces of floor(max_cycles / B) consecutive cycles per stream, each one decode batch.  When rec_capacity is too small,
+ * all C cycles are still decoded and the live state still advances past them; records beyond rec_capacity are dropped
+ * cycle-major (n_rec trimmed to what was copied) and the call returns FT8_E_CAPACITY.  ft8_get_stats gives totals over the
+ * call; ft8_last_kernel_ms: 0 = the whole call, 1-11 summed over the pieces. */
+int ft8_decode_cycles_live_seq(ft8_handle* h, const void* audio, int audio_dtype, int B, int C, int odd_even,
+                               ft8_record* rec, int rec_capacity, int32_t* n_rec, int mem);
 
 /* Optional double buffering for callers that stream batches from host memory: starts the host->device copy of the NEXT
  * batch on a second stream and returns at once.  The host buffer must stay valid and UNCHANGED until the copy has been

@@ -102,6 +102,8 @@ struct ft8_handle {
     // live mode (ft8_decode_cycles_live): the reference's two-cycle waterfall ring per stream + the previous cycle's last window
     // (float32 whatever the input dtype; zero for a stream that has no previous cycle)
     DevBuf<float> d_ring, d_tail;
+    // consecutive live cycles (ft8_decode_cycles_live_seq): one SEQ_ROWS-row grid and one previous-cycle tail per cycle of a piece
+    DevBuf<float> d_seq_grid, d_seq_tail;
     DevBuf<float2> d_Y; size_t y_cycles = 0;
     DevBuf<float2> d_spec;
     DevBuf<float> d_best_score; DevBuf<int16_t> d_best_h0;
@@ -491,9 +493,9 @@ static int launch_spectrogram(ft8_handle* h, const void* d_audio, int dtype, int
     return FT8_OK;
 }
 
-// d_grid points at the first of the B cycles; b0 = index of that cycle in the handle's per-cycle arrays
-static int launch_sync(ft8_handle* h, const float* d_grid, int grid_rows, int B, int odd_even, int b0 = 0) {
-    const int cycle_h0 = odd_even ? 375 : 0;
+// d_grid points at the first of the B cycles; b0 = index of that cycle in the handle's per-cycle arrays; cycle_h0 = grid row
+// of the cycle's hop 0
+static int launch_sync(ft8_handle* h, const float* d_grid, int grid_rows, int B, int cycle_h0, int b0 = 0) {
     const size_t K = h->cfg.max_cands;
     k_sync_scores<<<dim3(SY_HS * (N_F0 / SY_TF), B), SY_NT, SY_SMEM_BYTES, h->stream>>>(
         d_grid, grid_rows, cycle_h0, h->d_best_score + (size_t)b0 * N_F0 * SY_HS, h->d_best_h0 + (size_t)b0 * N_F0 * SY_HS,
@@ -683,7 +685,7 @@ extern "C" int ft8_sync(ft8_handle* h, const float* grid_db, int grid_rows, int 
     CK(cudaMemsetAsync(h->d_h0, 0, N * 2, h->stream));
     CK(cudaMemsetAsync(h->d_score, 0, N * 4, h->stream));
     CK(cudaEventRecord(h->ev[EV_OP_BEGIN], h->stream));
-    TRY(launch_sync(h, dg, grid_rows, B, odd_even));
+    TRY(launch_sync(h, dg, grid_rows, B, odd_even ? 375 : 0));
     CK(cudaEventRecord(h->ev[EV_OP_END], h->stream));
     if (payload_db) {
         CK(cudaMemsetAsync(d_pay, 0, N * 58 * 8 * sizeof(float), h->stream));
@@ -851,10 +853,72 @@ __global__ void k_save_tails(const T* __restrict__ audio, float* __restrict__ ta
     for (int i = threadIdx.x; i < NFFT_S; i += blockDim.x) t[i] = (float)x[i];
 }
 
-static int save_tails(ft8_handle* h, const void* d_audio, int dtype, int B) {
-    if (dtype == FT8_AUDIO_I16) k_save_tails<<<B, 256, 0, h->stream>>>((const int16_t*)d_audio, h->d_tail);
-    else k_save_tails<<<B, 256, 0, h->stream>>>((const float*)d_audio, h->d_tail);
+static int save_tails(ft8_handle* h, const void* d_audio, int dtype, int B, float* d_tail) {
+    if (dtype == FT8_AUDIO_I16) k_save_tails<<<B, 256, 0, h->stream>>>((const int16_t*)d_audio, d_tail);
+    else k_save_tails<<<B, 256, 0, h->stream>>>((const float*)d_audio, d_tail);
     CK(cudaGetLastError());
+    return FT8_OK;
+}
+
+// Consecutive live cycles (ft8_decode_cycles_live_seq) are decoded in pieces: `steps` cycle steps of `streams` streams, one
+// batch of steps * streams cycles, cycle i = step * streams + stream, the first step of parity `parity`.  Each cycle gets a
+// SEQ_ROWS-row grid: rows 0..5 are the previous cycle's hops 370..375, rows 6..380 its own hops 1..375.  The search runs on
+// it with cycle_h0 = SEQ_H0, so row SEQ_H0 + d holds what the live ring holds at 375 p + d: the sync search reads d in
+// 111..258, payload rows d = h0 + 4 + 4 s lie in [-5, 374], and d <= 0 is the previous cycle's hop 375 + d.
+struct SeqPiece { int streams, steps, parity; };
+constexpr int SEQ_BOUND = 6, SEQ_H0 = SEQ_BOUND - 1, SEQ_ROWS = SEQ_BOUND + 375;
+constexpr int ROW_F4 = GRID_COLS / 4;           // a grid row as float4 (3904 bytes: every row starts 16-byte aligned)
+
+// Rows 0..5 of cycles b0 .. b0 + gridDim.y - 1 of a piece: for a cycle after the piece's first step, rows 375..380 of the same
+// stream's cycle one step earlier (its hops 370..375); for the first step, the ring rows (375 p + d) mod 750, d = -5..0, that
+// a live call of parity p reads there.  Runs after S1 has written the own rows of those cycles.
+__global__ void k_seq_boundary(float* grid, const float* __restrict__ ring, int streams, int b0, int parity) {
+    const int i = b0 + blockIdx.y, r = blockIdx.x;
+    const float* src = i >= streams ? grid + ((size_t)(i - streams) * SEQ_ROWS + 375 + r) * GRID_COLS
+                                    : ring + ((size_t)i * LIVE_ROWS + (375 * parity + r - SEQ_H0 + LIVE_ROWS) % LIVE_ROWS) * GRID_COLS;
+    const float4* s = reinterpret_cast<const float4*>(src);
+    float4* d = reinterpret_cast<float4*>(grid + ((size_t)i * SEQ_ROWS + r) * GRID_COLS);
+    for (int k = threadIdx.x; k < ROW_F4; k += blockDim.x) d[k] = s[k];
+}
+
+// Ring write-back of gridDim.y / streams consecutive steps (grid points at the first, of parity `parity`): ring row
+// (375 p + h) mod 750 <- grid row SEQ_H0 + h, h = 1..375 -- the half a live call of that step would have written.
+__global__ void k_seq_store_ring(const float* __restrict__ grid, float* __restrict__ ring, int streams, int parity) {
+    const int j = blockIdx.y, hop = blockIdx.x + 1;
+    const int b = j % streams, p = parity ^ ((j / streams) & 1);
+    const float4* s = reinterpret_cast<const float4*>(grid + ((size_t)j * SEQ_ROWS + SEQ_H0 + hop) * GRID_COLS);
+    float4* d = reinterpret_cast<float4*>(ring + ((size_t)b * LIVE_ROWS + (375 * p + hop) % LIVE_ROWS) * GRID_COLS);
+    for (int k = threadIdx.x; k < ROW_F4; k += blockDim.x) d[k] = s[k];
+}
+
+// Front end of cycles b0 .. b0 + nb - 1 of a piece (d_audio = the whole piece): their tails (the last 3840 samples of the same
+// stream one step earlier; the piece's first step has its tails copied from d_tail already), S1 into rows 6..380 and the
+// boundary rows.  Adds its kernel launches other than S1 to *launches.
+static int seq_front(ft8_handle* h, const SeqPiece& sp, const char* d_audio, int dtype, int b0, int nb, int* launches) {
+    const size_t esz = sample_bytes(dtype);
+    const int lo = std::max(b0, sp.streams), hi = b0 + nb;
+    if (lo < hi) {
+        TRY(save_tails(h, d_audio + (size_t)(lo - sp.streams) * CYCLE_SAMPLES * esz, dtype, hi - lo, h->d_seq_tail + (size_t)lo * NFFT_S));
+        ++*launches;
+    }
+    float* g = h->d_seq_grid + (size_t)b0 * SEQ_ROWS * GRID_COLS;
+    TRY(launch_spectrogram(h, d_audio + (size_t)b0 * CYCLE_SAMPLES * esz, dtype, nb, g, 1, 375, SEQ_ROWS, -SEQ_H0, 0,
+                           h->d_seq_tail + (size_t)b0 * NFFT_S, 0));
+    k_seq_boundary<<<dim3(SEQ_BOUND, nb), 256, 0, h->stream>>>(h->d_seq_grid, h->d_ring, sp.streams, b0, sp.parity);
+    CK(cudaGetLastError());
+    ++*launches;
+    return FT8_OK;
+}
+
+// After the piece's kernels: the ring halves of its last two steps (one when it has one step; the half before that was
+// written by the previous piece or call) and every stream's tail, as the live calls of those steps leave them.
+static int seq_store(ft8_handle* h, const SeqPiece& sp, const char* d_audio, int dtype, int* launches) {
+    const int last = sp.steps - 1, first = std::max(0, last - 1);
+    TRY(save_tails(h, d_audio + (size_t)last * sp.streams * CYCLE_SAMPLES * sample_bytes(dtype), dtype, sp.streams, h->d_tail));
+    k_seq_store_ring<<<dim3(375, (last - first + 1) * sp.streams), 256, 0, h->stream>>>(
+        h->d_seq_grid + (size_t)first * sp.streams * SEQ_ROWS * GRID_COLS, h->d_ring, sp.streams, sp.parity ^ (first & 1));
+    CK(cudaGetLastError());
+    *launches += 2;
     return FT8_OK;
 }
 
@@ -934,7 +998,7 @@ static int finish_decode(ft8_handle* h, int B, ft8_record* rec, int rec_capacity
 
 static int decode_cycles_core(ft8_handle* h, const void* audio, int audio_dtype, int B, int odd_even, ft8_record* rec,
                               int rec_capacity, int32_t* n_rec, int mem, const void* next_audio_host, bool consume_pf,
-                              bool live = false) {
+                              bool live = false, const SeqPiece* seq = nullptr) {
     ENTER(h);
     if (!audio || !rec || !n_rec || B <= 0 || rec_capacity < 0) return fail(h, FT8_E_BADARG, "ft8_decode_cycles: bad argument");
     if ((size_t)B > h->cap_cycles) return fail(h, FT8_E_CAPACITY, "ft8_decode_cycles: B exceeds cfg.max_cycles");
@@ -944,18 +1008,25 @@ static int decode_cycles_core(ft8_handle* h, const void* audio, int audio_dtype,
     // Live mode: stream b keeps the reference's 750-row two-cycle ring (receiver.py:238, 295-306); this call's rows go to the
     // half odd_even selects, rows of the other half still hold the previous cycle, and the first hops' windows reach back into
     // the previous cycle's last samples -- so candidates with h0 < -32 read real rows, exactly as a live Receiver does.
+    // Consecutive live cycles (seq): one piece of ft8_decode_cycles_live_seq on SEQ_ROWS-row grids (see SeqPiece), chained
+    // to the calls before and after it through the same ring and tails.
     TRY(check_dtype(h, audio_dtype));
     const size_t esz = sample_bytes(audio_dtype);
-    const int cycle_h0 = live ? (odd_even ? 375 : 0) : 0;
-    const int grows = live ? LIVE_ROWS : GRID_ROWS;
+    const int cycle_h0 = seq ? SEQ_H0 : live ? (odd_even ? 375 : 0) : 0;
+    const int grows = seq ? SEQ_ROWS : live ? LIVE_ROWS : GRID_ROWS;
     float* gbase = h->d_grid;
-    if (live) {
+    if (live || seq) {
         if (!h->d_ring) {
             CK(h->d_ring.ensure(h->cap_cycles * (size_t)LIVE_ROWS * GRID_COLS, h->stream));
             CK(h->d_tail.ensure(h->cap_cycles * (size_t)NFFT_S, h->stream));
             TRY(clear_live(h));
         }
         gbase = h->d_ring;
+    }
+    if (seq) {
+        CK(h->d_seq_grid.ensure(h->cap_cycles * (size_t)SEQ_ROWS * GRID_COLS, h->stream));
+        CK(h->d_seq_tail.ensure(h->cap_cycles * (size_t)NFFT_S, h->stream));
+        gbase = h->d_seq_grid;
     }
     const void* da;
     bool prefetched;
@@ -968,6 +1039,8 @@ static int decode_cycles_core(ft8_handle* h, const void* audio, int audio_dtype,
     CK(cudaMemsetAsync(h->d_counts, 0, CNT_SLOTS * sizeof(int32_t), h->stream));
     CK(cudaMemsetAsync(h->d_stats, 0, sizeof(DevStats), h->stream));
     CK(cudaEventRecord(h->ev[EV_START], h->stream));
+    if (seq) CK(cudaMemcpyAsync(h->d_seq_tail, h->d_tail, (size_t)seq->streams * NFFT_S * sizeof(float), cudaMemcpyDeviceToDevice,
+                                h->stream));           // the tails of the piece's first step
     // Front end (S1, S2, F1) chunk by chunk.  Host audio is copied on the copy stream in up to 16 equal chunks, and a chunk's
     // kernels start as soon as it has landed, so the PCIe transfer hides behind the front end of the chunks before it
     // (measured best for a single handle: 28.6 k cycles/s vs 27.3-28.0 k for growing chunks); callers that stream batch
@@ -990,11 +1063,12 @@ static int decode_cycles_core(ft8_handle* h, const void* audio, int audio_dtype,
         const char* a = (const char*)da + (size_t)b0 * CYCLE_SAMPLES * esz;
         if (copy) CK(cudaStreamWaitEvent(h->stream, h->chunk_ev[c], 0));
         float* gc = gbase + (size_t)b0 * grows * GRID_COLS;
-        if (live) TRY(launch_spectrogram(h, a, audio_dtype, nb, gc, 1, 375, LIVE_ROWS, -cycle_h0, 0, h->d_tail + (size_t)b0 * NFFT_S, 1));
+        if (seq) TRY(seq_front(h, *seq, (const char*)da, audio_dtype, b0, nb, &launches));
+        else if (live) TRY(launch_spectrogram(h, a, audio_dtype, nb, gc, 1, 375, LIVE_ROWS, -cycle_h0, 0, h->d_tail + (size_t)b0 * NFFT_S, 1));
         else TRY(launch_spectrogram(h, a, audio_dtype, nb, gc));
         ++launches;
         if (nchunk == 1) CK(cudaEventRecord(h->ev[EV_SPECTROGRAM], h->stream));
-        TRY(launch_sync(h, gc, grows, nb, live ? odd_even : 0, b0)); launches += 2;
+        TRY(launch_sync(h, gc, grows, nb, cycle_h0, b0)); launches += 2;
         if (nchunk == 1) CK(cudaEventRecord(h->ev[EV_SYNC], h->stream));
         // F1 (independent of S1/S2; same stream)
         TRY(launch_cycle_spectrum(h, a, audio_dtype, nb, h->d_spec + (size_t)b0 * FINE_SPEC_STRIDE, FINE_SPEC_STRIDE, FINE_SPEC_STRIDE - 1));
@@ -1006,7 +1080,8 @@ static int decode_cycles_core(ft8_handle* h, const void* audio, int audio_dtype,
     }
     CK(cudaEventRecord(h->ev[EV_CYCLE_SPECTRUM], h->stream));
     if (next_audio_host && !prefetched) TRY(ft8_prefetch_audio(h, next_audio_host, audio_dtype, B));
-    if (live) { TRY(save_tails(h, da, audio_dtype, B)); ++launches; }   // after S1 has read the old tails
+    if (seq) TRY(seq_store(h, *seq, (const char*)da, audio_dtype, &launches));
+    else if (live) { TRY(save_tails(h, da, audio_dtype, B, h->d_tail)); ++launches; }   // after S1 has read the old tails
     CandState cs = cand_state(h);
     // ipass 0
     k_pass0<<<persistent_blocks(h, 8), WARPS_PER_CTA * 32, sizeof(PassSmem), h->stream>>>(
@@ -1052,6 +1127,53 @@ extern "C" int ft8_decode_cycles_live(ft8_handle* h, const void* audio, int audi
                                       int rec_capacity, int32_t* n_rec, int mem) {
     if (odd_even != 0 && odd_even != 1) return fail(h, FT8_E_BADARG, "ft8_decode_cycles_live: odd_even must be 0 or 1");
     return decode_cycles_core(h, audio, audio_dtype, B, odd_even, rec, rec_capacity, n_rec, mem, nullptr, false, true);
+}
+
+// C steps of B streams in pieces of floor(max_cycles / B) steps; each piece is one decode batch.  Records of a piece land after
+// those of the pieces before it (cycle-major, so the capacity cut of finish_decode stays cycle-major over the whole call);
+// their cycle index is the piece's local one and is shifted here.
+extern "C" int ft8_decode_cycles_live_seq(ft8_handle* h, const void* audio, int audio_dtype, int B, int C, int odd_even,
+                                          ft8_record* rec, int rec_capacity, int32_t* n_rec, int mem) {
+    ENTER(h);
+    if (odd_even != 0 && odd_even != 1) return fail(h, FT8_E_BADARG, "ft8_decode_cycles_live_seq: odd_even must be 0 or 1");
+    if (!audio || !rec || !n_rec || B <= 0 || C <= 0 || rec_capacity < 0)
+        return fail(h, FT8_E_BADARG, "ft8_decode_cycles_live_seq: bad argument");
+    if ((size_t)B > h->cap_cycles) return fail(h, FT8_E_CAPACITY, "ft8_decode_cycles_live_seq: B exceeds cfg.max_cycles");
+    TRY(check_dtype(h, audio_dtype));
+    const int per = (int)(h->cap_cycles / B);
+    const size_t step_bytes = (size_t)B * CYCLE_SAMPLES * sample_bytes(audio_dtype);
+    ft8_stats total{};
+    float ms[MS_COUNT] = {};
+    int written = 0;
+    bool overflow = false;
+    CK(cudaEventRecord(h->ev[EV_OP_BEGIN], h->stream));
+    for (int c0 = 0; c0 < C; c0 += per) {
+        const SeqPiece sp{B, std::min(per, C - c0), odd_even ^ (c0 & 1)};
+        const int nb = sp.steps * B;
+        ft8_record* r = rec + written;
+        int32_t* n = n_rec + (size_t)c0 * B;
+        const int rc = decode_cycles_core(h, (const char*)audio + (size_t)c0 * step_bytes, audio_dtype, nb, sp.parity, r,
+                                          rec_capacity - written, n, mem, nullptr, false, false, &sp);
+        if (rc != FT8_OK && rc != FT8_E_CAPACITY) return rc;
+        overflow = overflow || rc == FT8_E_CAPACITY;
+        int got = 0;
+        for (int i = 0; i < nb; ++i) got += n[i];
+        for (int i = 0; i < got; ++i) r[i].cycle += c0 * B;
+        written += got;
+        const ft8_stats& s = h->stats;
+        total.cycles += s.cycles; total.candidates += s.candidates; total.stopped_sd += s.stopped_sd;
+        total.fine_evals += s.fine_evals; total.fine_pass += s.fine_pass; total.ldpc_calls += s.ldpc_calls;
+        total.ldpc_iters += s.ldpc_iters; total.osd_calls += s.osd_calls; total.decoded += s.decoded; total.emitted += s.emitted;
+        total.kernel_launches += s.kernel_launches; total.fine_rechecked += s.fine_rechecked;
+        for (int i = MS_SPECTROGRAM; i < MS_COUNT; ++i) ms[i] += h->last_ms[i];
+    }
+    CK(cudaEventRecord(h->ev[EV_OP_END], h->stream));
+    CK(cudaEventSynchronize(h->ev[EV_OP_END]));
+    CK(cudaEventElapsedTime(&ms[MS_TOTAL], h->ev[EV_OP_BEGIN], h->ev[EV_OP_END]));
+    h->stats = total;
+    memcpy(h->last_ms, ms, sizeof(ms));
+    if (overflow) return fail(h, FT8_E_CAPACITY, "ft8_decode_cycles_live_seq: rec_capacity too small (records truncated)");
+    return FT8_OK;
 }
 
 extern "C" int ft8_live_reset(ft8_handle* h) {

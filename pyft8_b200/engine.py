@@ -290,6 +290,28 @@ class Engine:
         self._check(self._lib.ft8_decode_cycles_live(self._h, _ptr(a), dt, B, int(odd_even), _ptr(rec), len(rec), _ptr(n), L.MEM_HOST))
         return rec[:int(n[:B].sum())], n[:B]
 
+    def decode_cycles_live_seq(self, audio, odd_even, rec=None, n=None):
+        """C consecutive live cycles of B streams in one call (ft8_decode_cycles_live_seq): audio [C, B, 180000], or
+        [C, 180000] for one stream, int16/float32, cycle c of parity odd_even ^ (c & 1).  Bit-identical with C
+        decode_cycles_live calls, and leaves the same live state.  Returns (records, n[C, B]); a record's `cycle` is c*B + b.
+        `n`, when given, is a flat int32 array of at least C*B entries."""
+        a = np.ascontiguousarray(audio)
+        if a.ndim == 2:
+            a = a[:, None, :]
+        if a.ndim != 3 or a.shape[2] != 180000 or a.shape[0] == 0 or a.shape[1] == 0:
+            raise ValueError("audio must be [C, B, 180000] or [C, 180000] (C consecutive 15 s cycles of B streams)")
+        if a.dtype == np.int16:
+            dt = L.AUDIO_I16
+        elif a.dtype == np.float32:
+            dt = L.AUDIO_F32
+        else:
+            raise ValueError("audio dtype must be int16 or float32")
+        C_, B = a.shape[:2]
+        rec, n = self._outputs(C_ * B, rec, n)
+        self._check(self._lib.ft8_decode_cycles_live_seq(self._h, _ptr(a), dt, B, C_, int(odd_even), _ptr(rec), len(rec), _ptr(n),
+                                                         L.MEM_HOST))
+        return rec[:int(n[:C_ * B].sum())], n[:C_ * B].reshape(C_, B)
+
     def live_reset(self):
         self._check(self._lib.ft8_live_reset(self._h))
 

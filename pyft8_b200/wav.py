@@ -38,18 +38,22 @@ def write_wav(path, audio):
 
 def decode_wav(path, receiver=None, live=False, **kw):
     """Decode a recording: list (per 15 s cycle) of message dicts.  live=True keeps the two-cycle waterfall ring across the
-    recording's consecutive cycles (Engine.decode_cycles_live) instead of decoding each cycle in isolation."""
+    recording's consecutive cycles (Engine.decode_cycles_live_seq, the first cycle even) instead of decoding each cycle in
+    isolation."""
     from .receiver import Receiver, format_records
     audio = read_wav(path)
     rx = receiver or Receiver("", None, **kw)
     if not live:
         return rx.decode_cycles(audio, emit=False)
     from .engine import Engine
-    eng = Engine(device=rx._device, max_cycles=1, max_cands=rx.max_cands, sync_score_min=rx.sync_score_min)
-    out = []
-    for i in range(len(audio)):
-        rec, _ = eng.decode_cycles_live(audio[i], i & 1)
-        mb = format_records(rec)
-        out.append([t for t, k in zip(mb.text.tolist(), mb.keep.tolist()) if k])
+    # the library decodes the recording in pieces of max_cycles cycles, chained through the live state
+    eng = Engine(device=rx._device, max_cycles=min(len(audio), 256), max_cands=rx.max_cands, sync_score_min=rx.sync_score_min)
+    rec, n = eng.decode_cycles_live_seq(audio, 0)
     eng.close()
+    out, off = [], 0
+    for k in n[:, 0].tolist():
+        # one cycle per unpacking batch, like a live receiver, so that hashed calls ('<...>') resolve as they do there
+        mb = format_records(rec[off:off + k])
+        off += k
+        out.append([t for t, keep in zip(mb.text.tolist(), mb.keep.tolist()) if keep])
     return out
