@@ -474,30 +474,30 @@ def _try_ldpc(c, ap, nc0, its, save):
             c.saved.append((f"{AP_PATTERNS[ap][0]}_LDPC{its}", c.llr))
 
 
-def _try_osd(c, name):
+def _try_osd(c, name, singleflips=30, doubleflips=2):
     if c.result is None:
         c.notes = f"{c.source}_{name}_OSD"
         c.n_osd += 1
-        b = osd(c.llr)
+        b = osd(c.llr, singleflips, doubleflips)     # osd_012(singleflips, doubleflips), decoders.py:223
         if b is not None:
             c.result, c.bits91 = "ok", b
 
 
-def _set_llr(c, p):
+def _set_llr(c, p, llr_sd_min=5):
     with np.errstate(all="ignore"):
         c.llr, c.llr_sd, c.snr = db_to_llr(p)
-    if c.llr_sd <= 5:                      # receiver.py:221-222
+    if c.llr_sd <= llr_sd_min:             # Candidate(llr_sd_min), receiver.py:221-222
         c.result = "stop"
 
 
-def decode_step(c, spec):
+def decode_step(c, spec, llr_sd_min=5, osd_singleflips=30, osd_doubleflips=2):
     """Advance one candidate by one pass.  receiver.py:68-107."""
     if c.result == "stop":
         return
     ip = c.ipass
     if ip == 0:
         c.source = "grid"
-        _set_llr(c, c.payload)
+        _set_llr(c, c.payload, llr_sd_min)
         c.grid_sd = float(c.llr_sd)
         c.llr0 = c.llr.copy()
         for ap in range(5):
@@ -513,7 +513,7 @@ def decode_step(c, spec):
             c.tsec = float(c.tsec + r["tt"] / 200)
             c.fHz = float(c.fHz + r["ff"] / 16)
             with np.errstate(all="ignore"):
-                _set_llr(c, 20 * np.log10(r["grid"][list(PAYLOAD_SYMS), :]))
+                _set_llr(c, 20 * np.log10(r["grid"][list(PAYLOAD_SYMS), :]), llr_sd_min)
             c.fine_sd = float(c.llr_sd)
         else:
             c.result = "stop"
@@ -533,18 +533,22 @@ def decode_step(c, spec):
     elif ip == 5:
         for ap in range(5):
             c.llr = set_ap(c.llr0, ap)
-            _try_osd(c, AP_PATTERNS[ap][0])
+            _try_osd(c, AP_PATTERNS[ap][0], osd_singleflips, osd_doubleflips)
     elif ip == 6:
         for name, llr in c.saved:
             c.llr = llr
-            _try_osd(c, name)
+            _try_osd(c, name, osd_singleflips, osd_doubleflips)
     elif ip == 7:
         c.result = "stop"
     c.ipass += 1
 
 
-def decode_cycle(audio_i16, score_min=85, max_cands=200, odd_even=0, grid=None, cands=None):
+def decode_cycle(audio_i16, score_min=85, max_cands=200, odd_even=0, grid=None, cands=None, llr_sd_min=5,
+                 osd_singleflips=30, osd_doubleflips=2):
     """Whole path for one isolated cycle.  Mirrors receiver.py:389-398 without time starvation.
+
+    llr_sd_min: Candidate(llr_sd_min) (receiver.py:221-222); osd_singleflips / osd_doubleflips: osd_012(singleflips,
+    doubleflips) (decoders.py:223).  The defaults are the reference's.
 
     Returns (records, cands): ``records`` are the emitted decodes in emission order, each a dict
     with bits77, bits91, tsec, fHz, snr, notes (pass name + tweaks), cand index.  Emission de-dup
@@ -578,7 +582,7 @@ def decode_cycle(audio_i16, score_min=85, max_cands=200, odd_even=0, grid=None, 
             if c.ipass == 1 and spec is None:
                 spec = cycle_spectrum(audio_i16)
             ip = c.ipass
-            decode_step(c, spec)
+            decode_step(c, spec, llr_sd_min, osd_singleflips, osd_doubleflips)
             if c.result is not None:
                 c.final_ipass = ip
             if c.result == "ok":
@@ -589,6 +593,21 @@ def decode_cycle(audio_i16, score_min=85, max_cands=200, odd_even=0, grid=None, 
                                         notes=c.notes + c.tweaks, cand=c.idx, ipass=ip))
                 c.result = "stop"
     return records, cl
+
+
+def work_counters(cl):
+    """The library's per-call work counters (ft8_stats) of one decoded cycle's Cand list, counted as the kernels count:
+
+    candidates  every candidate                                  stopped_sd  stopped by the ipass-0 sd gate
+    fine_evals  candidates that reach ipass 1 (fine sync)        fine_pass   candidates that reach ipass 2
+    ldpc_calls  every LDPC decode (iteration-0 rejects included)
+    osd_calls   5 + len(saved) per candidate that reaches ipass 5: the library runs all of a candidate's OSD attempts and
+                then takes the first success in reference order, where the oracle's own n_osd stops at the first success.
+    """
+    # every candidate ends in some pass (final_ipass); one that ends in ipass 0 undecoded was stopped by the sd gate
+    return dict(candidates=len(cl), stopped_sd=sum(c.final_ipass == 0 and c.bits91 is None for c in cl),
+                fine_evals=sum(c.final_ipass >= 1 for c in cl), fine_pass=sum(c.final_ipass >= 2 for c in cl),
+                ldpc_calls=sum(c.n_ldpc for c in cl), osd_calls=sum(5 + len(c.saved) for c in cl if c.final_ipass >= 5))
 
 
 # --------------------------------------------------------------------------- message text (host side)

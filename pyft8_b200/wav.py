@@ -47,7 +47,8 @@ def decode_wav(path, receiver=None, live=False, **kw):
         return rx.decode_cycles(audio, emit=False)
     from .engine import Engine
     # the library decodes the recording in pieces of max_cycles cycles, chained through the live state
-    eng = Engine(device=rx._device, max_cycles=min(len(audio), 256), max_cands=rx.max_cands, sync_score_min=rx.sync_score_min)
+    eng = Engine(device=rx._device, max_cycles=min(len(audio), 256), max_cands=rx.max_cands, sync_score_min=rx.sync_score_min,
+                 search_f0_range=rx._search_ranges[0], search_h0_range=rx._search_ranges[1])
     rec, n = eng.decode_cycles_live_seq(audio, 0)
     eng.close()
     out, off = [], 0
