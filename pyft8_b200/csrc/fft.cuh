@@ -16,20 +16,13 @@
 
 namespace ft8 {
 
-// ---- complex helpers.  Two implementations with the SAME rounding sequence (products rounded once, fma exactly where
-// the formulas quoted below have fmaf), so they produce bit-identical results:
-//   * default: Blackwell packed fp32x2 (FFMA2 / FADD2 / FMUL2, one instruction per complex number; ptxas folds operand
-//     swaps, scalar broadcasts and per-half sign changes into modifiers such as R.F32x2.LO_HI.NP / R.F32, so a complex
-//     multiply is 2 instructions and a multiply by +-i inside an add is free);
-//   * -DFT8_SCALAR_F32: plain FFMA / FADD / FMUL.
-// Measured on B200 (tools/micro/ffma2_bench.cu, tools/variant_bench.py): FFMA2 sustains the FFMA flop rate with half the
-// issue slots (72 Tflop/s either way).  While the FFT kernels were bound by the shared-memory / L1 pipe the packed build
-// gained nothing (k_fine even lost 1 %); after the twiddle-table and pass-fusion work it is 2 % faster on the whole step
-// (k_spectrogram 8.15 -> 7.91 ms, k_fine 54.0 -> 52.0 ms), records bit-identical.
-#ifndef FT8_SCALAR_F32
-#define FT8_PACKED_F32X2 1
-#endif
-#ifdef FT8_PACKED_F32X2
+// ---- complex helpers on Blackwell packed fp32x2 (FFMA2 / FADD2 / FMUL2, one instruction per complex number; ptxas folds
+// operand swaps, scalar broadcasts and per-half sign changes into modifiers such as R.F32x2.LO_HI.NP / R.F32, so a
+// complex multiply is 2 instructions and a multiply by +-i inside an add is free).  Each half rounds like the scalar
+// instruction (products rounded once, fma exactly where the formulas below have fmaf).
+// Why packed, measured on B200 (tools/micro/ffma2_bench.cu, tools/variant_bench.py): FFMA2 sustains the FFMA flop rate
+// with half the issue slots (72 Tflop/s either way); against plain FFMA / FADD / FMUL the packed build is 2 % faster on
+// the whole step (k_spectrogram 8.15 -> 7.91 ms, k_fine 54.0 -> 52.0 ms), records bit-identical.
 typedef unsigned long long u64;
 __device__ __forceinline__ u64 pk(float lo, float hi) { u64 r; asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi)); return r; }
 __device__ __forceinline__ u64 P(float2 a) { return pk(a.x, a.y); }
@@ -40,14 +33,18 @@ __device__ __forceinline__ u64 add2(u64 a, u64 b) { u64 d; asm("add.rn.f32x2 %0,
 __device__ __forceinline__ u64 sub2(u64 a, u64 b) { u64 d; asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b)); return d; }
 __device__ __forceinline__ u64 bc(float s) { return pk(s, s); }                      // scalar broadcast
 __device__ __forceinline__ u64 sw(float2 a) { return pk(a.y, a.x); }                // swapped halves
+// (fmaf(a.x, b.x, -a.y*b.y), fmaf(a.x, b.y, a.y*b.x))
 __device__ __forceinline__ float2 cmul(float2 a, float2 b) { return U(fma2(bc(a.x), P(b), mul2(pk(b.y, -b.x), bc(-a.y)))); }
+// a * conj(b) = (fmaf(a.x, b.x, a.y*b.y), fmaf(a.y, b.x, -a.x*b.y))
 __device__ __forceinline__ float2 cmulc(float2 a, float2 b) { return U(fma2(P(a), bc(b.x), mul2(pk(a.y, -a.x), bc(b.y)))); }
 __device__ __forceinline__ float2 cadd(float2 a, float2 b) { return U(add2(P(a), P(b))); }
 __device__ __forceinline__ float2 csub(float2 a, float2 b) { return U(sub2(P(a), P(b))); }
+// s*a + c per component, s*a, a*b per component, a*(sx,sy) + c per component
 __device__ __forceinline__ float2 caxpy(float s, float2 a, float2 c) { return U(fma2(bc(s), P(a), P(c))); }
 __device__ __forceinline__ float2 cscale(float s, float2 a) { return U(mul2(bc(s), P(a))); }
 __device__ __forceinline__ float2 cmul_elem(float2 a, float2 b) { return U(mul2(P(a), P(b))); }
 __device__ __forceinline__ float2 cfma_elem(float2 a, float sx, float sy, float2 c) { return U(fma2(P(a), pk(sx, sy), P(c))); }
+// d + s*rot90<INV>(x) and d - s*rot90<INV>(x)   (rot90 = times +i for INV, -i otherwise; s = 1: a plain add/sub)
 template <bool INV> __device__ __forceinline__ float2 addrot(float2 d, float2 x, float s = 1.0f) {
     return U(fma2(sw(x), INV ? pk(-s, s) : pk(s, -s), P(d)));
 }
@@ -58,33 +55,6 @@ template <bool INV> __device__ __forceinline__ float2 subrot(float2 d, float2 x,
 __device__ __forceinline__ float2 cmac(float2 acc, float2 v, float2 w) {
     return U(fma2(bc(v.x), P(w), fma2(pk(w.y, -w.x), bc(-v.y), P(acc))));
 }
-#else
-// (fmaf(a.x, b.x, -a.y*b.y), fmaf(a.x, b.y, a.y*b.x))
-__device__ __forceinline__ float2 cmul(float2 a, float2 b) {
-    return make_float2(fmaf(a.x, b.x, -a.y * b.y), fmaf(a.x, b.y, a.y * b.x));
-}
-// a * conj(b) = (fmaf(a.x, b.x, a.y*b.y), fmaf(a.y, b.x, -a.x*b.y))
-__device__ __forceinline__ float2 cmulc(float2 a, float2 b) {
-    return make_float2(fmaf(a.x, b.x, a.y * b.y), fmaf(a.y, b.x, -a.x * b.y));
-}
-__device__ __forceinline__ float2 cadd(float2 a, float2 b) { return make_float2(a.x + b.x, a.y + b.y); }
-__device__ __forceinline__ float2 csub(float2 a, float2 b) { return make_float2(a.x - b.x, a.y - b.y); }
-// s*a + c per component, s*a, a*b per component, a*(sx,sy) + c per component
-__device__ __forceinline__ float2 caxpy(float s, float2 a, float2 c) { return make_float2(fmaf(s, a.x, c.x), fmaf(s, a.y, c.y)); }
-__device__ __forceinline__ float2 cscale(float s, float2 a) { return make_float2(s * a.x, s * a.y); }
-__device__ __forceinline__ float2 cmul_elem(float2 a, float2 b) { return make_float2(a.x * b.x, a.y * b.y); }
-__device__ __forceinline__ float2 cfma_elem(float2 a, float sx, float sy, float2 c) { return make_float2(fmaf(a.x, sx, c.x), fmaf(a.y, sy, c.y)); }
-// d + s*rot90<INV>(x) and d - s*rot90<INV>(x)   (rot90 = times +i for INV, -i otherwise; s = 1: a plain add/sub)
-template <bool INV> __device__ __forceinline__ float2 addrot(float2 d, float2 x, float s = 1.0f) {
-    return INV ? make_float2(fmaf(x.y, -s, d.x), fmaf(x.x, s, d.y)) : make_float2(fmaf(x.y, s, d.x), fmaf(x.x, -s, d.y));
-}
-template <bool INV> __device__ __forceinline__ float2 subrot(float2 d, float2 x, float s = 1.0f) {
-    return INV ? make_float2(fmaf(x.y, s, d.x), fmaf(x.x, -s, d.y)) : make_float2(fmaf(x.y, -s, d.x), fmaf(x.x, s, d.y));
-}
-__device__ __forceinline__ float2 cmac(float2 acc, float2 v, float2 w) {
-    return make_float2(fmaf(v.x, w.x, fmaf(-v.y, w.y, acc.x)), fmaf(v.x, w.y, fmaf(v.y, w.x, acc.y)));
-}
-#endif
 // multiply by -i (forward) or +i (inverse)
 template <bool INV> __device__ __forceinline__ float2 rot90(float2 a) {
     return INV ? make_float2(-a.y, a.x) : make_float2(a.y, -a.x);
@@ -350,23 +320,6 @@ __device__ __forceinline__ void pass_inplace_batched(float2* buf, int tid, const
         if (it < ITEMS) {
             const int b = it / NBF, t = it - b * NBF;
             Pass<N, R, S, PM>::template compute_store<INV, TT, MapOut>(buf + b * STRIDE, t, a[i], W);
-        }
-    }
-    __syncthreads();
-}
-
-// Out-of-place pass src -> dst (both shared memory, distinct): one butterfly at a time per thread (low register
-// pressure), a single barrier at the end.
-template <int N, int R, int S, int NT, bool INV, bool TT = false, bool PM = false>
-__device__ __forceinline__ void pass_oop(const float2* src, float2* dst, int lt, const float2* __restrict__ W) {
-    constexpr int NBF = N / R;
-#pragma unroll
-    for (int t0 = 0; t0 < NBF; t0 += NT) {
-        const int t = t0 + lt;
-        if (NBF % NT == 0 || t < NBF) {
-            float2 a[R];
-            Pass<N, R, S, PM>::load(src, t, a);
-            Pass<N, R, S, PM>::template compute_store<INV, TT>(dst, t, a, W);
         }
     }
     __syncthreads();

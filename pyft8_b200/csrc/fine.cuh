@@ -225,15 +225,16 @@ __device__ __forceinline__ void fine_pass12(float2* dst, const float2* __restric
     fine_pass12_finish(in, dst, p2, TF, taper, w);
 }
 
-// Pass (8,25) px -> po by all 256 threads, p-major: thread tid owns p = tid % 16 in both of its butterflies (q = tid / 16 and
-// tid / 16 + 16), so its 7 twiddles w^(25 p k) live in registers for the whole kernel (tw8, loaded once) -- no twiddle loads
-// in this pass at all.  Loads have stride 25 elements across lanes, stores go to the padded operand layout
-// q + 201 p + 25 k (stride 201): both conflict-free.  One barrier at the end.
+// Pass (8,25) px -> po by NT threads (a multiple of 16), p-major: thread tid owns p = tid % 16 in every butterfly it runs
+// (q = tid / 16, tid / 16 + NT / 16, ...), so its 7 twiddles w^(25 p k) live in registers for the whole kernel (tw8, loaded
+// once) -- no twiddle loads in this pass at all.  Loads have stride 25 elements across lanes, stores go to the padded
+// operand layout q + 201 p + 25 k (stride 201): both conflict-free.  One barrier at the end.
+template <int NT>
 __device__ __forceinline__ void fine_pass3(const float2* src, float2* dst, int tid, const float2 (&tw8)[7]) {
     const int p = tid & 15;
 #pragma unroll
-    for (int r = 0; r < 2; ++r) {
-        const int q = (tid >> 4) + 16 * r;
+    for (int r = 0; r < (25 * 16 + NT - 1) / NT; ++r) {
+        const int q = (tid >> 4) + (NT / 16) * r;
         if (q < 25) {
             float2 a[8];
 #pragma unroll
@@ -248,15 +249,21 @@ __device__ __forceinline__ void fine_pass3(const float2* src, float2* dst, int t
     __syncthreads();
 }
 
-// Full last pass (16,200) of the winner: padded operands pb -> natural-order samples in dst.  One barrier at the end.
+// Full last pass (16,200) of the winner by NT threads: padded operands pb -> natural-order samples in dst.  One barrier at
+// the end.
+template <int NT>
 __device__ __forceinline__ void fine_last_full(const float2* src, float2* dst, int tid) {
-    if (tid < 200) {
-        float2 a[16];
 #pragma unroll
-        for (int j = 0; j < 16; ++j) a[j] = src[tid + 201 * j];
-        Dft<16, true>::run(a);
+    for (int t0 = 0; t0 < 200; t0 += NT) {
+        const int t = t0 + tid;
+        if (t < 200) {
+            float2 a[16];
 #pragma unroll
-        for (int k = 0; k < 16; ++k) dst[tid + 200 * k] = a[k];
+            for (int j = 0; j < 16; ++j) a[j] = src[t + 201 * j];
+            Dft<16, true>::run(a);
+#pragma unroll
+            for (int k = 0; k < 16; ++k) dst[t + 200 * k] = a[k];
+        }
     }
     __syncthreads();
 }
@@ -409,7 +416,7 @@ k_fine(const float2* __restrict__ spec, int spec_stride, const int32_t* __restri
         FineIn fin;
         FP_T(ts0);
         if (warp >= 4) fine_pass12_load(fin, sp, fb0 - 32, tid - 128);       // operands of the next transform: in flight during pass (8,25)
-        fine_pass3(px, po, tid, tw8);
+        fine_pass3<FINE_NT>(px, po, tid, tw8);
         FP_T(ts1);
         if (warp < 4) {
             fine_pass4_window(po, zwin, tb0 - 8 + 1152, 238, tid, w16);
@@ -441,7 +448,7 @@ k_fine(const float2* __restrict__ spec, int spec_stride, const int32_t* __restri
             const int fi = e < 4 ? e : e + 1;
             if (warp >= 4 && e < 7) fine_pass12_load(fin, sp, fb0 + (-32 + 8 * (e + 1 < 4 ? e + 1 : e + 2)), tid - 128);
             FP_T(t0);
-            fine_pass3(px, po, tid, tw8);
+            fine_pass3<FINE_NT>(px, po, tid, tw8);
             FP_T(t1);
             if (warp < 4) {
                 fine_pass4_window(po, zwin, tb0 + tt + 1152, 224, tid, w16);
@@ -470,7 +477,7 @@ k_fine(const float2* __restrict__ spec, int spec_stride, const int32_t* __restri
         //      per warp and call) and the Costas count + LLRs by warp 0, while the producer warps already build the first
         //      transform of this CTA's next item into px (unused during this stage)
         FP_T(tf0);
-        fine_last_full(pb, po, tid);
+        fine_last_full<FINE_NT>(pb, po, tid);
         FP_T(tf1);
         if (warp < 4) {
             const float2* z = po;

@@ -375,10 +375,8 @@ extern "C" int ft8_create(int device, const ft8_cfg* cfg_in, ft8_handle** out) {
     // four-step scratch Y: 768 KB per cycle, written by k_cs_cols and read back by k_cs_rows, in chunks of up to 1024 cycles.
     // Smaller, L2-resident chunks (VERDICT r1 item 7) were measured and are SLOWER: 3.18 ms per 4096 cycles at 1024, 3.50 at 256,
     // 3.88 at 128, 4.20 at 64, 5.00 at 32 (profiles/r02_experiments.md) -- both kernels sit on the L1/shared data pipe, not on
-    // HBM, so the 3x DRAM traffic costs nothing while small grids lose to tail effects.  FT8_Y_CYCLES overrides for experiments.
-    size_t ych = 1024;
-    if (const char* e = getenv("FT8_Y_CYCLES")) ych = (size_t)std::max(1, atoi(e));
-    h->y_cycles = std::min<size_t>(B, ych);
+    // HBM, so the 3x DRAM traffic costs nothing while small grids lose to tail effects.
+    h->y_cycles = std::min<size_t>(B, 1024);
     CKC(h->d_Y.ensure(h->y_cycles * CS_N));
     CKC(h->d_spec.ensure(B * FINE_SPEC_STRIDE));
     CKC(h->d_best_score.ensure(B * N_F0 * SY_HS));
@@ -399,14 +397,14 @@ extern "C" int ft8_create(int device, const ft8_cfg* cfg_in, ft8_handle** out) {
         CKC(upload(h->d_cycle_of, co));
     }
     CKC(cudaFuncSetAttribute(k_fine, cudaFuncAttributeMaxDynamicSharedMemorySize, FINE_SMEM_BYTES));
-    CKC(cudaFuncSetAttribute(k_fine_tscan<FT_NT, FT_CTAS>, cudaFuncAttributeMaxDynamicSharedMemorySize, FT_SMEM_BYTES));
-    CKC(cudaFuncSetAttribute(k_fine_final<FT_NT, FF_CTAS>, cudaFuncAttributeMaxDynamicSharedMemorySize, FF_SMEM_BYTES));
+    CKC(cudaFuncSetAttribute(k_fine_tscan, cudaFuncAttributeMaxDynamicSharedMemorySize, FT_SMEM_BYTES));
+    CKC(cudaFuncSetAttribute(k_fine_final, cudaFuncAttributeMaxDynamicSharedMemorySize, FF_SMEM_BYTES));
     CKC(cudaFuncSetAttribute(k_fscan_mma, cudaFuncAttributeMaxDynamicSharedMemorySize, FS_SMEM_BYTES));
     if (cfg.fine_mode == 0) {
         CKC(h->d_zwin.ensure(N * FS_WIN)); CKC(h->d_tso.ensure(N)); CKC(h->d_ff.ensure(N)); CKC(h->d_amb.ensure(N + 1));
     }
     {
-        const int sp_smem = SP_ROWS * SP_BUFS * SP_BUF_LEN * (int)sizeof(float2);
+        const int sp_smem = SP_BUF_LEN * (int)sizeof(float2);
         CKC(cudaFuncSetAttribute(k_spectrogram<int16_t, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, sp_smem));
         CKC(cudaFuncSetAttribute(k_spectrogram<float, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, sp_smem));
         CKC(cudaFuncSetAttribute(k_spectrogram<int16_t, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, sp_smem));
@@ -481,11 +479,11 @@ static int launch_spectrogram(ft8_handle* h, const void* d_audio, int dtype, int
                               int row_hi = 375, int out_rows = GRID_ROWS, int out_row0 = 0, int fill_row0 = 1,
                               const float* d_prev_tail = nullptr, int out_wrap = 0) {
     const bool ring = d_prev_tail != nullptr || out_wrap != 0;
-    dim3 grid((row_hi - row_lo + SP_ROWS) / SP_ROWS, B);
-    const int smem = SP_ROWS * SP_BUFS * SP_BUF_LEN * (int)sizeof(float2);
+    dim3 grid(row_hi - row_lo + 1, B);
+    const int smem = SP_BUF_LEN * (int)sizeof(float2);
 #define SP_LAUNCH(T, RING)                                                                                                          \
-    k_spectrogram<T, RING><<<grid, SP_ROWS * SP_NT, smem, h->stream>>>((const T*)d_audio, d_grid, h->d_hann, h->d_TS, h->d_W3840, row_lo, \
-                                                                       row_hi, out_rows, out_row0, fill_row0, d_prev_tail, out_wrap)
+    k_spectrogram<T, RING><<<grid, SP_NT, smem, h->stream>>>((const T*)d_audio, d_grid, h->d_hann, h->d_TS, h->d_W3840, row_lo, \
+                                                             row_hi, out_rows, out_row0, fill_row0, d_prev_tail, out_wrap)
     if (dtype == FT8_AUDIO_I16) { if (ring) SP_LAUNCH(int16_t, true); else SP_LAUNCH(int16_t, false); }
     else { if (ring) SP_LAUNCH(float, true); else SP_LAUNCH(float, false); }
 #undef SP_LAUNCH
@@ -543,7 +541,7 @@ static int launch_fine(ft8_handle* h, const float2* spec, int spec_stride, const
     CK(h->d_amb.ensure(need + 1, h->stream));
     const int nbt = list ? persistent_blocks(h, FT_CTAS) : std::min(persistent_blocks(h, FT_CTAS), n_direct);
     const int nb3 = list ? persistent_blocks(h, FF_CTAS) : std::min(persistent_blocks(h, FF_CTAS), n_direct);
-    k_fine_tscan<FT_NT, FT_CTAS><<<nbt, FT_NT, FT_SMEM_BYTES, h->stream>>>(spec, spec_stride, list, count, n_direct, cycle_of, f0, h0, h->d_TF, h->d_tso, h->d_zwin);
+    k_fine_tscan<<<nbt, FT_NT, FT_SMEM_BYTES, h->stream>>>(spec, spec_stride, list, count, n_direct, cycle_of, f0, h0, h->d_TF, h->d_tso, h->d_zwin);
     CK(cudaGetLastError());
     CK(cudaEventRecord(h->ev[EV_TSCAN_END], h->stream));
     const int nb1 = list ? h->n_sm : std::min(h->n_sm, (n_direct + FS_CAND - 1) / FS_CAND);
@@ -552,7 +550,7 @@ static int launch_fine(ft8_handle* h, const float2* spec, int spec_stride, const
                                                          h->d_bmat, h->d_w6400, h->d_ff, h->d_amb + 1, h->d_amb);
     CK(cudaGetLastError());
     CK(cudaEventRecord(h->ev[EV_FSCAN_END], h->stream));
-    k_fine_final<FT_NT, FF_CTAS><<<nb3, FT_NT, FF_SMEM_BYTES, h->stream>>>(spec, spec_stride, list, count, n_direct, cycle_of, f0, h0, h->d_TF, h->d_tso, h->d_ff,
+    k_fine_final<<<nb3, FT_NT, FF_SMEM_BYTES, h->stream>>>(spec, spec_stride, list, count, n_direct, cycle_of, f0, h0, h->d_TF, h->d_tso, h->d_ff,
                                                             fo, llr, sig_grid);
     CK(cudaGetLastError());
     // near-tie candidates of the frequency scan: decided by the literal nine-transform kernel (overwrites their results)

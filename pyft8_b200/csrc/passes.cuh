@@ -89,13 +89,7 @@ __device__ __forceinline__ void set_result(const CandState& cs, int slot, const 
 // ipass 0.  grid: [B][grid_rows][976].  payload_db (optional): [N][58][8].
 // prev[] of the decoder in registers needs ~90 registers: 5 CTAs/SM instead of 8 (measured: 5.80 ms with prev in shared
 // memory at 8 CTAs, 5.02 with the cheaper quotients, 4.33 with prev in registers at 5 CTAs)
-#ifndef PASS0_MINB
-#define PASS0_MINB 4
-#endif
-#ifndef PASS234_MINB
-#define PASS234_MINB 5
-#endif
-__global__ void __launch_bounds__(WARPS_PER_CTA * 32, PASS0_MINB)
+__global__ void __launch_bounds__(WARPS_PER_CTA * 32, 4)
 k_pass0(CandState cs, int n_slots, const float* __restrict__ grid, int grid_rows, int cycle_h0, float sd_min,
         float* __restrict__ payload_db, int llr_only, int32_t* __restrict__ list_fine, int32_t* __restrict__ count_fine,
         int32_t* __restrict__ next_slot, DevStats* __restrict__ stats) {
@@ -198,7 +192,7 @@ k_pass0(CandState cs, int n_slots, const float* __restrict__ grid, int grid_rows
 }
 
 // ipass 2..4 over list_fine.
-__global__ void __launch_bounds__(WARPS_PER_CTA * 32, PASS234_MINB)
+__global__ void __launch_bounds__(WARPS_PER_CTA * 32, 5)
 k_pass234(CandState cs, const int32_t* __restrict__ list, const int32_t* __restrict__ count, float sd_min,
           int32_t* __restrict__ list_osd, int32_t* __restrict__ count_osd, int32_t* __restrict__ next_item,
           DevStats* __restrict__ stats) {
@@ -276,10 +270,7 @@ struct OsdSmem {
 };
 
 // ipass 5-6: item = 10 * list index + attempt.  attempts 0..4: AP pattern on the fine llr; 5..9: saved llr.
-#ifndef OSD_MINB
-#define OSD_MINB 8
-#endif
-__global__ void __launch_bounds__(WARPS_PER_CTA * 32, OSD_MINB)
+__global__ void __launch_bounds__(WARPS_PER_CTA * 32, 8)
 k_osd_items(CandState cs, const int32_t* __restrict__ list, const int32_t* __restrict__ count, int S, int D,
             int32_t* __restrict__ next_item, DevStats* __restrict__ stats) {
     extern __shared__ __align__(16) unsigned char pass_smem_raw[];

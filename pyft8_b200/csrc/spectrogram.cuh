@@ -5,10 +5,10 @@
 //     grid[h, k] = 20*log10(|rfft(x[480h-3840 : 480h] * hanning(3840))[k]| + 1e-12),  k < 976, 1 <= h <= 375
 // with x = 0 before the cycle start and grid[0, :] = 1.0 (the reference's initial fill).
 //
-// One group of 128 threads per row, SP_ROWS rows per CTA (1 measured best on B200: 5.4 vs 6.1 ms / 2048 cycles for 4).  The 3840-point real transform is a
-// 1920-point complex Stockham FFT of z[n] = x[2n] + i*x[2n+1] in shared memory (passes 15,8,16);
+// One CTA of 128 threads per row (measured best on B200: 5.4 vs 6.1 ms / 2048 cycles with 4 rows per CTA).  The 3840-point
+// real transform is a 1920-point complex Stockham FFT of z[n] = x[2n] + i*x[2n+1] in shared memory (passes 15,8,16);
 // the first pass reads the windowed audio straight from global memory (int16 -> fp32 fused), the
-// epilogue untangles only the 976 bins that are kept and writes dB.  Rows of one CTA are adjacent,
+// epilogue untangles only the 976 bins that are kept and writes dB.  Consecutive CTAs take adjacent rows,
 // so their 7/8-overlapping windows hit L1/L2: HBM sees the audio once and the grid once.
 //
 // Round-2 experiments that REDUCED the shared-memory / L1 wavefronts per row and still lost (profiles/r02_experiments.md):
@@ -23,13 +23,8 @@
 
 namespace ft8 {
 
-#ifndef SP_ROWS_N
-#define SP_ROWS_N 1
-#endif
-constexpr int SP_ROWS = SP_ROWS_N;  // rows per CTA
-constexpr int SP_BUFS = 1;          // one in-place buffer per row (ping-pong buffers measured slower)
 constexpr int SP_NT = 128;          // threads per row
-constexpr int SP_BUF_LEN = 1936;      // 1920 + one pad element per 120 (the layout after the second pass)
+constexpr int SP_BUF_LEN = 1936;    // one in-place buffer (ping-pong buffers measured slower): 1920 + one pad element per 120
 constexpr int SP_T8_OFF = 14 * 128;  // per-pass twiddle tables of the 1920-point transform: [(15,1): 14 x 128 | (8,15): 7 x 16]
 constexpr int GRID_ROWS = 376, GRID_COLS = 976, CYCLE_SAMPLES = 180000, NFFT_S = 3840, HOP = 480;
 
@@ -40,22 +35,20 @@ __device__ __forceinline__ float2 load_sample_pair(const int16_t* a, int i) {
 }
 __device__ __forceinline__ float2 load_sample_pair(const float* a, int i) { return __ldg(reinterpret_cast<const float2*>(a + i)); }
 
-#ifndef SP_MIN_BLOCKS
-#define SP_MIN_BLOCKS 8   // 64 registers -> 8 CTAs (32 warps) per SM; measured best on B200
-#endif
 // RING = false: isolated cycles (the batch path; compiled exactly as before the live mode existed -- the extra branch in the
 // 15-operand load loop cost 27 % when it was a run-time test).  RING = true: live mode, see prev_tail / out_wrap.
+// Launch bounds: 64 registers -> 8 CTAs (32 warps) per SM; measured best on B200.
 template <typename T, bool RING = false>
-__global__ void __launch_bounds__(SP_ROWS* SP_NT, SP_MIN_BLOCKS)
+__global__ void __launch_bounds__(SP_NT, 8)
 k_spectrogram(const T* __restrict__ audio, float* __restrict__ grid, const float* __restrict__ hann,
               const float2* __restrict__ TS, const float2* __restrict__ W3840, int row_lo, int row_hi, int out_rows,
               int out_row0, int fill_row0, const float* __restrict__ prev_tail = nullptr, int out_wrap = 0) {
     extern __shared__ float2 sp_smem[];
     const int cyc = blockIdx.y;
-    const int g = threadIdx.x / SP_NT, lt = threadIdx.x % SP_NT;
-    const int h = row_lo + blockIdx.x * SP_ROWS + g;      // grid row = window ending at sample 480*h
+    const int lt = threadIdx.x;
+    const int h = row_lo + blockIdx.x;                    // grid row = window ending at sample 480*h
     const bool live = h <= row_hi;
-    float2* buf = sp_smem + g * SP_BUF_LEN * SP_BUFS;
+    float2* buf = sp_smem;
     const T* x = audio + (size_t)cyc * CYCLE_SAMPLES;
     // live ring (receiver.py:295-306): the windows of the first hops of a cycle reach back into the previous cycle's audio;
     // prev_tail holds its last 3840 samples per stream as float32, whatever T is (zeros for a stream without a previous

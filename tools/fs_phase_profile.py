@@ -21,5 +21,5 @@ v = [int(x) for x in buf]
 n_i, n_g, n_p = max(v[5], 1), max(v[9], 1), max(v[12], 1)
 print(json.dumps({"issuer_per_chunk_clk": {"issue_b(wait free it-2)": v[0] / n_i, "wait acc_free": v[1] / n_i, "wait a_ready": v[2] / n_i,
                                             "wait b_full": v[3] / n_i, "mma issue+commit": v[4] / n_i, "chunks": n_i},
-                  "generator_warp0_per_own_chunk_clk": {"loads+compute": v[6] / n_g, "wait stage free": v[7] / n_g, "split+st+wait+arrive": v[8] / n_g, "chunks": n_g},
+                  "generator_warp0_per_own_chunk_clk": {"issue next loads": v[6] / n_g, "wait stage free": v[7] / n_g, "compute+split+st+wait+arrive": v[8] / n_g, "chunks": n_g},
                   "generator_warp0_per_pass_clk": {"chunk loop": v[10] / n_p, "wait acc_ready": v[11] / n_p, "passes": n_p}}))

@@ -1,4 +1,4 @@
-// div_check.cu -- how often does the four-instruction division of csrc/ldpc.cuh (div_rn_fast) differ from IEEE div.rn?
+// div_check.cu -- how often does the residual-corrected quotient of csrc/ldpc.cuh's check-node update differ from IEEE div.rn?
 //   nvcc -arch=sm_100a -O3 -o div_check tools/micro/div_check.cu && ./div_check
 // Operands are drawn from the ranges the LDPC check-node update divides in (decoders.py:146-149): P / t with |t| in
 // (1e-6, 1], |P| <= |t|, and e / ((e - 1.18)(1.18 + e)) with e in [-1, 1].  Prints one JSON line.
