@@ -244,6 +244,12 @@ int ft8_synth_cycles(ft8_handle* h, const uint8_t* symbols, const float* f_hz, c
 /* Test hook: batched complex FFT through the library's shared-memory kernels (n in {32, 256, 375, 1920, 3200}). */
 int ft8_debug_fft(ft8_handle* h, int n, int inverse, const float* in, float* out, int batch);
 
+/* Test hook: the OSD attempts of pass 5 (the five AP patterns on one llr, with RR73, 73 and RRR sharing one reliability order
+ * and basis, as the decode runs them) on host llr[N][174] -> found[N][5], bits91[N][5][3], attempt k as ft8_osd gives it
+ * for the llr with AP pattern k applied. */
+int ft8_debug_osd_ap(ft8_handle* h, const float* llr, int N, int singleflips, int doubleflips, int32_t* found,
+                     uint32_t* bits91);
+
 #ifdef __cplusplus
 }
 #endif

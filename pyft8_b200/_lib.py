@@ -81,6 +81,7 @@ SIGNATURES = {
     "ft8_decode_cycles_stream": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, _P, C.c_int, _P, _P]),
     "ft8_synth_cycles": (C.c_int, [_P, _P, _P, _P, _P, C.c_int, C.c_int, C.c_float, C.c_uint64, _P, C.c_int]),
     "ft8_debug_fft": (C.c_int, [_P, C.c_int, C.c_int, _P, _P, C.c_int]),
+    "ft8_debug_osd_ap": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, _P, _P]),
 }
 
 _lib = None

@@ -1243,6 +1243,39 @@ extern "C" int ft8_debug_fft(ft8_handle* h, int n, int inverse, const float* in,
     return st.finish();
 }
 
+// ipass 5 of k_osd_items on each llr: work item 3 n + t runs the same osd_attempts call as k_osd_items' item t of a candidate
+__global__ void __launch_bounds__(WARPS_PER_CTA * 32, 8)
+k_debug_osd_ap(const float* __restrict__ llr, int N, int S, int D, int32_t* __restrict__ found, uint32_t* __restrict__ bits) {
+    extern __shared__ __align__(16) unsigned char pass_smem_raw[];
+    OsdSmem& sm = *reinterpret_cast<OsdSmem*>(pass_smem_raw);
+    const int wi = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const LaneSyn ls = load_lane_syn(lane);
+    load_osd_tables(sm.tab);
+    __syncthreads();
+    for (int it = blockIdx.x * WARPS_PER_CTA + wi; it < 3 * N; it += gridDim.x * WARPS_PER_CTA) {
+        const int n = it / 3, t = it - 3 * n;
+        osd_attempts(sm.w[wi], sm.tab, sm.llr[wi], llr + (size_t)n * 174, t, t == 2 ? 5 : t + 1, lane, ls, S, D,
+                     found + (size_t)n * 5, bits + (size_t)n * 15);
+        __syncwarp();
+    }
+}
+
+extern "C" int ft8_debug_osd_ap(ft8_handle* h, const float* llr, int N, int singleflips, int doubleflips, int32_t* found,
+                                uint32_t* bits91) {
+    ENTER(h);
+    if (!llr || !found || !bits91 || N <= 0 || singleflips < 0 || singleflips > OSD_MAX_FLIPS || doubleflips < 0)
+        return fail(h, FT8_E_BADARG, "ft8_debug_osd_ap: bad argument (singleflips must be 0..91)");
+    const float* dl; int32_t* df; uint32_t* db;
+    Staging st(h, FT8_MEM_HOST);
+    st.in(dl, llr, (size_t)N * 174 * 4);
+    st.out(df, found, (size_t)N * 5 * 4); st.out(db, bits91, (size_t)N * 15 * 4);
+    TRY(st.begin());
+    k_debug_osd_ap<<<std::min(persistent_blocks(h, 8), (3 * N + WARPS_PER_CTA - 1) / WARPS_PER_CTA), WARPS_PER_CTA * 32, sizeof(OsdSmem),
+                     h->stream>>>(dl, N, singleflips, doubleflips, df, db);
+    CK(cudaGetLastError());
+    return st.finish();
+}
+
 #ifdef FS_PROFILE
 extern "C" int ft8_debug_fs_prof(unsigned long long* out16, int reset) {
     cudaMemcpyFromSymbol(out16, ft8::g_fs_prof, sizeof(unsigned long long) * 16);

@@ -26,6 +26,9 @@
 // and flipping pivot k adds bit (row of k) of every image, plus the unit bit of k's own column when it is systematic.
 // CRC-14 is linear, so each of the 1+S vectors carries its 14-bit syndrome and a trial's CRC test is an XOR; the 91-bit
 // word of a trial is only assembled when that XOR is zero.
+// The work splits by what it depends on.  osd_basis (the order, the basis, the images and the flip syndromes) reads only
+// |llr|; osd_eval (u, the order-0 word and its syndrome, the trials) is the only part that reads the hard decisions.  Calls
+// whose inputs differ only in signs share one osd_basis (the AP attempts RR73, 73 and RRR, passes.cuh).
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -42,11 +45,11 @@ __constant__ OsdTables c_osd;
 constexpr int OSD_MAX_FLIPS = 91;
 
 struct OsdWarpScratch {
-    uint32_t order[176];             // sorted position -> entry | hard decision << 8 (32-bit: no sub-word extraction in the visit loop)
+    uint32_t order[176];             // sorted position -> entry (32-bit: no sub-word extraction in the visit loop)
     uint8_t piv_row[96];             // pivot k -> row
-    uint8_t piv_col[96];             // pivot k -> original column (255: a parity column)
+    uint8_t piv_col[96];             // pivot k -> original column (>= 91: a parity column)
     uint8_t pcol[96];                // parity rank (position among the parity columns in reliability order) -> column
-    uint16_t syn[OSD_MAX_FLIPS + 1]; // CRC syndrome of [0] the order-0 word, [1+i] the vector that flip i adds
+    uint16_t syn[OSD_MAX_FLIPS];     // CRC syndrome of the vector that flip i adds
     uint16_t ssyn[96];               // CRC syndrome of the systematic column whose image slot j holds (0: not a basis slot)
     uint32_t colw[3 * 97];           // the stored columns word-major [3][OSD_W_PITCH] (odd pitch: the three words of a slot
                                      // sit in different banks)
@@ -105,9 +108,15 @@ __device__ __forceinline__ uint32_t sel3(int w, uint32_t a0, uint32_t a1, uint32
           "+r"(ownrow[A])                                                                                                 \
         : "r"(pb), "r"(x0), "r"(x1), "r"(x2), "r"(jl), "r"(lane), "r"(p), "r"(TA), "r"(TB), "r"(TD))
 
-// Returns trial index + 1 of the first accepted trial word (0 = none); bits = that word.
-// llr: 174 floats in shared or global memory.
-__device__ __forceinline__ int osd_warp(OsdWarpScratch& s, const OsdCtaTables& g, const float* llr, int lane, const LaneSyn& ls, int S, int D, uint32_t* bits) {
+// What osd_basis leaves in registers for osd_eval: the lane's three stored columns and the row whose image each slot holds.
+struct OsdBasis {
+    uint32_t c0[3], c1[3], c2[3];
+    uint32_t ownrow[3];               // row (= systematic column) whose image the slot holds, 255: not a basis slot
+};
+
+// Steps 1-4 without the hard decisions: reliability order, basis, images, and the syndromes of the S flip vectors
+// (s.piv_row, s.piv_col, s.syn, s.ssyn, s.colw; ob).  llr: 174 floats in shared or global memory; only |llr| is read.
+__device__ __forceinline__ void osd_basis(OsdWarpScratch& s, const OsdCtaTables& g, const float* llr, int lane, int S, OsdBasis& ob) {
     constexpr uint32_t FULL = 0xffffffffu;
     // ---- 1. reliability order.  Fast path: bitonic sort of 256 32-bit keys (8 per lane, slot e = 32*r + lane), descending,
     //      key = code(|llr|) << 8 | (255 - index) with a monotone 24-bit code (zero, or 5 exponent bits for [2^-26, 2^5)
@@ -176,7 +185,7 @@ __device__ __forceinline__ int osd_warp(OsdWarpScratch& s, const OsdCtaTables& g
         }
         bad = __any_sync(FULL, bad);
     }
-    // ---- 2. publish the order with the hard decisions: entry = column for a systematic column, 128 + parity rank for a parity
+    // ---- 2. publish the order: entry = column for a systematic column, 128 + parity rank for a parity
     //      column (its rank among the parity columns in reliability order = the slot it will live in); rows whose
     //      systematic column comes late (position >= 96)
     uint32_t L0 = 0, L1 = 0, L2 = 0;
@@ -192,7 +201,7 @@ __device__ __forceinline__ int osd_warp(OsdWarpScratch& s, const OsdCtaTables& g
             pbase += __popc(bal);
             if (sp < 174) {
                 if (isp) s.pcol[prank] = (uint8_t)c;
-                s.order[sp] = (uint32_t)((isp ? 128 + prank : c) | ((llr[c] > 0.0f) ? 0x100 : 0));
+                s.order[sp] = (uint32_t)(isp ? 128 + prank : c);
                 if (r >= 3 && c < 91) {
                     const uint32_t b = 1u << (c & 31);
                     if (c < 32) L0 |= b; else if (c < 64) L1 |= b; else L2 |= b;
@@ -214,7 +223,7 @@ __device__ __forceinline__ int osd_warp(OsdWarpScratch& s, const OsdCtaTables& g
                 prank += (q >= 91) ? before : 0;
             }
             if (i >= 91) s.pcol[prank] = (uint8_t)i;
-            s.order[rank] = (uint32_t)((i >= 91 ? 128 + prank : i) | ((llr[i] > 0.0f) ? 0x100 : 0));
+            s.order[rank] = (uint32_t)(i >= 91 ? 128 + prank : i);
             if (rank >= 96 && i < 91) {
                 const uint32_t b = 1u << (i & 31);
                 if (i < 32) L0 |= b; else if (i < 64) L1 |= b; else L2 |= b;
@@ -224,8 +233,7 @@ __device__ __forceinline__ int osd_warp(OsdWarpScratch& s, const OsdCtaTables& g
     L0 = __reduce_or_sync(FULL, L0); L1 = __reduce_or_sync(FULL, L1); L2 = __reduce_or_sync(FULL, L2);
     // ---- 3. the 83 parity columns (slot r of lane l: the parity column of rank 32 r + l), eliminated in place
     __syncwarp();
-    uint32_t c0[3], c1[3], c2[3];
-    uint32_t ownrow[3];               // row (= systematic column) whose image the slot holds, 255: not a basis slot
+    uint32_t (&c0)[3] = ob.c0, (&c1)[3] = ob.c1, (&c2)[3] = ob.c2, (&ownrow)[3] = ob.ownrow;
 #pragma unroll
     for (int r = 0; r < 3; ++r) {
         const int j = 32 * r + lane;
@@ -235,13 +243,11 @@ __device__ __forceinline__ int osd_warp(OsdWarpScratch& s, const OsdCtaTables& g
     }
     uint32_t own0 = 0, own1 = 0, own2 = 0;        // slot holding the image of row lane / 32 + lane / 64 + lane
     uint32_t used0 = 0, used1 = 0, used2 = 0;     // rows already holding a pivot
-    uint32_t u0 = 0, u1 = 0, u2 = 0;              // u[row] = hard decision of that row's pivot column
-    uint32_t hs0 = 0, hs1 = 0, hs2 = 0;           // hard decisions of the basis' systematic columns, by column
     int npiv = 0;
     // One visit of a stored column (slot j, fetched as v0..v2): dependent -> false; else pick the pivot row, do the
     // bookkeeping and eliminate.  JR = 0..2: the slot index is static (parity column in rank order); JR = 3: dynamic (the
-    // stored image of a systematic column).  csys = the systematic column being visited, or 255.
-    auto visit = [&](auto JRc, uint32_t v0, uint32_t v1, uint32_t v2, int j, int jl, int csys, bool hb) -> bool {
+    // stored image of a systematic column).  col = the column being visited.
+    auto visit = [&](auto JRc, uint32_t v0, uint32_t v1, uint32_t v2, int j, int jl, int col) -> bool {
         constexpr int JR = decltype(JRc)::value;
         const uint32_t f0 = v0 & ~used0, f1 = v1 & ~used1, f2 = v2 & ~used2;
         if ((f0 | f1 | f2) == 0) return false;    // dependent column
@@ -252,26 +258,22 @@ __device__ __forceinline__ int osd_warp(OsdWarpScratch& s, const OsdCtaTables& g
         const uint32_t pb = gw & (0u - gw);
         const int pl = 31 - __clz(pb);
         const int p = 32 * pw + pl;
-        if (lane == 0) { s.piv_row[npiv] = (uint8_t)p; s.piv_col[npiv] = (uint8_t)csys; }
-        if (JR == 3 && hb) {
-            const uint32_t b = 1u << (csys & 31);
-            if (csys < 32) hs0 |= b; else if (csys < 64) hs1 |= b; else hs2 |= b;
-        }
+        if (lane == 0) { s.piv_row[npiv] = (uint8_t)p; s.piv_col[npiv] = (uint8_t)col; }
         // pw is warp-uniform: three copies of the update, each testing a fixed word
         uint32_t x0 = v0, x1 = v1, x2 = v2;       // the pivot column with the pivot row cleared
         constexpr int A = JR < 3 ? JR : 0, B = (A + 1) % 3, D = (A + 2) % 3;
         if (pw == 0) {
-            used0 |= pb; if (hb) u0 |= pb;
+            used0 |= pb;
             if (lane == pl) own0 = (uint32_t)j;
             x0 &= ~pb;
             if (JR < 3) { OSD_ELIM_S(A, B, D, c0[A], c0[B], c0[D]); } else { OSD_ELIM(c0[0], c0[1], c0[2]); }
         } else if (pw == 1) {
-            used1 |= pb; if (hb) u1 |= pb;
+            used1 |= pb;
             if (lane == pl) own1 = (uint32_t)j;
             x1 &= ~pb;
             if (JR < 3) { OSD_ELIM_S(A, B, D, c1[A], c1[B], c1[D]); } else { OSD_ELIM(c1[0], c1[1], c1[2]); }
         } else {
-            used2 |= pb; if (hb) u2 |= pb;
+            used2 |= pb;
             if (lane == pl) own2 = (uint32_t)j;
             x2 &= ~pb;
             if (JR < 3) { OSD_ELIM_S(A, B, D, c2[A], c2[B], c2[D]); } else { OSD_ELIM(c2[0], c2[1], c2[2]); }
@@ -280,18 +282,14 @@ __device__ __forceinline__ int osd_warp(OsdWarpScratch& s, const OsdCtaTables& g
     };
     uint32_t e_next = s.order[0];
     for (int sp = 0; sp < 174; ++sp) {
-        const uint32_t e = e_next;
+        const int c = (int)e_next;
         e_next = s.order[sp + 1];                 // order[] is padded; the entry after the last one is never used
-        const int c = (int)(e & 0xFFu);
-        const bool hb = (e >> 8) != 0;
         bool piv;
         if (c < 128) {                            // systematic column c
             const int w = c >> 5;
             const uint32_t b = 1u << (c & 31);
             if ((sel3(w, used0, used1, used2) & b) == 0) {        // untouched unit vector on a free row: nothing to eliminate
-                if (w == 0) { used0 |= b; if (hb) { u0 |= b; hs0 |= b; } }
-                else if (w == 1) { used1 |= b; if (hb) { u1 |= b; hs1 |= b; } }
-                else { used2 |= b; if (hb) { u2 |= b; hs2 |= b; } }
+                if (w == 0) used0 |= b; else if (w == 1) used1 |= b; else used2 |= b;
                 if (lane == 0) { s.piv_row[npiv] = (uint8_t)c; s.piv_col[npiv] = (uint8_t)c; }
                 piv = true;
             } else {                                               // its image lives in a basis slot
@@ -300,42 +298,32 @@ __device__ __forceinline__ int osd_warp(OsdWarpScratch& s, const OsdCtaTables& g
                 const uint32_t v0 = __shfl_sync(FULL, sel3(jr, c0[0], c0[1], c0[2]), jl);
                 const uint32_t v1 = __shfl_sync(FULL, sel3(jr, c1[0], c1[1], c1[2]), jl);
                 const uint32_t v2 = __shfl_sync(FULL, sel3(jr, c2[0], c2[1], c2[2]), jl);
-                piv = visit(std::integral_constant<int, 3>{}, v0, v1, v2, j, jl, c, hb);
+                piv = visit(std::integral_constant<int, 3>{}, v0, v1, v2, j, jl, c);
             }
         } else {                                  // parity column of rank j: slot j / 32 of lane j % 32
             const int j = c - 128, jl = j & 31;
+            const int col = s.pcol[j];
             if (j < 32) {
-                piv = visit(std::integral_constant<int, 0>{}, __shfl_sync(FULL, c0[0], jl), __shfl_sync(FULL, c1[0], jl), __shfl_sync(FULL, c2[0], jl), j, jl, 255, hb);
+                piv = visit(std::integral_constant<int, 0>{}, __shfl_sync(FULL, c0[0], jl), __shfl_sync(FULL, c1[0], jl), __shfl_sync(FULL, c2[0], jl), j, jl, col);
             } else if (j < 64) {
-                piv = visit(std::integral_constant<int, 1>{}, __shfl_sync(FULL, c0[1], jl), __shfl_sync(FULL, c1[1], jl), __shfl_sync(FULL, c2[1], jl), j, jl, 255, hb);
+                piv = visit(std::integral_constant<int, 1>{}, __shfl_sync(FULL, c0[1], jl), __shfl_sync(FULL, c1[1], jl), __shfl_sync(FULL, c2[1], jl), j, jl, col);
             } else {
-                piv = visit(std::integral_constant<int, 2>{}, __shfl_sync(FULL, c0[2], jl), __shfl_sync(FULL, c1[2], jl), __shfl_sync(FULL, c2[2], jl), j, jl, 255, hb);
+                piv = visit(std::integral_constant<int, 2>{}, __shfl_sync(FULL, c0[2], jl), __shfl_sync(FULL, c1[2], jl), __shfl_sync(FULL, c2[2], jl), j, jl, col);
             }
         }
         if (piv && ++npiv == 91) break;
     }
     __syncwarp();
-    // ---- 4. CRC syndromes of the 1+S vectors (vector 0 = order-0 word, vector 1+i = what flip i adds).  Only the 14-bit
-    //      syndromes are needed to test a trial; the 91-bit words themselves are built on demand (osd_word) for the rare
-    //      trials whose syndrome is zero.  A slot that is not a basis slot contributes nothing (syndrome 0).
-    uint32_t slot_syn[3];
-#pragma unroll
-    for (int k = 0; k < 3; ++k) slot_syn[k] = (ownrow[k] < 91) ? (uint32_t)g.syn[ownrow[k]] : 0u;
-    {
-        uint32_t syn = (((hs0 >> lane) & 1u) ? ls.s0 : 0u) ^ (((hs1 >> lane) & 1u) ? ls.s1 : 0u) ^ (((hs2 >> lane) & 1u) ? ls.s2 : 0u);
-#pragma unroll
-        for (int k = 0; k < 3; ++k)
-            if ((__popc(c0[k] & u0) + __popc(c1[k] & u1) + __popc(c2[k] & u2)) & 1) syn ^= slot_syn[k];
-        syn = __reduce_xor_sync(FULL, syn);
-        if (lane == 0) s.syn[0] = (uint16_t)syn;
-    }
-    // flip vectors, one per lane: publish the stored columns word-major and let lane i walk the 83 slots for the bit of
-    // its pivot row (a per-vector warp reduction costs 30 x ~40 instructions; this loop ~6 x 83)
+    // ---- 4. CRC syndromes of the S flip vectors (vector i = what flip i adds).  Only the 14-bit syndromes are needed to
+    //      test a trial; the 91-bit words themselves are built on demand (osd_word) for the rare trials whose syndrome is
+    //      zero.  A slot that is not a basis slot contributes nothing (syndrome 0).
+    //      Publish the stored columns word-major and let lane i walk the 83 slots for the bit of its pivot row (a per-vector
+    //      warp reduction costs 30 x ~40 instructions; this loop ~6 x 83).
 #pragma unroll
     for (int k = 0; k < 3; ++k) {
         const int j = 32 * k + lane;
         s.colw[j] = c0[k]; s.colw[OSD_W_PITCH + j] = c1[k]; s.colw[2 * OSD_W_PITCH + j] = c2[k];
-        s.ssyn[j] = (uint16_t)slot_syn[k];
+        s.ssyn[j] = (ownrow[k] < 91) ? g.syn[ownrow[k]] : (uint16_t)0;
     }
     __syncwarp();
     for (int i0 = 0; i0 < S; i0 += 32) {
@@ -348,10 +336,41 @@ __device__ __forceinline__ int osd_warp(OsdWarpScratch& s, const OsdCtaTables& g
 #pragma unroll 4
         for (int q = 0; q < 83; ++q)
             if ((cw[q] >> sh) & 1u) syn ^= (uint32_t)s.ssyn[q];
-        if (act) s.syn[1 + i] = (uint16_t)syn;
+        if (act) s.syn[i] = (uint16_t)syn;
     }
     __syncwarp();
-    // 91-bit word of vector vi (-1: none), XOR-accumulated into w0..w2; every lane gets the result
+}
+
+// Step 5 for the hard decisions of llr (llr[c] > 0; NaN and -0 are 0) on the basis osd_basis found for the same |llr|.
+// Returns trial index + 1 of the first accepted trial word (0 = none); bits = that word, else the order-0 word.
+__device__ __forceinline__ int osd_eval(const OsdWarpScratch& s, const OsdCtaTables& g, const float* llr, int lane, const LaneSyn& ls, int S, int D,
+                                        const OsdBasis& ob, uint32_t* bits) {
+    constexpr uint32_t FULL = 0xffffffffu;
+    const uint32_t (&c0)[3] = ob.c0, (&c1)[3] = ob.c1, (&c2)[3] = ob.c2, (&ownrow)[3] = ob.ownrow;
+    // u[row] = hard decision of that row's pivot column; hs = hard decisions of the basis' systematic columns, by column
+    uint32_t u0 = 0, u1 = 0, u2 = 0, hs0 = 0, hs1 = 0, hs2 = 0;
+#pragma unroll
+    for (int r = 0; r < 3; ++r) {
+        const int k = 32 * r + lane;
+        if (k < 91) {
+            const int col = s.piv_col[k];
+            if (llr[col] > 0.0f) {
+                const int row = s.piv_row[k];
+                const uint32_t rb = 1u << (row & 31), cb = 1u << (col & 31);
+                if (row < 32) u0 |= rb; else if (row < 64) u1 |= rb; else u2 |= rb;
+                if (col < 32) hs0 |= cb; else if (col < 64) hs1 |= cb; else if (col < 91) hs2 |= cb;
+            }
+        }
+    }
+    u0 = __reduce_or_sync(FULL, u0); u1 = __reduce_or_sync(FULL, u1); u2 = __reduce_or_sync(FULL, u2);
+    hs0 = __reduce_or_sync(FULL, hs0); hs1 = __reduce_or_sync(FULL, hs1); hs2 = __reduce_or_sync(FULL, hs2);
+    // CRC syndrome of the order-0 word
+    uint32_t bs = (((hs0 >> lane) & 1u) ? ls.s0 : 0u) ^ (((hs1 >> lane) & 1u) ? ls.s1 : 0u) ^ (((hs2 >> lane) & 1u) ? ls.s2 : 0u);
+#pragma unroll
+    for (int k = 0; k < 3; ++k)
+        if ((__popc(c0[k] & u0) + __popc(c1[k] & u1) + __popc(c2[k] & u2)) & 1) bs ^= s.ssyn[32 * k + lane];
+    bs = __reduce_xor_sync(FULL, bs);
+    // 91-bit word of vector vi (0: order 0, i + 1: flip i, -1: none), XOR-accumulated into w0..w2; every lane gets the result
     auto osd_word = [&](int vi, uint32_t& w0, uint32_t& w1, uint32_t& w2) {
         if (vi < 0) return;
         uint32_t x0 = 0, x1 = 0, x2 = 0;
@@ -361,10 +380,10 @@ __device__ __forceinline__ int osd_warp(OsdWarpScratch& s, const OsdCtaTables& g
         for (int k = 0; k < 3; ++k) {
             const int c = ownrow[k];
             if (c < 91) {
-                uint32_t b;
-                if (vi == 0) b = (__popc(c0[k] & u0) + __popc(c1[k] & u1) + __popc(c2[k] & u2)) & 1u;
-                else b = (((prow < 32) ? c0[k] : ((prow < 64) ? c1[k] : c2[k])) >> (prow & 31)) & 1u;
-                if (b) { const uint32_t bit = 1u << (c & 31); if (c < 32) x0 |= bit; else if (c < 64) x1 |= bit; else x2 |= bit; }
+                uint32_t bt;
+                if (vi == 0) bt = (__popc(c0[k] & u0) + __popc(c1[k] & u1) + __popc(c2[k] & u2)) & 1u;
+                else bt = (((prow < 32) ? c0[k] : ((prow < 64) ? c1[k] : c2[k])) >> (prow & 31)) & 1u;
+                if (bt) { const uint32_t bit = 1u << (c & 31); if (c < 32) x0 |= bit; else if (c < 64) x1 |= bit; else x2 |= bit; }
             }
         }
         x0 = __reduce_or_sync(FULL, x0); x1 = __reduce_or_sync(FULL, x1); x2 = __reduce_or_sync(FULL, x2);
@@ -372,13 +391,12 @@ __device__ __forceinline__ int osd_warp(OsdWarpScratch& s, const OsdCtaTables& g
         else if (pcol < 91) { const uint32_t bit = 1u << (pcol & 31); if (pcol < 32) x0 |= bit; else if (pcol < 64) x1 |= bit; else x2 |= bit; }
         w0 ^= x0; w1 ^= x1; w2 ^= x2;
     };
-    // ---- 5. enumerate trials in the reference's order; first with payload != 0, CRC ok, valid payload
-    //      trial 0: base; 1..S: single flips i = 0..S-1; then pairs (i, j), j < D, j < i, i-major.
+    // enumerate trials in the reference's order; first with payload != 0, CRC ok, valid payload
+    // trial 0: base; 1..S: single flips i = 0..S-1; then pairs (i, j), j < D, j < i, i-major.
     const int nsingle = S;
     const int npair = (S <= D) ? S * (S - 1) / 2 : D * (D - 1) / 2 + (S - D) * D;      // sum over i < S of min(i, D)
     const int ntrial = 1 + nsingle + npair;
     const int tri = D * (D - 1) / 2;               // pairs of the rows i < D (row i has i of them); every later row has D
-    const uint32_t bs = s.syn[0];
     for (int base = 0; base < ntrial; base += 32) {
         const int tr = base + lane;
         bool pass = false;
@@ -392,8 +410,8 @@ __device__ __forceinline__ int osd_warp(OsdWarpScratch& s, const OsdCtaTables& g
                 else { int i = 0; while (q >= i) { q -= i; ++i; } fi = i; fj = q; }
             }
             uint32_t syn = bs;
-            if (fi >= 0) syn ^= s.syn[1 + fi];
-            if (fj >= 0) syn ^= s.syn[1 + fj];
+            if (fi >= 0) syn ^= s.syn[fi];
+            if (fj >= 0) syn ^= s.syn[fj];
             pass = (syn == 0);
         }
         uint32_t ballot = __ballot_sync(FULL, pass);
@@ -414,6 +432,14 @@ __device__ __forceinline__ int osd_warp(OsdWarpScratch& s, const OsdCtaTables& g
     bits[0] = bits[1] = bits[2] = 0u;
     osd_word(0, bits[0], bits[1], bits[2]);           // nothing accepted: report the order-0 word
     return 0;
+}
+
+// Returns trial index + 1 of the first accepted trial word (0 = none); bits = that word.
+// llr: 174 floats in shared or global memory.
+__device__ __forceinline__ int osd_warp(OsdWarpScratch& s, const OsdCtaTables& g, const float* llr, int lane, const LaneSyn& ls, int S, int D, uint32_t* bits) {
+    OsdBasis ob;
+    osd_basis(s, g, llr, lane, S, ob);
+    return osd_eval(s, g, llr, lane, ls, S, D, ob, bits);
 }
 
 }  // namespace ft8

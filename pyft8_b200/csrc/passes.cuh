@@ -5,7 +5,7 @@
 //   k_pass0    ipass 0   grid LLRs; for AP in NoAP,CQ,RR73,73,RRR: GOOD91 then LDPC(35,5)      -> list_fine
 //   k_fine     ipass 1   fine sync (fine.cuh)
 //   k_pass234  ipass 2-4 gate (nsync > 6, sd > sd_min); GOOD91 x2; LDPC(35,5) x2; LDPC(90,20) x5 (+save) -> list_osd
-//   k_osd_items ipass 5-6 one warp per (candidate, OSD attempt): 5 AP'd llrs then the saved post-LDPC llrs
+//   k_osd_items ipass 5-6 one warp per OSD work item: 5 AP'd llrs (RR73, 73, RRR as one item) then the saved post-LDPC llrs
 //   k_osd_resolve        first successful attempt in reference order wins
 // All kernels are persistent: warps pull work from device-resident lists through atomic cursors (the cost per candidate
 // varies from nothing to 110 LDPC iterations), so the host never reads a count back between passes (no sync; the
@@ -269,7 +269,26 @@ struct OsdSmem {
     float llr[WARPS_PER_CTA][176];
 };
 
-// ipass 5-6: item = 10 * list index + attempt.  attempts 0..4: AP pattern on the fine llr; 5..9: saved llr.
+// OSD attempts k0 .. k1-1 of one candidate: attempt k < 5 is AP pattern k on src, k >= 5 is src itself.  Results go to
+// found[k], bits[3 k .. 3 k + 2]; returns the number of attempts run.  The attempts of one call must have equal |llr|: one
+// attempt, or the AP patterns 2..4 (RR73, 73 and RRR force the same positions 58..76 to +-5 and differ only in the signs).
+// The order, the basis and the flip syndromes are then found once, and each attempt only redoes its hard decisions.
+__device__ __forceinline__ int osd_attempts(OsdWarpScratch& s, const OsdCtaTables& g, float* llr, const float* src, int k0, int k1,
+                                            int lane, const LaneSyn& ls, int S, int D, int32_t* found, uint32_t* bits) {
+    OsdBasis ob;
+    for (int k = k0; k < k1; ++k) {
+        apply_ap(llr, src, k < 5 ? k : 0, lane);
+        if (k == k0) osd_basis(s, g, llr, lane, S, ob);
+        uint32_t w[3];
+        const int f = osd_eval(s, g, llr, lane, ls, S, D, ob, w);
+        if (lane == 0) { found[k] = f; bits[3 * k] = w[0]; bits[3 * k + 1] = w[1]; bits[3 * k + 2] = w[2]; }
+    }
+    return k1 - k0;
+}
+
+// ipass 5-6: item = 8 * list index + t.  t = 0, 1: AP attempt t; t = 2: AP attempts 2..4 on one basis; t = 3..7: saved
+// llr t - 3 (attempt t + 2).  Attempt k of a candidate writes osd_found / osd_bits at slot * 10 + k.
+constexpr int OSD_ITEMS_PER_CAND = 8;
 __global__ void __launch_bounds__(WARPS_PER_CTA * 32, 8)
 k_osd_items(CandState cs, const int32_t* __restrict__ list, const int32_t* __restrict__ count, int S, int D,
             int32_t* __restrict__ next_item, DevStats* __restrict__ stats) {
@@ -279,31 +298,23 @@ k_osd_items(CandState cs, const int32_t* __restrict__ list, const int32_t* __res
     const LaneSyn ls = load_lane_syn(lane);
     load_osd_tables(sm.tab);
     __syncthreads();
-    const int warps_total = gridDim.x * WARPS_PER_CTA;
-    const int n_items = *count * 10;
+    const int n_items = *count * OSD_ITEMS_PER_CAND;
     unsigned long long n_osd = 0;
-    (void)warps_total;
     for (;;) {
         int item = 0;
         if (lane == 0) item = atomicAdd(next_item, 1);
         item = __shfl_sync(0xffffffffu, item, 0);
         if (item >= n_items) break;
-        const int slot = list[item / 10], k = item % 10;
-        int found = 0;
-        uint32_t bits[3] = {0, 0, 0};
-        const bool run = (k < 5) || (k - 5 < cs.saved_n[slot]);
-        if (run) {
+        const int slot = list[item / OSD_ITEMS_PER_CAND], t = item % OSD_ITEMS_PER_CAND;
+        const int k0 = t < 3 ? t : t + 2, k1 = t == 2 ? 5 : k0 + 1;
+        int32_t* found = cs.osd_found + slot * 10;
+        uint32_t* bits = cs.osd_bits + slot * 30;
+        if (k0 < 5 || k0 - 5 < cs.saved_n[slot]) {
             // attempts 0..4: Candidate._set_AP pattern on the fine llr; 5..9: llr saved after a failed LDPC(90,20)
-            const float* src = (k < 5) ? cs.llr_fine + (size_t)slot * 174 : cs.saved_llr + ((size_t)slot * 5 + (k - 5)) * 174;
-            apply_ap(sm.llr[wi], src, (k < 5) ? k : 0, lane);
-            found = osd_warp(sm.w[wi], sm.tab, sm.llr[wi], lane, ls, S, D, bits);
-            ++n_osd;
-        }
-        if (lane == 0) {
-            cs.osd_found[slot * 10 + k] = found;
-            cs.osd_bits[(slot * 10 + k) * 3] = bits[0];
-            cs.osd_bits[(slot * 10 + k) * 3 + 1] = bits[1];
-            cs.osd_bits[(slot * 10 + k) * 3 + 2] = bits[2];
+            const float* src = (k0 < 5) ? cs.llr_fine + (size_t)slot * 174 : cs.saved_llr + ((size_t)slot * 5 + (k0 - 5)) * 174;
+            n_osd += osd_attempts(sm.w[wi], sm.tab, sm.llr[wi], src, k0, k1, lane, ls, S, D, found, bits);
+        } else if (lane == 0) {
+            found[k0] = 0; bits[3 * k0] = 0u; bits[3 * k0 + 1] = 0u; bits[3 * k0 + 2] = 0u;
         }
         __syncwarp();
     }

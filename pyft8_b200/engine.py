@@ -365,3 +365,12 @@ class Engine:
         out = np.empty_like(a)
         self._check(self._lib.ft8_debug_fft(self._h, a.shape[1], int(bool(inverse)), _ptr(a), _ptr(out), a.shape[0]))
         return out
+
+    def debug_osd_ap(self, llr, singleflips=30, doubleflips=2):
+        """The decode's pass-5 OSD attempts on each llr: found[N][5], bits[N][5][3] for AP patterns 0..4."""
+        x = np.ascontiguousarray(llr, np.float32).reshape(-1, 174)
+        N = x.shape[0]
+        found = np.empty((N, 5), np.int32)
+        bits = np.empty((N, 5, 3), np.uint32)
+        self._check(self._lib.ft8_debug_osd_ap(self._h, _ptr(x), N, int(singleflips), int(doubleflips), _ptr(found), _ptr(bits)))
+        return found, bits
