@@ -197,6 +197,29 @@ int ft8_decode_cycles_live(ft8_handle* h, const void* audio, int audio_dtype, in
                            ft8_record* rec, int rec_capacity, int32_t* n_rec, int mem);
 int ft8_live_reset(ft8_handle* h);
 
+/* Progressive form of ft8_decode_cycles_live: the live decode of the open cycle of B streams, released hop by hop at the
+ * hop a running reference Receiver emits each message (receiver.py:376-412, its scheduler loop run once after every hop,
+ * with the clock one microsecond after the hop).  audio is each stream's cycle buffer [B][180000]: only samples
+ * < 480 * hop are valid, and the call reads only those that arrived since its previous call.  hop increases strictly
+ * within a cycle (1..375); B and odd_even stay.  The call that passes hop S = search_h0_hi + 173 (260 by default) searches
+ * the ring as it is then and runs pass 0 on that snapshot; a candidate then runs pass k at hop d + k,
+ * d = max(S + 1, h0 + 285), its fine stage on the audio buffer as the receiver holds it at hop d + 1.  A call returns the
+ * records with emission hop e <= hop that earlier calls have not released, stream-major (ft8_record.cycle = stream) and in
+ * emission order -- e, then llr_sd at that hop descending, then candidate rank -- with n_rec[B] per stream and emit_hop[i]
+ * = e.  A record is a duplicate (emitted = 0) if an earlier one of the same stream-cycle, released or not, has its payload.
+ * The call with hop = 375 completes the cycle: it releases everything left (e up to 377, in the next cycle's first hops)
+ * and leaves ring, tail and previous cycle of every stream exactly as ft8_decode_cycles_live of the same audio does, so the
+ * two entries can follow each other at cycle boundaries.  FT8_E_BADARG: hop not increasing, B or odd_even changed within a
+ * cycle, odd_even equal to the last completed live cycle's, or ft8_decode_cycles_live / _seq called while a cycle is open
+ * (ft8_live_reset abandons it).  Other calls (isolated decodes, stage ops) may come in between and do not disturb it.
+ * Capacity as in ft8_decode_cycles (the released records count as released even when cut).  ft8_get_stats: the work of
+ * this call (cycles = B only in the completing call); ft8_last_kernel_ms(0): the call's device time. */
+int ft8_decode_cycles_live_progress(ft8_handle* h, const void* audio, int audio_dtype, int B, int odd_even, int hop,
+                                    ft8_record* rec, uint16_t* emit_hop, int rec_capacity, int32_t* n_rec, int mem);
+/* The search hop S of ft8_decode_cycles_live_progress for this handle's search range (260 for the default range): the first
+ * hop whose call searches; records can be released from hop S + 1 on. */
+int ft8_progress_search_hop(ft8_handle* h, int* hop);
+
 /* C consecutive live cycles of B streams in one call.  audio is [C][B][180000] (time-major: audio + c*B*180000 is the
  * batch a c-th ft8_decode_cycles_live call would get), so one stream's recording (B = 1) is one contiguous array.
  * Equivalent to, and bit-identical with:

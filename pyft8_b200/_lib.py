@@ -77,6 +77,8 @@ SIGNATURES = {
     "ft8_decode_cycles": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, _P, C.c_int, _P, C.c_int]),
     "ft8_decode_cycles_live": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, _P, C.c_int, _P, C.c_int]),
     "ft8_decode_cycles_live_seq": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, _P, C.c_int, _P, C.c_int]),
+    "ft8_decode_cycles_live_progress": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, C.c_int, _P, C.c_int]),
+    "ft8_progress_search_hop": (C.c_int, [_P, C.POINTER(C.c_int)]),
     "ft8_live_reset": (C.c_int, [_P]),
     "ft8_decode_cycles_stream": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, _P, C.c_int, _P, _P]),
     "ft8_synth_cycles": (C.c_int, [_P, _P, _P, _P, _P, C.c_int, C.c_int, C.c_float, C.c_uint64, _P, C.c_int]),

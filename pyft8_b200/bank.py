@@ -14,9 +14,13 @@ plus 'receiver'; `set_band(r, band)`; per-receiver waterfall rows on request (`w
 GUI reads, receiver.py:272-278); and the live waterfall semantics: each receiver's 750-row two-cycle ring lives on the
 device (`live_ring=True`, ft8_decode_cycles_live), so the first hops of a cycle see the previous cycle's audio and early
 candidates (h0 < -32) read the previous cycle's rows, exactly like a running reference Receiver (receiver.py:295-306,
-360).  What differs, stated: a cycle is searched and decoded when its 15 s are complete (the reference starts searching
-10.4 s into the cycle and decodes candidates as their payload region fills, receiver.py:389-407); the messages are the
-same and come out in the same order, up to 4.6 s later, and "ran out of decoding time" cannot happen.
+360).  By default a cycle is searched and decoded when its 15 s are complete (the reference starts searching 10.4 s into
+the cycle and decodes candidates as their payload region fills, receiver.py:389-407): the messages are the same and come
+out in the same order, up to 4.6 s later.  With `progressive=True` the bank follows the reference's schedule too
+(ft8_decode_cycles_live_progress): once the slowest receiver has passed the search hop, a progress call every
+`progress_hops` hops releases each message at the hop a running Receiver emits it (its 'decode_hop'), and the final call
+at the end of the cycle releases the rest.  Calls are lock-step over all receivers, at the slowest one's hop.  What stays
+different in either mode: "ran out of decoding time" cannot happen.
 """
 import queue
 import threading
@@ -42,15 +46,22 @@ def _pinned(shape):
 
 class ReceiverBank:
     def __init__(self, n_receivers, on_message=None, bands=None, device=0, engine=None, clock=None, sync_score_min=85,
-                 max_cands=200, columnar=False, decoder=None, live_ring=True):
+                 max_cands=200, columnar=False, decoder=None, live_ring=True, progressive=False, progress_hops=1):
         self.n = int(n_receivers)
         self.on_message = on_message
         self.bands = list(bands) if bands is not None else [None] * self.n
         self.columnar = columnar
         self.live_ring = live_ring    # True: every receiver keeps the reference's two-cycle waterfall ring on the device
                                       # (ft8_decode_cycles_live); False: each cycle decoded in isolation (SURVEY H5)
+        if progressive and not live_ring:
+            raise ValueError("progressive=True needs live_ring=True")
+        if int(progress_hops) < 1:
+            raise ValueError("progress_hops must be >= 1")
+        self.progressive = progressive    # release messages during the cycle at the reference's hops (see module docstring)
+        self.progress_hops = int(progress_hops)
         self._tu = TimeUtils(clock)
-        self._decoder = decoder       # test seam: callable(audio[R,180000], next_audio) -> record array
+        self._decoder = decoder       # test seam: callable(audio[R,180000]) -> record array; progressive:
+                                      # callable(audio[R,180000], hop) -> (record array, emission hops)
         self.engine = engine
         if decoder is None and engine is None:
             self.engine = Engine(device=device, max_cycles=self.n, max_cands=max_cands, sync_score_min=sync_score_min)
@@ -61,7 +72,13 @@ class ReceiverBank:
         self._pos = np.zeros(self.n, np.int64)            # samples of that cycle received so far
         self._q = queue.Queue()
         self._results = queue.Queue()
-        self._busy = set()                                # halves handed to the decoder and not yet released
+        self._busy = {}                                   # half -> cycle handed to the decoder and not yet released
+        # progressive mode: search hop, last progress hop requested for the open cycle, the latest requested hop and the
+        # last decoded hop per cycle (queued calls of one cycle collapse into the latest), the cycle's label
+        self._search_hop = self.engine.search_hop if self.engine is not None else 260
+        self._req = 0
+        self._latest, self._done, self._label = {}, {}, {}
+        self._seen = {}                                   # cycle -> (receiver, text) released by its earlier calls
         self._cv = threading.Condition()
         self._state = threading.RLock()                   # guards _cyc/_pos/_open and the close-of-cycle decision
         self._eng_lock = threading.Lock()                 # one handle = one stream: calls are serialised
@@ -75,7 +92,7 @@ class ReceiverBank:
     def _half_for(self, c):
         """Buffer half of cycle c, once the decoder has released it (it held cycle c - 2)."""
         with self._cv:
-            while (c & 1) in self._busy:
+            while self._busy.get(c & 1, c) != c:
                 self._cv.wait(0.05)
         return self._buf[c & 1]
 
@@ -105,6 +122,7 @@ class ReceiverBank:
                     closed += 1
             else:
                 self._pos[r] = p + k
+                self._progress()
         return closed
 
     def feed_all(self, block):
@@ -132,13 +150,46 @@ class ReceiverBank:
                 closed += 1
             else:
                 self._pos += k
+                self._progress()
         return closed
 
+    def _label_of(self, no, in_cycle):
+        """(cyclestart string, odd_even label) of cycle `no`, read from the clock during the cycle or just after it"""
+        if no not in self._label:
+            t = self._tu.time() - (0.0 if in_cycle else 1.0)
+            self._label[no] = (self._tu.cyclestart_string(t), self._tu.odd_even() ^ (0 if in_cycle else 1))
+        return self._label[no]
+
+    def _request(self, no, hop, in_cycle):
+        cs, odd_even = self._label_of(no, in_cycle)
+        with self._cv:
+            self._busy[no & 1] = no
+            self._latest[no] = hop
+        self._q.put((no, no & 1, cs, odd_even, list(self.bands)))
+
+    def _progress(self):
+        """progressive mode: a progress call when the slowest receiver's hop in the open cycle crosses a multiple of
+        progress_hops at or after the first hop that can release a message (search hop + 1)"""
+        if not self.progressive:
+            return
+        o = self._open
+        pos = np.where(self._cyc > o, 180000, self._pos)
+        hop = int(pos.min()) // 480
+        hop -= hop % self.progress_hops
+        if self._search_hop + 1 <= hop < 375 and hop > self._req:
+            self._req = hop
+            self._request(o, hop, True)
+
     def _close_cycle(self, cyclestart_string=None):
+        if self.progressive:
+            self._request(self._open, 375, self._req > 0)
+            self._req = 0
+            self._open += 1
+            return
         cs = cyclestart_string if cyclestart_string is not None else self._tu.cyclestart_string(self._tu.time() - 1.0)
         half = self._open & 1
         with self._cv:
-            self._busy.add(half)
+            self._busy[half] = self._open
         self._q.put((self._open, half, cs, self._tu.odd_even() ^ 1, list(self.bands)))
         self._open += 1
 
@@ -149,6 +200,9 @@ class ReceiverBank:
             if item is None:
                 return
             no, half, cs, odd_even, bands = item
+            if self.progressive:
+                self._run_progress(no, half, cs, odd_even, bands)
+                continue
             try:
                 audio = self._buf[half]
                 if self._decoder is not None:
@@ -160,36 +214,76 @@ class ReceiverBank:
                             rec, _ = self.engine.decode_cycles_live(audio, no & 1)
                         else:
                             rec, _ = self.engine.decode_cycles(audio, odd_even)
-                with self._cv:                            # audio consumed: the feeder may reuse this half
-                    self._busy.discard(half)
-                    self._cv.notify_all()
+                self._release(half)                       # audio consumed: the feeder may reuse this half
                 mb = format_records(rec, [cs] * self.n)
-                if self.columnar:
-                    out = mb
-                else:
-                    out = []
-                    kept = np.flatnonzero(mb.keep)
-                    for i, txt in zip(kept.tolist(), mb.msg_tuple[kept].tolist()):
-                        r = rec[i]
-                        m = record_to_message(r, cs, bands[int(r["cycle"])], odd_even, self._tu.time(), msg=txt)
-                        m["receiver"] = int(r["cycle"])
-                        out.append(m)
-                        if self.on_message:
-                            self.on_message(m)
+                out = mb if self.columnar else self._messages(rec, mb, cs, odd_even, bands)
                 self._results.put((no, out))
             except Exception as e:                        # surface decoder failures to the feeding thread
                 self._results.put((no, e))
             finally:
+                self._release(half)
+
+    def _release(self, half):
+        with self._cv:
+            self._busy.pop(half, None)
+            self._cv.notify_all()
+
+    def _messages(self, rec, mb, cs, odd_even, bands, emit_hop=None, seen=None):
+        """message dicts of the kept rows of a formatted batch (and on_message for each); in progressive mode also
+        'decode_hop', and rows whose (receiver, text) an earlier call of the cycle released are dropped"""
+        out = []
+        kept = np.flatnonzero(mb.keep)
+        for i, txt in zip(kept.tolist(), mb.msg_tuple[kept].tolist()):
+            r = rec[i]
+            if seen is not None:
+                key = (int(r["cycle"]), " ".join(txt))
+                if key in seen:
+                    continue
+                seen.add(key)
+            m = record_to_message(r, cs, bands[int(r["cycle"])], odd_even, self._tu.time(), msg=txt)
+            m["receiver"] = int(r["cycle"])
+            if emit_hop is not None:
+                m["decode_hop"] = int(emit_hop[i])
+            out.append(m)
+            if self.on_message:
+                self.on_message(m)
+        return out
+
+    def _run_progress(self, no, half, cs, odd_even, bands):
+        with self._cv:
+            hop = self._latest.get(no)
+        if hop is None or hop <= self._done.get(no, 0):
+            return                                    # collapsed into a later call of the same cycle
+        try:
+            audio = self._buf[half]
+            if self._decoder is not None:
+                rec, eh = self._decoder(audio, hop)
+            else:
+                with self._eng_lock:
+                    rec, _, eh = self.engine.decode_cycles_live_progress(audio, no & 1, hop)
+            self._done[no] = hop
+            seen = self._seen.setdefault(no, set())
+            mb = format_records(rec, [cs] * self.n)
+            self._results.put((no, hop, self._messages(rec, mb, cs, odd_even, bands, eh, seen)))
+        except Exception as e:                        # surface decoder failures to the feeding thread
+            self._done[no] = hop
+            self._results.put((no, hop, e))
+        finally:
+            if hop == 375:
+                self._release(half)
                 with self._cv:
-                    self._busy.discard(half)
-                    self._cv.notify_all()
+                    self._latest.pop(no, None)
+                self._done.pop(no, None)
+                self._label.pop(no, None)
+                self._seen.pop(no, None)
 
     def results(self, block=True, timeout=None):
-        """(cycle number, list of message dicts | MessageBatch) of the next decoded cycle; raises what the decoder raised."""
-        no, out = self._results.get(block, timeout)
-        if isinstance(out, Exception):
-            raise out
-        return no, out
+        """(cycle number, list of message dicts | MessageBatch) of the next decoded cycle; in progressive mode (cycle number,
+        hop, list of message dicts) of the next progress call.  Raises what the decoder raised."""
+        item = self._results.get(block, timeout)
+        if isinstance(item[-1], Exception):
+            raise item[-1]
+        return item
 
     # ------------------------------------------------------------------------------------------------ GUI support
     def waterfall(self, r):

@@ -61,9 +61,10 @@ template <typename T> class DevBuf {
 };
 
 // slots of d_counts / h_counts: the work-list lengths of the fine and OSD stages, the records written, the near-tie
-// candidates of the frequency scan, the work cursors of k_pass234 / k_osd_items / k_pass0, ft8_fine's out-of-range count
+// candidates of the frequency scan, the work cursors of k_pass234 / k_osd_items / k_pass0, ft8_fine's out-of-range count;
+// then the spectrum slots of a progressive hop and the near-tie candidates summed over the hops of a progressive call
 enum CountSlot { CNT_FINE, CNT_OSD, CNT_RECORDS, CNT_NEAR_TIE, CNT_CURSOR_PASS234, CNT_CURSOR_OSD, CNT_CURSOR_PASS0,
-                 CNT_FINE_BAD, CNT_SLOTS };
+                 CNT_FINE_BAD, CNT_PROG_SPEC, CNT_PROG_TIES, CNT_SLOTS };
 
 // timing events: event i (1..8) ends stage i of a decode as listed at ft8_last_kernel_ms; then the pair around a stand-alone
 // op and the two boundaries inside the three-kernel fine stage
@@ -73,6 +74,44 @@ enum Event { EV_START, EV_SPECTROGRAM, EV_SYNC, EV_CYCLE_SPECTRUM, EV_PASS0, EV_
 // `which` of ft8_last_kernel_ms
 enum KernelMs { MS_TOTAL, MS_SPECTROGRAM, MS_SYNC, MS_CYCLE_SPECTRUM, MS_PASS0, MS_FINE, MS_PASS234, MS_OSD, MS_RECORDS,
                 MS_FINE_TSCAN, MS_FINE_FSCAN, MS_FINE_FINAL, MS_COUNT };
+
+// Per-candidate state of B streams x max_cands slots (the arrays CandState views).
+struct CandBufs {
+    DevBuf<int16_t> f0, h0; DevBuf<float> score; DevBuf<int32_t> ncand;
+    DevBuf<uint8_t> status; DevBuf<float> llr_grid, grid_sd; DevBuf<int8_t> grid_snr;
+    DevBuf<float> llr_fine; DevBuf<FineOut> fine; DevBuf<float> saved; DevBuf<uint8_t> saved_n, saved_ap;
+    DevBuf<uint32_t> bits; DevBuf<uint8_t> ripass, rap, rmethod; DevBuf<uint16_t> rnits;
+    DevBuf<int32_t> osd_found; DevBuf<uint32_t> osd_bits;
+    cudaError_t ensure(size_t B, size_t N, cudaStream_t st) {
+        cudaError_t e = cudaSuccess;
+        auto E = [&](cudaError_t r) { if (e == cudaSuccess) e = r; };
+        E(f0.ensure(N, st)); E(h0.ensure(N, st)); E(score.ensure(N, st)); E(ncand.ensure(B, st));
+        E(status.ensure(N, st)); E(llr_grid.ensure(N * 174, st)); E(grid_sd.ensure(N, st)); E(grid_snr.ensure(N, st));
+        E(llr_fine.ensure(N * 174, st)); E(fine.ensure(N, st)); E(saved.ensure(N * 5 * 174, st)); E(saved_n.ensure(N, st));
+        E(saved_ap.ensure(N * 5, st)); E(bits.ensure(N * 3, st)); E(ripass.ensure(N, st)); E(rap.ensure(N, st));
+        E(rmethod.ensure(N, st)); E(rnits.ensure(N, st)); E(osd_found.ensure(N * 10, st)); E(osd_bits.ensure(N * 30, st));
+        return e;
+    }
+    CandState view(int K) const {
+        CandState cs;
+        cs.K = K; cs.n_cand = ncand; cs.f0 = f0; cs.h0 = h0; cs.score = score; cs.status = status; cs.llr_grid = llr_grid;
+        cs.grid_sd = grid_sd; cs.grid_snr = grid_snr; cs.llr_fine = llr_fine; cs.fine = fine; cs.saved_llr = saved;
+        cs.saved_n = saved_n; cs.saved_ap = saved_ap; cs.bits91 = bits; cs.r_ipass = ripass; cs.r_ap = rap; cs.r_method = rmethod;
+        cs.r_nits = rnits; cs.osd_found = osd_found; cs.osd_bits = osd_bits;
+        return cs;
+    }
+};
+
+// The open cycle of ft8_decode_cycles_live_progress: its streams, parity, last hop, and the per-candidate state that lives
+// from the search to the cycle's final call (its own buffers, so that other calls in between cannot disturb it).
+struct ProgCycle {
+    bool open = false;
+    int B = 0, parity = 0, hop = 0;
+    CandBufs cand;
+    DevBuf<int32_t> spec_of;          // [slots]: spectrum slot of a candidate in the hop whose fine stage it is in
+    DevBuf<int32_t> spec_stream;      // [streams]: stream of each spectrum slot of that hop
+    DevBuf<uint16_t> emit;            // [slots]: emission hop of each record of the call
+};
 
 struct ft8_handle {
     int device = 0;
@@ -102,6 +141,11 @@ struct ft8_handle {
     // live mode (ft8_decode_cycles_live): the reference's two-cycle waterfall ring per stream + the previous cycle's last window
     // (float32 whatever the input dtype; zero for a stream that has no previous cycle)
     DevBuf<float> d_ring, d_tail;
+    // and each stream's whole previous cycle (the fine stage of a progressive hop reads it) and, while a progressive cycle is
+    // open, its samples so far; float32 like the tail.  The scratch of a progressive hop: the rolled audio per spectrum slot.
+    DevBuf<float> d_prev_audio, d_cur_audio, d_roll;
+    int last_parity = -1;             // parity of the last completed live cycle, -1 after a reset
+    ProgCycle prog;
     // consecutive live cycles (ft8_decode_cycles_live_seq): one SEQ_ROWS-row grid and one previous-cycle tail per cycle of a piece
     DevBuf<float> d_seq_grid, d_seq_tail;
     DevBuf<float2> d_Y; size_t y_cycles = 0;
@@ -493,14 +537,19 @@ static int launch_spectrogram(ft8_handle* h, const void* d_audio, int dtype, int
 
 // d_grid points at the first of the B cycles; b0 = index of that cycle in the handle's per-cycle arrays; cycle_h0 = grid row
 // of the cycle's hop 0
-static int launch_sync(ft8_handle* h, const float* d_grid, int grid_rows, int B, int cycle_h0, int b0 = 0) {
+static int launch_sync(ft8_handle* h, const float* d_grid, int grid_rows, int B, int cycle_h0, int b0 = 0,
+                       CandBufs* out = nullptr) {
     const size_t K = h->cfg.max_cands;
+    int16_t* f0 = out ? (int16_t*)out->f0 : (int16_t*)h->d_f0;
+    int16_t* h0 = out ? (int16_t*)out->h0 : (int16_t*)h->d_h0;
+    float* score = out ? (float*)out->score : (float*)h->d_score;
+    int32_t* ncand = out ? (int32_t*)out->ncand : (int32_t*)h->d_ncand;
     k_sync_scores<<<dim3(SY_HS * (N_F0 / SY_TF), B), SY_NT, SY_SMEM_BYTES, h->stream>>>(
         d_grid, grid_rows, cycle_h0, h->d_best_score + (size_t)b0 * N_F0 * SY_HS, h->d_best_h0 + (size_t)b0 * N_F0 * SY_HS,
         h->cfg.search_h0_lo, h->cfg.search_h0_hi);
     CK(cudaGetLastError());
     k_topk<<<B, 960, 0, h->stream>>>(h->d_best_score + (size_t)b0 * N_F0 * SY_HS, h->d_best_h0 + (size_t)b0 * N_F0 * SY_HS, h->cfg.sync_score_min,
-                                     h->cfg.max_cands, h->d_f0 + b0 * K, h->d_h0 + b0 * K, h->d_score + b0 * K, h->d_ncand + b0,
+                                     h->cfg.max_cands, f0 + b0 * K, h0 + b0 * K, score + b0 * K, ncand + b0,
                                      h->cfg.search_f0_lo, h->cfg.search_f0_hi);
     CK(cudaGetLastError());
     return FT8_OK;
@@ -858,6 +907,48 @@ static int save_tails(ft8_handle* h, const void* d_audio, int dtype, int B, floa
     return FT8_OK;
 }
 
+// samples [lo, hi) of each of B cycles [B][180000] -> the same place of dst [B][180000] float32 (exact for int16).  lo and
+// hi are multiples of the 480-sample hop, so with 16-byte aligned audio (VEC) each thread moves 8 samples with 16-byte
+// accesses; a caller's device pointer with less alignment takes the sample-by-sample form.
+__device__ __forceinline__ void load8(const int16_t* p, float4& a, float4& b) {
+    const uint4 u = *reinterpret_cast<const uint4*>(p);
+    const short2* s = reinterpret_cast<const short2*>(&u);
+    a = make_float4(s[0].x, s[0].y, s[1].x, s[1].y);
+    b = make_float4(s[2].x, s[2].y, s[3].x, s[3].y);
+}
+__device__ __forceinline__ void load8(const float* p, float4& a, float4& b) {
+    a = reinterpret_cast<const float4*>(p)[0];
+    b = reinterpret_cast<const float4*>(p)[1];
+}
+template <typename T, bool VEC>
+__global__ void k_take_samples(const T* __restrict__ audio, int lo, int hi, float* __restrict__ dst) {
+    const size_t c = (size_t)blockIdx.y * CYCLE_SAMPLES;
+    if constexpr (!VEC) {
+        for (int i = lo + blockIdx.x * blockDim.x + threadIdx.x; i < hi; i += gridDim.x * blockDim.x) dst[c + i] = (float)audio[c + i];
+    } else {
+        for (int i = lo + 8 * (blockIdx.x * blockDim.x + threadIdx.x); i < hi; i += 8 * gridDim.x * blockDim.x) {
+            float4 a, b;
+            load8(audio + c + i, a, b);
+            reinterpret_cast<float4*>(dst + c + i)[0] = a;
+            reinterpret_cast<float4*>(dst + c + i)[1] = b;
+        }
+    }
+}
+
+static int take_samples(ft8_handle* h, const void* d_audio, int dtype, int B, int lo, int hi, float* dst) {
+    const bool vec = (uintptr_t)d_audio % 16 == 0;
+    const dim3 grid(std::min(vec ? 32 : 64, (hi - lo + (vec ? 2047 : 1023)) / (vec ? 2048 : 1024)), B);
+    if (dtype == FT8_AUDIO_I16) {
+        if (vec) k_take_samples<int16_t, true><<<grid, 256, 0, h->stream>>>((const int16_t*)d_audio, lo, hi, dst);
+        else k_take_samples<int16_t, false><<<grid, 256, 0, h->stream>>>((const int16_t*)d_audio, lo, hi, dst);
+    } else {
+        if (vec) k_take_samples<float, true><<<grid, 256, 0, h->stream>>>((const float*)d_audio, lo, hi, dst);
+        else k_take_samples<float, false><<<grid, 256, 0, h->stream>>>((const float*)d_audio, lo, hi, dst);
+    }
+    CK(cudaGetLastError());
+    return FT8_OK;
+}
+
 // Consecutive live cycles (ft8_decode_cycles_live_seq) are decoded in pieces: `steps` cycle steps of `streams` streams, one
 // batch of steps * streams cycles, cycle i = step * streams + stream, the first step of parity `parity`.  Each cycle gets a
 // SEQ_ROWS-row grid: rows 0..5 are the previous cycle's hops 370..375, rows 6..380 its own hops 1..375.  The search runs on
@@ -912,11 +1003,13 @@ static int seq_front(ft8_handle* h, const SeqPiece& sp, const char* d_audio, int
 // written by the previous piece or call) and every stream's tail, as the live calls of those steps leave them.
 static int seq_store(ft8_handle* h, const SeqPiece& sp, const char* d_audio, int dtype, int* launches) {
     const int last = sp.steps - 1, first = std::max(0, last - 1);
-    TRY(save_tails(h, d_audio + (size_t)last * sp.streams * CYCLE_SAMPLES * sample_bytes(dtype), dtype, sp.streams, h->d_tail));
+    const char* a = d_audio + (size_t)last * sp.streams * CYCLE_SAMPLES * sample_bytes(dtype);
+    TRY(save_tails(h, a, dtype, sp.streams, h->d_tail));
+    TRY(take_samples(h, a, dtype, sp.streams, 0, CYCLE_SAMPLES, h->d_prev_audio));
     k_seq_store_ring<<<dim3(375, (last - first + 1) * sp.streams), 256, 0, h->stream>>>(
         h->d_seq_grid + (size_t)first * sp.streams * SEQ_ROWS * GRID_COLS, h->d_ring, sp.streams, sp.parity ^ (first & 1));
     CK(cudaGetLastError());
-    *launches += 2;
+    *launches += 3;
     return FT8_OK;
 }
 
@@ -930,7 +1023,19 @@ static int clear_live(ft8_handle* h) {
     k_fill<<<h->n_sm * 8, 256, 0, h->stream>>>(h->d_ring, h->cap_cycles * (size_t)LIVE_ROWS * GRID_COLS, 1.0f);
     CK(cudaGetLastError());
     CK(cudaMemsetAsync(h->d_tail, 0, h->cap_cycles * (size_t)NFFT_S * sizeof(float), h->stream));
+    CK(cudaMemsetAsync(h->d_prev_audio, 0, h->cap_cycles * (size_t)CYCLE_SAMPLES * sizeof(float), h->stream));
+    h->prog.open = false;
+    h->last_parity = -1;
     return FT8_OK;
+}
+
+// the live state of every stream: ring, tail and previous cycle, allocated and cleared on first use
+static int ensure_live(ft8_handle* h) {
+    if (h->d_ring) return FT8_OK;
+    CK(h->d_ring.ensure(h->cap_cycles * (size_t)LIVE_ROWS * GRID_COLS, h->stream));
+    CK(h->d_tail.ensure(h->cap_cycles * (size_t)NFFT_S, h->stream));
+    CK(h->d_prev_audio.ensure(h->cap_cycles * (size_t)CYCLE_SAMPLES, h->stream));
+    return clear_live(h);
 }
 
 // Decode prologue.  A pending prefetch is consumed only by the streaming entry (consume_pf), whose caller named this very
@@ -958,8 +1063,10 @@ static int take_audio(ft8_handle* h, const void* audio, int dtype, int B, int me
 
 // Decode epilogue: counts, records and statistics back to the host.  Records are cycle-major, so when rec_capacity cuts
 // them the per-cycle counts are trimmed to what was copied.
-static int finish_decode(ft8_handle* h, int B, ft8_record* rec, int rec_capacity, int32_t* n_rec, int launches) {
-    CK(cudaMemcpyAsync(h->h_counts, h->d_counts, (CNT_NEAR_TIE + 1) * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+// A progressive call (d_emit != NULL) also copies the records' emission hops; its stage times are not separated.
+static int finish_decode(ft8_handle* h, int B, ft8_record* rec, int rec_capacity, int32_t* n_rec, int launches,
+                         const uint16_t* d_emit = nullptr, uint16_t* emit_hop = nullptr) {
+    CK(cudaMemcpyAsync(h->h_counts, h->d_counts, CNT_SLOTS * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaMemcpyAsync(h->h_stats, h->d_stats, sizeof(DevStats), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaMemcpyAsync(n_rec, h->d_rec_n, (size_t)B * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
@@ -967,6 +1074,7 @@ static int finish_decode(ft8_handle* h, int B, ft8_record* rec, int rec_capacity
     const int ncopy = std::min(nrec, rec_capacity);
     if (ncopy > 0) {
         CK(cudaMemcpyAsync(rec, h->d_rec, (size_t)ncopy * sizeof(ft8_record), cudaMemcpyDeviceToHost, h->stream));
+        if (d_emit) CK(cudaMemcpyAsync(emit_hop, d_emit, (size_t)ncopy * sizeof(uint16_t), cudaMemcpyDeviceToHost, h->stream));
         CK(cudaStreamSynchronize(h->stream));
     }
     const bool overflow = nrec > rec_capacity;
@@ -975,10 +1083,10 @@ static int finish_decode(ft8_handle* h, int B, ft8_record* rec, int rec_capacity
         for (int b = 0; b < B; ++b) { const int t = std::min(n_rec[b], left); n_rec[b] = t; left -= t; }
     }
     const int64_t emitted = (int64_t)h->h_stats->emitted;
+    memset(h->last_ms, 0, sizeof(h->last_ms));
     CK(cudaEventElapsedTime(&h->last_ms[MS_TOTAL], h->ev[EV_START], h->ev[EV_RECORDS]));
-    for (int i = MS_SPECTROGRAM; i <= MS_RECORDS; ++i) CK(cudaEventElapsedTime(&h->last_ms[i], h->ev[i - 1], h->ev[i]));
-    h->last_ms[MS_FINE_TSCAN] = h->last_ms[MS_FINE_FSCAN] = h->last_ms[MS_FINE_FINAL] = 0.0f;
-    if (h->cfg.fine_mode == 0) {
+    if (!d_emit) for (int i = MS_SPECTROGRAM; i <= MS_RECORDS; ++i) CK(cudaEventElapsedTime(&h->last_ms[i], h->ev[i - 1], h->ev[i]));
+    if (h->cfg.fine_mode == 0 && !d_emit) {
         CK(cudaEventElapsedTime(&h->last_ms[MS_FINE_TSCAN], h->ev[EV_PASS0], h->ev[EV_TSCAN_END]));
         CK(cudaEventElapsedTime(&h->last_ms[MS_FINE_FSCAN], h->ev[EV_TSCAN_END], h->ev[EV_FSCAN_END]));
         CK(cudaEventElapsedTime(&h->last_ms[MS_FINE_FINAL], h->ev[EV_FSCAN_END], h->ev[EV_FINE]));
@@ -989,7 +1097,7 @@ static int finish_decode(ft8_handle* h, int B, ft8_record* rec, int rec_capacity
     s.fine_evals = (int64_t)h->h_stats->fine_evals; s.fine_pass = (int64_t)h->h_stats->fine_pass;
     s.ldpc_calls = (int64_t)h->h_stats->ldpc_calls; s.ldpc_iters = (int64_t)h->h_stats->ldpc_iters;
     s.osd_calls = (int64_t)h->h_stats->osd_calls; s.decoded = nrec; s.emitted = emitted; s.kernel_launches = launches;
-    s.fine_rechecked = h->cfg.fine_mode == 0 ? h->h_counts[CNT_NEAR_TIE] : 0;
+    s.fine_rechecked = h->cfg.fine_mode == 1 ? 0 : d_emit ? h->h_counts[CNT_PROG_TIES] : h->h_counts[CNT_NEAR_TIE];
     if (overflow) return fail(h, FT8_E_CAPACITY, "ft8_decode_cycles: rec_capacity too small (records truncated)");
     return FT8_OK;
 }
@@ -1014,11 +1122,8 @@ static int decode_cycles_core(ft8_handle* h, const void* audio, int audio_dtype,
     const int grows = seq ? SEQ_ROWS : live ? LIVE_ROWS : GRID_ROWS;
     float* gbase = h->d_grid;
     if (live || seq) {
-        if (!h->d_ring) {
-            CK(h->d_ring.ensure(h->cap_cycles * (size_t)LIVE_ROWS * GRID_COLS, h->stream));
-            CK(h->d_tail.ensure(h->cap_cycles * (size_t)NFFT_S, h->stream));
-            TRY(clear_live(h));
-        }
+        if (h->prog.open) return fail(h, FT8_E_BADARG, "ft8_decode_cycles_live: a progressive cycle is open (finish it with hop 375 or call ft8_live_reset)");
+        TRY(ensure_live(h));
         gbase = h->d_ring;
     }
     if (seq) {
@@ -1079,7 +1184,11 @@ static int decode_cycles_core(ft8_handle* h, const void* audio, int audio_dtype,
     CK(cudaEventRecord(h->ev[EV_CYCLE_SPECTRUM], h->stream));
     if (next_audio_host && !prefetched) TRY(ft8_prefetch_audio(h, next_audio_host, audio_dtype, B));
     if (seq) TRY(seq_store(h, *seq, (const char*)da, audio_dtype, &launches));
-    else if (live) { TRY(save_tails(h, da, audio_dtype, B, h->d_tail)); ++launches; }   // after S1 has read the old tails
+    else if (live) {                                   // after S1 has read the old tails
+        TRY(save_tails(h, da, audio_dtype, B, h->d_tail));
+        TRY(take_samples(h, da, audio_dtype, B, 0, CYCLE_SAMPLES, h->d_prev_audio));
+        launches += 2;
+    }
     CandState cs = cand_state(h);
     // ipass 0
     k_pass0<<<persistent_blocks(h, 8), WARPS_PER_CTA * 32, sizeof(PassSmem), h->stream>>>(
@@ -1124,7 +1233,9 @@ extern "C" int ft8_decode_cycles(ft8_handle* h, const void* audio, int audio_dty
 extern "C" int ft8_decode_cycles_live(ft8_handle* h, const void* audio, int audio_dtype, int B, int odd_even, ft8_record* rec,
                                       int rec_capacity, int32_t* n_rec, int mem) {
     if (odd_even != 0 && odd_even != 1) return fail(h, FT8_E_BADARG, "ft8_decode_cycles_live: odd_even must be 0 or 1");
-    return decode_cycles_core(h, audio, audio_dtype, B, odd_even, rec, rec_capacity, n_rec, mem, nullptr, false, true);
+    const int rc = decode_cycles_core(h, audio, audio_dtype, B, odd_even, rec, rec_capacity, n_rec, mem, nullptr, false, true);
+    if (rc == FT8_OK || rc == FT8_E_CAPACITY) h->last_parity = odd_even;
+    return rc;
 }
 
 // C steps of B streams in pieces of floor(max_cycles / B) steps; each piece is one decode batch.  Records of a piece land after
@@ -1153,6 +1264,7 @@ extern "C" int ft8_decode_cycles_live_seq(ft8_handle* h, const void* audio, int 
         const int rc = decode_cycles_core(h, (const char*)audio + (size_t)c0 * step_bytes, audio_dtype, nb, sp.parity, r,
                                           rec_capacity - written, n, mem, nullptr, false, false, &sp);
         if (rc != FT8_OK && rc != FT8_E_CAPACITY) return rc;
+        h->last_parity = sp.parity ^ ((sp.steps - 1) & 1);
         overflow = overflow || rc == FT8_E_CAPACITY;
         int got = 0;
         for (int i = 0; i < nb; ++i) got += n[i];
@@ -1172,6 +1284,183 @@ extern "C" int ft8_decode_cycles_live_seq(ft8_handle* h, const void* audio, int 
     memcpy(h->last_ms, ms, sizeof(ms));
     if (overflow) return fail(h, FT8_E_CAPACITY, "ft8_decode_cycles_live_seq: rec_capacity too small (records truncated)");
     return FT8_OK;
+}
+
+// ------------------------------------------------------------------------------------------ progressive live decoding
+// One CTA per stream: its candidates still pending after pass 0 whose fine stage runs at hop T (d + 1 == T) go to `list`
+// (*count), and a stream that has any gets one spectrum slot (*n_spec, spec_stream[slot] = stream, spec_of[cand] = slot).
+__global__ void __launch_bounds__(256) k_prog_due(CandState cs, int S, int T, int32_t* __restrict__ list, int32_t* __restrict__ count,
+                                                  int32_t* __restrict__ spec_of, int32_t* __restrict__ spec_stream,
+                                                  int32_t* __restrict__ n_spec) {
+    __shared__ int s_any, s_slot;
+    const int b = blockIdx.x, n = cs.n_cand[b];
+    if (threadIdx.x == 0) s_any = 0;
+    __syncthreads();
+    bool due[4] = {};
+    for (int k = 0, r = threadIdx.x; k < 4 && r < n; ++k, r += blockDim.x) {     // max_cands <= 928 < 4 * 256
+        const int slot = b * cs.K + r;
+        due[k] = cs.status[slot] == ST_PENDING && prog_due_hop(S, cs.h0[slot]) + 1 == T;
+        if (due[k]) s_any = 1;
+    }
+    __syncthreads();
+    if (!s_any) return;
+    if (threadIdx.x == 0) { s_slot = atomicAdd(n_spec, 1); spec_stream[s_slot] = b; }
+    __syncthreads();
+    for (int k = 0, r = threadIdx.x; k < 4 && r < n; ++k, r += blockDim.x) {
+        if (!due[k]) continue;
+        const int slot = b * cs.K + r;
+        spec_of[slot] = s_slot;
+        list[atomicAdd(count, 1)] = slot;
+    }
+}
+
+// The audio AudioIn.get_cycle_spectrum transforms at hop T of a cycle (receiver.py:280-286): the last 180000 samples
+// (prev[480 T ..] then cur[.. 480 T)) rolled by int((15 - cycle_time) * 12000) = 180000 - 480 T - 1 with the clock one
+// microsecond after the hop, i.e. out = [prev[179999], cur[0 .. 480 T - 1], prev[480 T .. 179998]].
+__global__ void k_prog_roll(const float* __restrict__ cur, const float* __restrict__ prev, const int32_t* __restrict__ spec_stream,
+                            int T, float* __restrict__ out) {
+    const size_t b = (size_t)spec_stream[blockIdx.y] * CYCLE_SAMPLES;
+    float* o = out + (size_t)blockIdx.y * CYCLE_SAMPLES;
+    const int n_cur = HOP * T;
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < CYCLE_SAMPLES; i += gridDim.x * blockDim.x)
+        o[i] = i == 0 ? prev[b + CYCLE_SAMPLES - 1] : i <= n_cur ? cur[b + i - 1] : prev[b + i - 1];
+}
+
+__global__ void k_add_count(int32_t* __restrict__ acc, const int32_t* __restrict__ v) { *acc += *v; }
+
+// The fine stage and passes 2-6 of the candidates whose fine stage runs at hop T (pass 1 at d + 1; passes 2-6 need no
+// further audio, so they run now and only their emission waits for hop d + k).  Returns FT8_OK with nothing launched but
+// k_prog_due when no candidate is due.
+static int prog_hop(ft8_handle* h, const CandState& cs, int B, int S, int T, int* launches) {
+    ProgCycle& pc = h->prog;
+    CK(cudaMemsetAsync(h->d_counts, 0, CNT_FINE_BAD * sizeof(int32_t), h->stream));
+    CK(cudaMemsetAsync(h->d_counts + CNT_PROG_SPEC, 0, sizeof(int32_t), h->stream));
+    k_prog_due<<<B, 256, 0, h->stream>>>(cs, S, T, h->d_list_fine, h->d_counts + CNT_FINE, pc.spec_of, pc.spec_stream,
+                                         h->d_counts + CNT_PROG_SPEC);
+    CK(cudaGetLastError()); ++*launches;
+    CK(cudaMemcpyAsync(h->h_counts, h->d_counts, CNT_SLOTS * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    const int n_spec = h->h_counts[CNT_PROG_SPEC];
+    if (n_spec == 0) return FT8_OK;
+    k_prog_roll<<<dim3(32, n_spec), 256, 0, h->stream>>>(h->d_cur_audio, h->d_prev_audio, pc.spec_stream, T, h->d_roll);
+    CK(cudaGetLastError()); ++*launches;
+    TRY(launch_cycle_spectrum(h, h->d_roll, FT8_AUDIO_F32, n_spec, h->d_spec, FINE_SPEC_STRIDE, FINE_SPEC_STRIDE - 1));
+    *launches += 2 * ((n_spec + (int)h->y_cycles - 1) / (int)h->y_cycles);
+    TRY(launch_fine(h, h->d_spec, FINE_SPEC_STRIDE, h->d_list_fine, h->d_counts + CNT_FINE, 0, pc.spec_of, cs.f0, cs.h0,
+                    cs.fine, cs.llr_fine, nullptr));
+    *launches += fine_launches(h);
+    if (h->cfg.fine_mode == 0) {
+        k_add_count<<<1, 1, 0, h->stream>>>(h->d_counts + CNT_PROG_TIES, h->d_counts + CNT_NEAR_TIE);
+        CK(cudaGetLastError()); ++*launches;
+    }
+    k_pass234<<<persistent_blocks(h, 8), WARPS_PER_CTA * 32, sizeof(PassSmem), h->stream>>>(
+        cs, h->d_list_fine, h->d_counts + CNT_FINE, h->cfg.llr_sd_min, h->d_list_osd, h->d_counts + CNT_OSD,
+        h->d_counts + CNT_CURSOR_PASS234, h->d_stats);
+    CK(cudaGetLastError()); ++*launches;
+    k_osd_items<<<persistent_blocks(h, 8), WARPS_PER_CTA * 32, sizeof(OsdSmem), h->stream>>>(
+        cs, h->d_list_osd, h->d_counts + CNT_OSD, h->cfg.osd_singleflips, h->cfg.osd_doubleflips, h->d_counts + CNT_CURSOR_OSD,
+        h->d_stats);
+    CK(cudaGetLastError()); ++*launches;
+    k_osd_resolve<<<persistent_blocks(h, 2), 128, 0, h->stream>>>(cs, h->d_list_osd, h->d_counts + CNT_OSD, h->d_stats);
+    CK(cudaGetLastError()); ++*launches;
+    return FT8_OK;
+}
+
+// Hop after which the progressive search runs: one past Receiver.search_start_hop = search_h0_hi + 43 * 4 (receiver.py:320,
+// 405), i.e. 260 with the default range
+static int prog_search_hop(const ft8_handle* h) { return h->cfg.search_h0_hi + 173; }
+
+extern "C" int ft8_progress_search_hop(ft8_handle* h, int* hop) {
+    if (!h || !hop) return FT8_E_BADARG;
+    *hop = prog_search_hop(h);
+    return FT8_OK;
+}
+
+extern "C" int ft8_decode_cycles_live_progress(ft8_handle* h, const void* audio, int audio_dtype, int B, int odd_even, int hop,
+                                               ft8_record* rec, uint16_t* emit_hop, int rec_capacity, int32_t* n_rec, int mem) {
+    ENTER(h);
+    if (!audio || !rec || !emit_hop || !n_rec || B <= 0 || rec_capacity < 0 || (odd_even != 0 && odd_even != 1) || hop < 1 || hop > 375)
+        return fail(h, FT8_E_BADARG, "ft8_decode_cycles_live_progress: bad argument (odd_even 0 or 1, 1 <= hop <= 375)");
+    if ((size_t)B > h->cap_cycles) return fail(h, FT8_E_CAPACITY, "ft8_decode_cycles_live_progress: B exceeds cfg.max_cycles");
+    TRY(check_dtype(h, audio_dtype));
+    ProgCycle& pc = h->prog;
+    if (pc.open && (B != pc.B || odd_even != pc.parity || hop <= pc.hop))
+        return fail(h, FT8_E_BADARG, "ft8_decode_cycles_live_progress: B and odd_even must stay and hop must increase within a cycle");
+    if (!pc.open && h->last_parity >= 0 && odd_even == h->last_parity)
+        return fail(h, FT8_E_BADARG, "ft8_decode_cycles_live_progress: odd_even must alternate from cycle to cycle");
+    TRY(ensure_live(h));
+    const size_t K = h->cfg.max_cands, N = (size_t)B * K;
+    CK(h->d_cur_audio.ensure(h->cap_cycles * (size_t)CYCLE_SAMPLES, h->stream));
+    CK(h->d_roll.ensure(h->cap_cycles * (size_t)CYCLE_SAMPLES, h->stream));
+    CK(pc.cand.ensure(h->cap_cycles, h->cap_slots, h->stream));
+    CK(pc.spec_of.ensure(h->cap_slots, h->stream));
+    CK(pc.spec_stream.ensure(h->cap_cycles, h->stream));
+    CK(pc.emit.ensure(h->cap_slots, h->stream));
+    if (h->pf_host) { CK(cudaStreamSynchronize(h->copy_stream)); h->pf_host = nullptr; }   // a pending prefetch is dropped
+    if (!pc.open) { pc.open = true; pc.B = B; pc.parity = odd_even; pc.hop = 0; }
+    const int prev = pc.hop, cycle_h0 = 375 * odd_even;
+    const int S = prog_search_hop(h);
+    const CandState cs = pc.cand.view((int)K);
+    int launches = 0;
+    CK(cudaMemsetAsync(h->d_counts, 0, CNT_SLOTS * sizeof(int32_t), h->stream));
+    CK(cudaMemsetAsync(h->d_stats, 0, sizeof(DevStats), h->stream));
+    CK(cudaEventRecord(h->ev[EV_START], h->stream));
+    // the samples that arrived since the previous call
+    const size_t esz = sample_bytes(audio_dtype), lo = (size_t)HOP * prev, hi = (size_t)HOP * hop;
+    const void* da = audio;
+    if (mem == FT8_MEM_HOST) {
+        CK(h->d_audio.ensure((size_t)B * CYCLE_SAMPLES * esz, h->stream));
+        CK(cudaMemcpy2DAsync(h->d_audio + lo * esz, CYCLE_SAMPLES * esz, (const char*)audio + lo * esz, CYCLE_SAMPLES * esz,
+                             (hi - lo) * esz, B, cudaMemcpyHostToDevice, h->stream));
+        da = h->d_audio;
+    }
+    TRY(take_samples(h, da, audio_dtype, B, (int)lo, (int)hi, h->d_cur_audio)); ++launches;
+    // ring rows of the new hops; the search and pass 0 read the ring as it is at hop S
+    auto rows = [&](int r0, int r1) -> int {
+        if (r0 >= r1) return FT8_OK;
+        ++launches;
+        return launch_spectrogram(h, h->d_cur_audio, FT8_AUDIO_F32, B, h->d_ring, r0 + 1, r1, LIVE_ROWS, -cycle_h0, 0, h->d_tail, 1);
+    };
+    if (prev < S && hop >= S) {
+        TRY(rows(prev, S));
+        TRY(launch_sync(h, h->d_ring, LIVE_ROWS, B, cycle_h0, 0, &pc.cand)); launches += 2;
+        k_pass0<<<persistent_blocks(h, 8), WARPS_PER_CTA * 32, sizeof(PassSmem), h->stream>>>(
+            cs, (int)N, h->d_ring, LIVE_ROWS, cycle_h0, h->cfg.llr_sd_min, nullptr, 0, h->d_list_fine, h->d_counts + CNT_FINE,
+            h->d_counts + CNT_CURSOR_PASS0, h->d_stats);
+        CK(cudaGetLastError()); ++launches;
+        TRY(rows(S, hop));
+    } else {
+        TRY(rows(prev, hop));
+    }
+    // fine stage and passes 2-6 hop by hop: at most one spectrum per stream at a time
+    for (int T = std::max(prev + 1, S + 2); T <= std::min(hop, 372); ++T) TRY(prog_hop(h, cs, B, S, T, &launches));
+    if (hop >= S) {
+        // records with e in (prev, hop]; the final call releases everything left (e up to 377, in the next cycle's hops)
+        const int e_hi = hop == 375 ? 1 << 20 : hop;
+        k_prog_rec<false><<<B, REC_NT, 0, h->stream>>>(cs, cs.fine, S, prev, e_hi, h->d_rec_n, nullptr, nullptr, nullptr, h->d_stats);
+        CK(cudaGetLastError());
+        k_rec_scan<<<1, 1024, 0, h->stream>>>(h->d_rec_n, B, h->d_rec_base, h->d_counts + CNT_RECORDS);
+        CK(cudaGetLastError());
+        k_prog_rec<true><<<B, REC_NT, 0, h->stream>>>(cs, cs.fine, S, prev, e_hi, nullptr, h->d_rec_base, h->d_rec, pc.emit, h->d_stats);
+        CK(cudaGetLastError());
+        launches += 3;
+    } else {
+        CK(cudaMemsetAsync(h->d_rec_n, 0, (size_t)B * sizeof(int32_t), h->stream));
+        CK(cudaMemsetAsync(h->d_counts + CNT_RECORDS, 0, sizeof(int32_t), h->stream));
+    }
+    if (hop == 375) {
+        // the cycle is complete: tails and previous cycle as ft8_decode_cycles_live of the same audio leaves them
+        TRY(save_tails(h, h->d_cur_audio, FT8_AUDIO_F32, B, h->d_tail));
+        CK(cudaMemcpyAsync(h->d_prev_audio, h->d_cur_audio, (size_t)B * CYCLE_SAMPLES * sizeof(float), cudaMemcpyDeviceToDevice,
+                           h->stream));
+        ++launches;
+    }
+    CK(cudaEventRecord(h->ev[EV_RECORDS], h->stream));
+    pc.hop = hop;
+    if (hop == 375) { pc.open = false; h->last_parity = odd_even; }
+    const int rc = finish_decode(h, B, rec, rec_capacity, n_rec, launches, pc.emit, emit_hop);
+    h->stats.cycles = hop == 375 ? B : 0;        // counted once, by the call that completes the cycles
+    return rc;
 }
 
 extern "C" int ft8_live_reset(ft8_handle* h) {

@@ -114,6 +114,9 @@ class Engine:
             raise RuntimeError(f"ft8_create failed ({rc}): {msg}")
         self.device = int(device)
         self.max_cycles, self.max_cands = int(max_cycles), int(max_cands)
+        hop = C.c_int()
+        self._check(self._lib.ft8_progress_search_hop(self._h, C.byref(hop)))
+        self.search_hop = hop.value                       # the hop whose progress call searches (ft8_progress_search_hop)
 
     def close(self):
         if getattr(self, "_h", None):
@@ -311,6 +314,33 @@ class Engine:
         self._check(self._lib.ft8_decode_cycles_live_seq(self._h, _ptr(a), dt, B, C_, int(odd_even), _ptr(rec), len(rec), _ptr(n),
                                                          L.MEM_HOST))
         return rec[:int(n[:C_ * B].sum())], n[:C_ * B].reshape(C_, B)
+
+    def decode_cycles_live_progress(self, audio, odd_even, hop, rec=None, n=None, emit_hop=None):
+        """Progressive live decoding of the open cycle of B streams (ft8_decode_cycles_live_progress): audio [B,180000]
+        int16/float32 is each stream's cycle buffer, valid below sample 480*hop.  Call with increasing hop (1..375) within a
+        cycle, the last call with hop=375; alternate odd_even from cycle to cycle like decode_cycles_live.  Returns
+        (records released by this call, stream-major in emission order, n_rec[B], emit_hop[uint16] per record)."""
+        a, dt = self._audio(audio)
+        B = a.shape[0]
+        rec, n = self._outputs(B, rec, n)
+        if emit_hop is None:
+            emit_hop = np.zeros(len(rec), np.uint16)
+        elif emit_hop.dtype != np.uint16 or len(emit_hop) < len(rec) or not emit_hop.flags.c_contiguous:
+            raise ValueError("emit_hop must be a contiguous uint16 array at least as long as rec")
+        self._check(self._lib.ft8_decode_cycles_live_progress(self._h, _ptr(a), dt, B, int(odd_even), int(hop), _ptr(rec), _ptr(emit_hop),
+                                                              len(rec), _ptr(n), L.MEM_HOST))
+        k = int(n[:B].sum())
+        return rec[:k], n[:B], emit_hop[:k]
+
+    def decode_cycles_live_progress_dev(self, audio_ptr, dtype, B, odd_even, hop, rec=None, n=None, emit_hop=None):
+        """Same, with the [B,180000] audio already resident on this engine's device (raw pointer)."""
+        rec, n = self._outputs(B, rec, n)
+        if emit_hop is None:
+            emit_hop = np.zeros(len(rec), np.uint16)
+        self._check(self._lib.ft8_decode_cycles_live_progress(self._h, C.c_void_p(audio_ptr), dtype, B, int(odd_even), int(hop),
+                                                              _ptr(rec), _ptr(emit_hop), len(rec), _ptr(n), L.MEM_DEVICE))
+        k = int(n[:B].sum())
+        return rec[:k], n[:B], emit_hop[:k]
 
     def live_reset(self):
         self._check(self._lib.ft8_live_reset(self._h))
